@@ -6,7 +6,7 @@ windows (res x res pixels each) through ground-state solve -> latching -> sensor
 BASELINE config 4 -- 8-dot latched array, 16384 envs PER GPU (weak scaling: envs shard by contiguous env id, no
 collective on the step path), 64x64 scans, full sensor-noise model.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0.  `value` = pixels/s with descriptors and models resident in HBM; `e2e` = the same
@@ -281,6 +281,30 @@ def issue_roofline(kernels, pixels_per_s: float, sm_count: int, sm_mhz: float):
             "traffic_note": "DRAM bytes per pixel of the listed kernels (dram__bytes_read.sum + dram__bytes_write.sum)"}
 
 
+def dump_outputs(out_dir: str, prefix: str, z, n, res: int, budget_bytes: int, seed: int):
+    """Write what a timed launch returned, for output-for-output comparison of two builds: a fixed, seeded sample of
+    whole scans as ``<prefix>z.npy`` (scans, res, res) float32 sensor images, ``<prefix>n.npy`` (scans, res, res, N)
+    float32 charge occupations and ``<prefix>scan_index.npy`` (float64), the sampled scans' positions in the batch.
+    The three files together stay within ``budget_bytes``."""
+    import torch
+    pp = res * res
+    n_dot = n.shape[-1]
+    n_scan = z.numel() // pp
+    count = min(n_scan, (budget_bytes - 3 * 128) // (pp * 4 * (1 + n_dot) + 8))       # 128 B: one .npy header
+    if count < 1:
+        raise SystemExit(f"--dump-outputs: one {res}x{res} scan exceeds the {budget_bytes}-byte budget of '{prefix}'")
+    pick = np.sort(np.random.default_rng(seed).choice(n_scan, size=count, replace=False))
+    idx = torch.from_numpy(pick).to(z.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, prefix + "z.npy"), z.view(n_scan, res, res)[idx].float().cpu().numpy())
+    np.save(os.path.join(out_dir, prefix + "n.npy"), n.view(n_scan, res, res, n_dot)[idx].float().cpu().numpy())
+    np.save(os.path.join(out_dir, prefix + "scan_index.npy"), pick.astype(np.float64))
+
+
+# --dump-outputs budgets (bytes): the headline launch and the tunnel-path block, under 64 MB in all
+DUMP_BYTES_MAIN, DUMP_BYTES_TUNNEL = 45_900_000, 17_900_000
+
+
 def tunnel_kernels(n_dot: int):
     # (the fix-up passes of the block-walk select kernel and of the Householder eigen kernel over the pixels the
     # enumeration / Noda kernels gave up on, < 0.5 % of them, are not counted)
@@ -289,10 +313,10 @@ def tunnel_kernels(n_dot: int):
 
 
 def tunnel_path_block(eng, n_dot: int, res: int, flags: int, with_cpu: bool, n_env: int = 512, steps: int = 5,
-                      warmup: int = 5, sm_mhz: float = 1965.0):
+                      warmup: int = 5, sm_mhz: float = 1965.0, dump_dir: str | None = None):
     """Path B on the same GPU (what env.step runs in barrier mode): device-resident timing (CUDA events, warmed) AND the
     end-to-end host-buffer call, the issue-slot roofline from the committed ncu figure, and the C restatement of the
-    reference's formulation on the host cores."""
+    reference's formulation on the host cores.  ``dump_dir``: write a sample of the last timed launch's outputs there."""
     import torch
     from qdsim import N_F32, N_NONE
     dev, mb, sets = build_workload(n_env, n_dot, res, 0, 1, "B")
@@ -315,6 +339,8 @@ def tunnel_path_block(eng, n_dot: int, res: int, flags: int, with_cpu: bool, n_e
     torch.cuda.synchronize()
     launches = eng.launch_count - l0
     ms = e0.elapsed_time(e1) / steps
+    if dump_dir:
+        dump_outputs(dump_dir, "tunnel_", z, n, res, DUMP_BYTES_TUNNEL, seed=2027)
     z_host = torch.empty(pixels, dtype=torch.float32).pin_memory().numpy()
     pin = torch.empty(scans.nbytes, dtype=torch.uint8).pin_memory()
     pin.numpy()[:] = scans.view(np.uint8)
@@ -380,7 +406,12 @@ def main():
     ap.add_argument("--path", default="A", choices=["A", "B"],
                     help="A: constant-interaction ChargeSensedDotArray path (headline); B: tunnel-coupled path of "
                          "env.step in barrier mode (secondary; use e.g. --n-dot 4 --n-env 1024)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of the last timed step's sensor images and charge occupations "
+                         "(and of the tunnel-path block's) to DIR as .npy files, 64 MB at most")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -492,6 +523,8 @@ def main():
     total_ms = max_over_ranks(ev[0].elapsed_time(ev[-1]))
     ms_per_step = total_ms / args.steps
     value = world * pixels / (ms_per_step * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, "", z_dev, n_dev, res, DUMP_BYTES_MAIN, seed=2026)
 
     # ---- parity on the timed batch itself (outside every timed region; rank 0) ----
     parity = None
@@ -655,8 +688,9 @@ def main():
         }
     # ---- (4) secondary: the tunnel-coupled path that QADAPT's env.step executes in barrier mode (Path B) ----
     if rank == 0 and world == 1 and args.path == "A" and not args.no_path_b:
-        out["env_step_tunnel_path"] = tunnel_path_block(eng, N, res, flags, not args.no_cpu_baseline,
-                                                        sm_mhz=float((clocks or {}).get("sm_mhz") or 1965.0))
+        out["env_step_tunnel_path"] = tunnel_path_block(eng, N, res, flags, not args.no_cpu_baseline, steps=args.steps,
+                                                        sm_mhz=float((clocks or {}).get("sm_mhz") or 1965.0),
+                                                        dump_dir=args.dump_outputs)
     # the one collective of the design, OFF the step path: per-env episode statistics to every rank (NCCL all-gather)
     if world > 1:
         from qdsim import parallel

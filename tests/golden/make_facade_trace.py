@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Record what the REAL reference facade passes to the drop-in classes, and what comes back (CPU container only).
 
-``QarrayBaseClass._get_obs`` (/root/reference/src/qadapt/environment/qarray_base_class.py:171-229) is imported unchanged
+``QarrayBaseClass._get_obs`` (src/qadapt/environment/qarray_base_class.py:171-229) is imported unchanged
 (tests/ref_harness.py) and driven for a few observations in BOTH modes -- barrier mode (``TunnelCoupledChargeSensed``:
 ``gate_voltage_composer.do2d('vP#', ..., add_full_crosstalk=True)`` -> ``charge_sensor_open(vg_flat, vb)``, :143-163) and
 non-barrier mode (``ChargeSensedDotArray.do2d_open``, :128-137) -- with the virtual gate matrix as the env leaves it

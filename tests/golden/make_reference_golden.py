@@ -1,10 +1,10 @@
-"""Golden vectors made by the REFERENCE ITSELF, run in this container (needs /root/reference; the fixtures travel, the
-reference does not):
+"""Golden vectors made by the REFERENCE ITSELF (needs the upstream project's ``src`` tree; the fixtures are committed,
+the reference is not):
 
-    python tests/golden/make_reference_golden.py
+    QADAPT_SRC=<upstream checkout>/src python tests/golden/make_reference_golden.py
 
 The reference's tunnel-coupled simulator (Path B, what ``env.step`` executes) is in-tree Python
-(/root/reference/src/qarray_latched/DotArrays/*.py).  It is imported unmodified through ``refshim`` (eager NumPy
+(src/qarray_latched/DotArrays/*.py).  It is imported unmodified through ``refshim`` (eager NumPy
 evaluation of its jax calls, inert shims for the absent ``qarray`` type names), constructed exactly like
 ``QarrayBaseClass._load_model_with_barriers`` does (src/qadapt/environment/qarray_base_class.py:817-838) and driven
 exactly like ``_get_charge_sensor_data`` does (:143-163): ``gate_voltage_composer.do2d('vP#', ..., gate_voltages,
@@ -170,9 +170,9 @@ def run_reference_path_a(n_dot, res, seed, pair):
         import jax.numpy as jnp
         helpers = sys.modules["qarray_latched.DotArrays._helper_functions"]
         composer_mod = sys.modules["qarray_latched.DotArrays.GateVoltageComposer"]
-        fn = _reference_functions(os.path.join(refshim.REF_SRC, "qarray_latched", "functions.py"),
+        fn = _reference_functions(os.path.join(refshim.ref_src(), "qarray_latched", "functions.py"),
                                   ["free_energy", "open_charge_configurations_jax"], {"jnp": jnp})
-        opt = _reference_functions(os.path.join(refshim.REF_SRC, "qarray_latched", "optimal_v_calc.py"),
+        opt = _reference_functions(os.path.join(refshim.ref_src(), "qarray_latched", "optimal_v_calc.py"),
                                    ["optimal_Vg", "compute_optimal_virtual_gate_matrix"],
                                    {"np": np, "CddInv": None, "Cgd_holes": None, "VectorList": None})
         cdd, cdd_inv, cgd = (np.array(a) for a in helpers.convert_to_maxwell(Cdd, Cgd))
@@ -219,7 +219,7 @@ def run_reference_virtualisation(n_env=5, n_dot=6, n_step=8, seed=31):
     import refshim
     from qdsim import synth
     rng = np.random.default_rng(seed)
-    base = os.path.join(refshim.REF_SRC, "qadapt", "capacitance_model")
+    base = os.path.join(refshim.ref_src(), "qadapt", "capacitance_model")
     out = {}
     for method, fname, cls in (("kalman", "KalmanUpdater.py", "KalmanCapacitanceUpdater"),
                                ("direct", "DirectUpdater.py", "DirectCapacitanceUpdater")):
@@ -247,7 +247,7 @@ def run_reference_virtualisation(n_env=5, n_dot=6, n_step=8, seed=31):
     # VGM update, barrier mode
     dev = synth.sample_barrier_devices(n_env, n_dot, seed=seed)
     mb = synth.tunnel_batch(dev)
-    fn = _reference_functions(os.path.join(refshim.REF_SRC, "qadapt", "environment", "qarray_base_class.py"),
+    fn = _reference_functions(os.path.join(refshim.ref_src(), "qadapt", "environment", "qarray_base_class.py"),
                               ["_update_virtual_gate_matrix", "_set_vgm_for_target_effective_coupling"], {"np": np})
     est = rng.uniform(0.0, 0.6, size=(n_env, n_dot, n_dot))
     est = 0.5 * (est + est.transpose(0, 2, 1))

@@ -1,4 +1,4 @@
-"""Test infrastructure: run the REFERENCE's own tunnel-coupled simulator (``/root/reference/src/qarray_latched``,
+"""Test infrastructure: run the REFERENCE's own tunnel-coupled simulator (``src/qarray_latched`` of the upstream project,
 unmodified, imported where it lies) in a container that has neither ``jax`` nor ``qarray``.
 
 Two stand-ins are installed into ``sys.modules`` before the reference is imported:
@@ -15,17 +15,25 @@ Two stand-ins are installed into ``sys.modules`` before the reference is importe
   in-tree reference code only -- Maxwell conversion, grid composer, relaxation, candidate selection, Hamiltonian,
   ground state, occupation expectation, sensor.
 
-Used by ``tests/golden/make_reference_golden.py`` (fixture generator) and, when ``/root/reference`` is present, by
-``tests/test_reference_golden.py::test_reference_regenerates`` .  Never imported by the product.
+Used by ``tests/golden/make_reference_golden.py`` (fixture generator) and, when ``QADAPT_SRC`` points at the upstream
+``src`` tree, by ``tests/test_reference_golden.py::test_reference_regenerates`` .  Never imported by the product.
 """
 from __future__ import annotations
 
+import os
 import sys
 import types
 
 import numpy as np
 
-REF_SRC = "/root/reference/src"
+
+def ref_src() -> str:
+    """``src`` of a checkout of the upstream project, from ``QADAPT_SRC``.  Raises when it is not set or not a directory:
+    without it the product's own drop-in ``qarray_latched`` would be the one imported."""
+    src = os.environ.get("QADAPT_SRC", "")
+    if not src or not os.path.isdir(src):
+        raise RuntimeError(f"QADAPT_SRC={src!r}: set it to the src directory of a checkout of the upstream project")
+    return os.path.abspath(src)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -243,13 +251,14 @@ class reference_modules:
             del sys.modules[k]
         sys.modules.update(make_jax())
         sys.modules.update(make_qarray())
+        src = ref_src()
         self._path = list(sys.path)
-        sys.path.insert(0, REF_SRC)
+        sys.path.insert(0, src)
         import importlib
         tccs = importlib.import_module("qarray_latched.DotArrays.TunnelCoupledChargeSensed")
         tccs = sys.modules["qarray_latched.DotArrays.TunnelCoupledChargeSensed"]
         bvm = sys.modules["qarray_latched.DotArrays.barrier_voltage_model"]
-        assert tccs.__file__.startswith(REF_SRC), tccs.__file__
+        assert os.path.abspath(tccs.__file__).startswith(src + os.sep), tccs.__file__
         return types.SimpleNamespace(TunnelCoupledChargeSensed=tccs.TunnelCoupledChargeSensed,
                                      BarrierVoltageModel=bvm.BarrierVoltageModel, tccs=tccs)
 

@@ -1,5 +1,5 @@
-"""Test-only harness: import the REAL reference facade / env from /root/reference on top of our drop-in ``qarray`` /
-``qarray_latched`` packages, in a container without a GPU.
+"""Test-only harness: import the REAL reference facade / env from the upstream ``src`` tree (``QADAPT_SRC``) on top of
+our drop-in ``qarray`` / ``qarray_latched`` packages, on a machine without a GPU.
 
 * modules the reference imports but this path never needs (jax.numpy, matplotlib, gymnasium) get tiny stand-ins;
 * the engine behind the drop-in classes is replaced by ``OracleEngine`` -- the CPU oracle answering the same calls.
@@ -14,7 +14,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference/src"
+from util import REFERENCE_SRC as REF
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "rl-agent-for-qubit-array-tuning_b200")
 

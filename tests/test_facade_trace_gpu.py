@@ -1,6 +1,6 @@
 """The reference facade's own call sequence, replayed on the CUDA engine (north_star: "src/qadapt's env ... run unchanged on
 top").  tests/golden/make_facade_trace.py recorded -- in the CPU container, with the REAL ``QarrayBaseClass._get_obs``
-(/root/reference/src/qadapt/environment/qarray_base_class.py:171-229) on top of the drop-in classes -- every constructor
+(src/qadapt/environment/qarray_base_class.py:171-229) on top of the drop-in classes -- every constructor
 kwarg, VGM assignment, ``do2d`` / ``charge_sensor_open`` / ``do2d_open`` argument and scan seed, together with the outputs of
 the CPU oracle engine.  Here the SAME drop-in classes are built from the recorded kwargs and driven with the recorded
 arguments, with ``libqdsim.so`` underneath; outputs are compared with the recorded ones.  Barrier and non-barrier mode."""

@@ -7,7 +7,9 @@ import types
 import numpy as np
 import pytest
 
-REF = "/root/reference/src/qadapt/environment/multi_agent_wrapper.py"
+from util import reference_path
+
+REF = reference_path("qadapt", "environment", "multi_agent_wrapper.py")
 
 
 def _make(n_env=5, n_dot=4, engine=None, **cfg):

@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import composer
+from util import reference_path
 
 
 def _state(n_env, n_dot, seed):
@@ -201,8 +202,8 @@ def test_agent_views_follow_the_reference_channel_and_transpose_rule():
     assert views["barrier_2"]["image"].data_ptr() == obs["image"][:, 2:3].data_ptr()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/qadapt/utils/vary_peak_width.py") and
-                    not os.path.exists("/root/reference/src/qadapt/environment/utils/vary_peak_width.py"),
+@pytest.mark.skipif(not os.path.exists(reference_path("qadapt", "utils", "vary_peak_width.py")) and
+                    not os.path.exists(reference_path("qadapt", "environment", "utils", "vary_peak_width.py")),
                     reason="reference tree not present")
 def test_variable_peak_width_matches_reference_class():
     """obs_scans(peak_width_alpha=...) against the reference's own VaryPeakWidth (utils/vary_peak_width.py), imported
@@ -210,7 +211,7 @@ def test_variable_peak_width_matches_reference_class():
     import glob
     import importlib.util
     from qdsim import obs, synth
-    path = glob.glob("/root/reference/src/qadapt/**/vary_peak_width.py", recursive=True)[0]
+    path = glob.glob(reference_path("qadapt", "**", "vary_peak_width.py"), recursive=True)[0]
     spec = importlib.util.spec_from_file_location("ref_vpw", path)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
@@ -230,7 +231,7 @@ def test_variable_peak_width_matches_reference_class():
             assert scans["peak_width"][env * (n - 1) + ch] == want
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/qadapt/environment/qarray_base_class.py"),
+@pytest.mark.skipif(not os.path.exists(reference_path("qadapt", "environment", "qarray_base_class.py")),
                     reason="reference tree not present")
 def test_radial_noise_descriptor_and_oracle_match_the_reference_method(monkeypatch):
     """S7: QarrayBaseClass._apply_radial_noise (qarray_base_class.py:444-493), compiled from the reference's source text and
@@ -240,7 +241,7 @@ def test_radial_noise_descriptor_and_oracle_match_the_reference_method(monkeypat
     import types
     from oracle import noise
     from qdsim import obs, synth
-    path = "/root/reference/src/qadapt/environment/qarray_base_class.py"
+    path = reference_path("qadapt", "environment", "qarray_base_class.py")
     tree = ast.parse(open(path).read(), filename=path)
     body = [n for n in ast.walk(tree) if isinstance(n, ast.FunctionDef) and n.name == "_apply_radial_noise"]
     ns = {"np": np}

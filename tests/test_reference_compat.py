@@ -1,5 +1,5 @@
-"""Import-surface compatibility with the REAL reference facade, when /root/reference is present (this container only;
-the GPU box does not have it).  The reference's QarrayBaseClass is imported unchanged with our ``qarray`` /
+"""Import-surface compatibility with the REAL reference facade, when ``QADAPT_SRC`` points at the upstream project's
+``src`` tree.  The reference's QarrayBaseClass is imported unchanged with our ``qarray`` /
 ``qarray_latched`` packages first on sys.path, and constructs its model through our classes.  Nothing here computes."""
 import os
 import sys
@@ -8,7 +8,7 @@ import types
 import numpy as np
 import pytest
 
-REF = "/root/reference/src"
+from util import REFERENCE_SRC as REF
 pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
 
 

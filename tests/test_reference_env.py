@@ -1,6 +1,6 @@
 """The REAL reference ``QuantumDeviceEnv`` (src/qadapt/environment/env.py) running reset() / step() UNCHANGED on top of
 our drop-in ``qarray`` / ``qarray_latched`` packages (north_star: "src/qadapt's env ... run unchanged on top").
-Only in this container (needs /root/reference); the engine is the CPU oracle here, see tests/ref_harness.py."""
+Needs the upstream ``src`` tree (``QADAPT_SRC``); the engine is the CPU oracle here, see tests/ref_harness.py."""
 import os
 
 import numpy as np
@@ -9,7 +9,7 @@ import yaml
 
 import ref_harness
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(ref_harness.REF), reason="reference tree not present")
+needs_reference = pytest.mark.skipif(not os.path.isdir(ref_harness.REF), reason="reference tree not present")
 
 
 def _config(tmp_path, num_dots=4, res=10, update_method=None):
@@ -26,6 +26,7 @@ def _config(tmp_path, num_dots=4, res=10, update_method=None):
 # update_method "fake" is bit-rotted in the reference itself for barrier models: fake_capacitance_model returns the
 # (N, N+1) model.cgd, which QarrayBaseClass._update_virtual_gate_matrix then fails to hstack (qarray_base_class.py:922);
 # "kalman" / "direct" need the CNN checkpoint.
+@needs_reference
 @pytest.mark.parametrize("update_method", [None, "perfect"])
 def test_reference_env_reset_and_step_run_unchanged(monkeypatch, tmp_path, update_method):
     base, envmod, eng = ref_harness.install(monkeypatch)
@@ -49,6 +50,7 @@ def test_reference_env_reset_and_step_run_unchanged(monkeypatch, tmp_path, updat
     assert state["virtual_gate_matrix"].shape == (5, 5) and len(state["gate_ground_truth"]) == 4
 
 
+@needs_reference
 def test_batched_env_shell_matches_the_reference_env_logic(monkeypatch, tmp_path):
     """BatchedDeviceEnv (qdsim/vector_env.py) against the REAL QuantumDeviceEnv on the same device and ranges:
     ground truth, action rescale, rewards, the scan windows it would launch, the radial-noise amplitude field."""

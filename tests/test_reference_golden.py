@@ -1,7 +1,7 @@
 """Parity against the REFERENCE ITSELF (tests/golden/ref_*.npz).
 
 The fixtures were produced by running the reference's unmodified in-tree simulator
-(/root/reference/src/qarray_latched/DotArrays: TunnelCoupledChargeSensed.charge_sensor_open -> _ground_state_open ->
+(src/qarray_latched/DotArrays: TunnelCoupledChargeSensed.charge_sensor_open -> _ground_state_open ->
 build_charge_states / hamiltonian_build / barrier_voltage_model, plus GateVoltageComposer.do2d and the Maxwell
 conversion) in this container -- see tests/golden/make_reference_golden.py and tests/golden/refshim.py.  They pin, with
 numbers that come from reference code only:
@@ -22,6 +22,7 @@ import numpy as np
 import pytest
 
 from oracle import scan as oscan
+from util import reference_path
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_CASES = ["ref_4dot_tunnel_identity_vgm", "ref_4dot_tunnel_perfect_vgm_cbb", "ref_5dot_tunnel_low_occupancy",
@@ -117,10 +118,10 @@ def test_oracle_matches_reference(name):
         assert np.abs(d["n"] - np.rint(d["n"])).max() > 1e-2      # the fixture exercises real tunnel mixing
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/qarray_latched"), reason="reference tree not present")
+@pytest.mark.skipif(not os.path.isdir(reference_path("qarray_latched")), reason="reference tree not present")
 def test_reference_regenerates_fixture():
     """The committed fixtures are what the reference produces today (guards against stale or hand-edited files): one of
-    each family is regenerated from /root/reference and compared."""
+    each family is regenerated from the upstream ``src`` tree (``QADAPT_SRC``) and compared."""
     import sys
     sys.path.insert(0, os.path.join(HERE, "golden"))
     import make_reference_golden as gen

@@ -8,7 +8,9 @@ import types
 import numpy as np
 import pytest
 
-REF = "/root/reference/src/qadapt/environment/multi_agent_wrapper.py"
+from util import reference_path
+
+REF = reference_path("qadapt", "environment", "multi_agent_wrapper.py")
 
 
 def _reference_methods(names):

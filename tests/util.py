@@ -2,9 +2,20 @@
 Model / Scan objects so both sides see the same numbers."""
 from __future__ import annotations
 
+import os
+
 import numpy as np
 
 from oracle import scan as oscan
+
+# ``src`` of a checkout of the upstream project (edwindn/rl-agent-for-qubit-array-tuning).  The tests that run its own code
+# next to ours skip when ``QADAPT_SRC`` does not point at one.
+REFERENCE_SRC = os.environ.get("QADAPT_SRC", "")
+
+
+def reference_path(*parts: str) -> str:
+    """``parts`` under the upstream ``src`` tree, or "" (which exists nowhere) when ``QADAPT_SRC`` is not set."""
+    return os.path.join(REFERENCE_SRC, *parts) if REFERENCE_SRC else ""
 
 
 def oracle_model(mb, e: int, flags: int = 0):
