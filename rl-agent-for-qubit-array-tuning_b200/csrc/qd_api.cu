@@ -376,7 +376,7 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
           ctx->launches += 1;
         }
         // fix-up launches: items of 8 pixels (no state is carried between marked pixels), so that a stretch of marked pixels
-        // is spread over several warps; col_parts carries the marking kernel's item length to the mark look-up
+        // is spread over several warps; mark_ppi carries the marking kernel's item length to the mark look-up
         const int fix_ppi = (ppi % 8 == 0) ? 8 : (int)ppi;          // (must divide the marking kernel's item length)
         const int fix_ips = (int)((max_pix + fix_ppi - 1) / fix_ppi);
         long long fix_grid = ((long long)nc * fix_ips + gw - 1) / gw;
@@ -386,8 +386,8 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
           qd::KArgs sa = g;
           long long sgrid = ggrid;
           if (ks2) {
-            sa.topt |= 16;
-            sa.col_parts = (int)ppi;
+            sa.fixup = 1;
+            sa.mark_ppi = (int)ppi;
             sa.rows_per_item = fix_ppi;
             sa.items_per_scan = fix_ips;
             sgrid = fix_grid;
@@ -423,13 +423,11 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
           qd::KArgs ea = g;
           long long egrid = ggrid;
           if (!householder_only) {
-            ea.topt |= 8;
-            ea.col_parts = (int)ppi;
+            ea.fixup = 1;
+            ea.mark_ppi = (int)ppi;
             ea.rows_per_item = fix_ppi;
             ea.items_per_scan = fix_ips;
             egrid = fix_grid;
-          } else {
-            ea.topt &= ~8;
           }
           ea.slot_bytes = qd::qd_tunnel_eigen_slot_bytes(ctx->L);
           const size_t smem = (size_t)ea.slot_bytes * gw;

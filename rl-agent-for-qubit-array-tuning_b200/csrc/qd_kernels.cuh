@@ -43,6 +43,10 @@ struct KArgs {
   double* tpot;                        // [slots][16]  dot potentials g[0..8), tunnel couplings |t|[8..15), cdd scale s_c [15]
   long long tstride;                   // pixels per scan slot (largest scan of the upload)
   int topt;                            // tunnel path: optimisation switches (QDSIM_TUNNEL_OPT, default all on; A/B and bisection)
+  // tunnel path, select / eigen kernels: a fix-up launch redoes only the pixels the marking kernel (select2 / eigen2)
+  // marked; its items are shorter than the marking kernel's, whose item length (pixels) locates the item-level marks
+  int fixup;
+  int mark_ppi;
   float e2_kappa, e2_qsafe, e2_tol;    // qd_tunnel_eigen2_kernel: shift aggressiveness, contraction safety factor, stopping tolerance
   // single-scan fast path (one do2d_open): the descriptor travels in the kernel parameters instead of through a
   // host-to-device copy; `scans` is then unused
@@ -677,6 +681,171 @@ __device__ __forceinline__ uint64_t pack_key(const double (&nd)[N], bool integra
   return k;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Stages shared by the scan kernels (qd_scan_kernel, qd_scan_fast_kernel; the staging also by the tunnel kernels).
+// ---------------------------------------------------------------------------------------------------------------
+
+// Stage the head of the env record (`rec_bytes`) and the scan descriptor into the warp's slot: lane 0 issues two TMA bulk
+// copies on one mbarrier, the warp waits and flips the phase.  use_one: the one descriptor of a single-scan call sits in
+// the kernel parameters -- the lanes copy it and TMA brings the record alone.
+__device__ __forceinline__ void stage_item(const KArgs& a, const qd_scan* gscan, uint32_t rec_bytes, double* rec, qd_scan* sc,
+                                           uint64_t* bar, uint32_t& phase, int lane, bool use_one = false) {
+  if (use_one) {
+    if (lane == 0) {
+      fence_proxy_async();
+      mbar_expect_tx(bar, rec_bytes);
+      tma_bulk_g2s(rec, a.records + (size_t)a.one.env_id * a.L.rec_doubles, rec_bytes, bar);
+    }
+    const double* src = reinterpret_cast<const double*>(&a.one);
+    double* dst = reinterpret_cast<double*>(sc);
+    for (int i = lane; i < (int)(sizeof(qd_scan) / 8); i += 32) dst[i] = src[i];
+    __syncwarp();
+  } else if (lane == 0) {
+    const int env = gscan->env_id;
+    fence_proxy_async();
+    mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
+    tma_bulk_g2s(rec, a.records + (size_t)env * a.L.rec_doubles, rec_bytes, bar);
+    tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
+  }
+  mbar_wait(bar, phase);
+  phase ^= 1u;
+}
+
+// Rows [row0, row1) and columns [cx0, cx1) of item `part` of an nx x ny scan: a block of rows_per_item rows, split along x
+// into col_parts ranges of whole 32-pixel chunks.
+struct ItemWindow {
+  int row0, row1, cx0, cx1;
+  bool empty;
+};
+__device__ __forceinline__ ItemWindow item_window(const KArgs& a, int part, int nx, int ny) {
+  const int cparts = a.col_parts > 1 ? a.col_parts : 1;
+  const int rpart = part / cparts, cpart = part - rpart * cparts;
+  ItemWindow w;
+  w.row0 = rpart * a.rows_per_item;
+  w.row1 = min(ny, w.row0 + a.rows_per_item);
+  const int n_chunk_x = (nx + 31) >> 5;
+  w.cx0 = ((n_chunk_x * cpart) / cparts) << 5;
+  w.cx1 = min(nx, ((n_chunk_x * (cpart + 1)) / cparts) << 5);
+  w.empty = w.row0 >= ny || w.cx0 >= w.cx1;
+  return w;
+}
+
+// Per-item affine forms of the dot potentials (der[0..8) g0, [8..16) gx, [16..24) gy) and of the sensor potential
+// (der[24..27) us0, usx, usy) on an affine scan window, one lane per row of cgd (lanes 0..N).
+// Occupations are bounded by the largest dot potential of the window (+1 for the ceil candidate, +2 on the tunnel path;
+// the relaxed occupations never exceed max(g, 0) on an M-matrix).  uint8 charge maps and the packed latching keys hold
+// 0..255: windows that could leave that range are flagged instead of saturating silently.  check_overflow = false for
+// brute force, whose occupations are bounded by max_charge_carriers instead.
+template <int N>
+__device__ __forceinline__ void item_affine_forms(const KArgs& a, const double* rec, const qd_scan* sc, double* der, int lane,
+                                                  bool check_overflow = true) {
+  const qd_layout& L = a.L;
+  const int NV = L.n_volt;
+  if (lane <= N) {
+    const double* arow = (lane < N) ? rec + L.o_a + lane * NV : rec + L.o_sa;
+    double s0 = 0.0, sx = 0.0, sy = 0.0;
+    for (int k = 0; k < NV; ++k) {
+      const double c = arow[k];
+      s0 = fma(c, sc->v0[k], s0);
+      sx = fma(c, sc->dx[k], sx);
+      sy = fma(c, sc->dy[k], sy);
+    }
+    if (lane < N) {
+      der[lane] = s0; der[8 + lane] = sx; der[16 + lane] = sy;
+      const double gmax = s0 + fmax(sx * (double)(sc->nx - 1), 0.0) + fmax(sy * (double)(sc->ny - 1), 0.0);
+      const bool replaced = (a.flags & QD_FLAG_RADIAL) && sc->rad_mode == 2;      // no occupations are computed there
+      if (check_overflow && !replaced && !(gmax < 252.0) && a.status)
+        *reinterpret_cast<volatile unsigned*>(a.status) = QD_STATUS_OCC_OVERFLOW;
+    } else { der[24] = s0; der[25] = sx; der[26] = sy; }
+  }
+}
+
+// The random draws of a pixel: one Philox4x32-10 block (purpose 0, counter = pixel index) -> Box-Muller pair (white,
+// radial), latching uniform, telegraph uniform.  All zero when nothing random is on.
+struct PixelDraws {
+  float z_white, z_rad, u_latch, u_tele;
+};
+__device__ __forceinline__ PixelDraws pixel_draws(bool need_rng, uint64_t seed, long long pix) {
+  PixelDraws d = {0.f, 0.f, 0.f, 0.f};
+  if (need_rng) {
+    const Philox4 w = philox4x32_10(seed, (uint64_t)pix, 0u);
+    box_muller(w.w0, w.w1, d.z_white, d.z_rad);
+    d.u_latch = u24(w.w2);
+    d.u_tele = u24(w.w3);
+  }
+  return d;
+}
+
+// Hysteresis latching of one 32-pixel chunk along x, on packed keys (8 bits per dot), from the held configuration
+// `held_key`; `todo` = the lanes still to resolve.  Loops over events only: the first lane whose key differs from the
+// held one, the differing dots classified by a byte-nonzero mask, p_leads / p_inter looked up.  The lanes from there on
+// that want the same new configuration form a run; every one of them faces the same (held -> new) transition, so the
+// first of them whose uniform is below p accepts and the ones before it stay latched to the held configuration.
+// take_held(i, rejected, acc) runs on every lane once per event, while held_key is still the configuration held so far
+// (i: first differing lane, rejected: lanes that keep the held configuration, acc: accepting lane, 32 if none): it moves
+// whatever else travels with the configuration.
+template <typename TakeHeld>
+__device__ __forceinline__ void latch_chunk(uint64_t& key, uint64_t& held_key, unsigned todo, float u_latch, const double* rec,
+                                            const qd_layout& L, int lane, TakeHeld&& take_held) {
+  while (true) {
+    const unsigned diff = __ballot_sync(0xffffffffu, key != held_key) & todo;
+    if (!diff) break;
+    const int i = __ffs(diff) - 1;
+    const uint64_t ck = shfl_u64(key, i);
+    const uint64_t x = ck ^ held_key;
+    const uint64_t nz = (((x & 0x7f7f7f7f7f7f7f7fULL) + 0x7f7f7f7f7f7f7f7fULL) | x) & 0x8080808080808080ULL;
+    const int ndiff = __popcll(nz);
+    double p_acc = 2.0;                            // > every uniform: accept
+    if (ndiff == 1) {
+      p_acc = rec[L.o_pleads + ((__ffsll((long long)nz) - 1) >> 3)];
+    } else if (ndiff == 2) {
+      const int d0 = (__ffsll((long long)nz) - 1) >> 3;
+      const int d1 = (63 - __clzll((long long)nz)) >> 3;
+      p_acc = rec[L.o_pinter + d0 * 8 + d1];
+    }
+    const unsigned from_i = ~((1u << i) - 1u);
+    const unsigned same = __ballot_sync(0xffffffffu, key == ck) & todo & from_i;
+    const unsigned brk = ~same & from_i & todo;
+    const unsigned run = same & ~(brk ? (~0u << (__ffs(brk) - 1)) : 0u);
+    const unsigned acc = __ballot_sync(0xffffffffu, (double)u_latch < p_acc) & run;
+    const int acl = acc ? __ffs(acc) - 1 : 32;
+    const unsigned rejected = run & ((acl >= 32) ? ~0u : ((1u << acl) - 1u));
+    if ((rejected >> lane) & 1u) key = held_key;
+    take_held(i, rejected, acl);
+    if (acl < 32) held_key = ck;
+    const int done_to = (acl < 32) ? acl : (31 - __clz(run));
+    todo &= ~((2u << done_to) - 1u);
+  }
+}
+
+// Telegraph state at the start of row iy: the stationary draw (Philox purpose 1), or state 0 on a flat pass, where the
+// chain runs on from row to row.
+__device__ __forceinline__ uint32_t tele_start(bool f_carry, uint64_t seed, int iy, const double* par) {
+  if (f_carry) return 0u;
+  const Philox4 wr = philox4x32_10(seed, (uint64_t)iy, 1u);
+  return ((double)u24(wr.w0) < par[QD_PAR_TELE_STAT]) ? 1u : 0u;
+}
+
+// Sensor: ten fp32 Lorentzians of the first differences of the free energy, x_k = x0 + k xs for k = -5..4.
+__device__ __forceinline__ float sensor_lorentz10(double x0, double xs) {
+  float zs = 0.f;
+#pragma unroll
+  for (int k = -5; k < 5; ++k) {
+    const float xk = (float)fma((double)k, xs, x0);
+    zs += rcp_approx(fmaf(xk, xk, 1.0f));
+  }
+  return zs;
+}
+
+// Amplitude of the radial noise at pixel (fx, fy) (rad_mode 1): rad_alpha * (|v| - rad_zero_radius) clamped to
+// [0, rad_max_amp], v = the pixel's voltage offset rad_x0 + fx rad_dx, rad_y0 + fy rad_dy.
+__device__ __forceinline__ float radial_amp(const qd_scan* sc, double fx, double fy) {
+  const float vx = (float)fma(fx, sc->rad_dx, sc->rad_x0);
+  const float vy = (float)fma(fy, sc->rad_dy, sc->rad_y0);
+  const float dist = sqrtf(fmaf(vx, vx, vy * vy));
+  return fminf(fmaxf((float)sc->rad_alpha * (dist - (float)sc->rad_zero_radius), 0.0f), (float)sc->rad_max_amp);
+}
+
 // THERMAL = false instantiations carry no Boltzmann-average code at all (the hard-argmin kernels are the hot ones; the
 // launch picks THERMAL = true only when QD_FLAG_THERMAL is set).
 // POINTS = true: explicit voltage list (a.points) instead of the affine descriptor -- the single-device entry points.
@@ -732,65 +901,17 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
     const int part = (int)(item - (long long)scan_id * a.items_per_scan);
     const qd_scan* gscan = a.scans + scan_id;
 
-    // ---- stage record + scan descriptor (TMA bulk, one mbarrier) ----
-    if (a.use_one) {
-      // the one descriptor of a single-scan call sits in the kernel parameters: lanes copy it, TMA brings the record
-      if (lane == 0) {
-        fence_proxy_async();
-        mbar_expect_tx(bar, rec_bytes);
-        tma_bulk_g2s(rec, a.records + (size_t)a.one.env_id * L.rec_doubles, rec_bytes, bar);
-      }
-      const double* src = reinterpret_cast<const double*>(&a.one);
-      double* dst = reinterpret_cast<double*>(sc);
-      for (int i = lane; i < (int)(sizeof(qd_scan) / 8); i += 32) dst[i] = src[i];
-      __syncwarp();
-    } else if (lane == 0) {
-      const int env = gscan->env_id;
-      fence_proxy_async();
-      mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
-      tma_bulk_g2s(rec, a.records + (size_t)env * L.rec_doubles, rec_bytes, bar);
-      tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1u;
+    stage_item(a, gscan, rec_bytes, rec, sc, bar, phase, lane, a.use_one);
     if constexpr (ALG == QD_ALG_DEFAULT) {
       if (lane == 0) { pc.meta[0] = 0u; pc.meta[1] = 0u; }    // the projection cache belongs to one env
     }
 
     const int nx = sc->nx, ny = sc->ny;
-    const int cparts = a.col_parts > 1 ? a.col_parts : 1;
-    const int rpart = part / cparts, cpart = part - rpart * cparts;
-    const int row0 = rpart * a.rows_per_item;
-    const int row1 = min(ny, row0 + a.rows_per_item);
-    // column range of this item: whole 32-pixel chunks, split evenly over the column parts
-    const int n_chunk_x = (nx + 31) >> 5;
-    const int cx0 = ((n_chunk_x * cpart) / cparts) << 5, cx1 = min(nx, ((n_chunk_x * (cpart + 1)) / cparts) << 5);
-    if (row0 >= ny || cx0 >= cx1) { __syncwarp(); continue; }
+    const ItemWindow w = item_window(a, part, nx, ny);
+    if (w.empty) { __syncwarp(); continue; }
+    const int row0 = w.row0, row1 = w.row1, cx0 = w.cx0, cx1 = w.cx1;
 
-    // ---- affine coefficients of the dot potentials and of the sensor potential ----
-    if constexpr (!POINTS) {
-      if (lane <= N) {
-        const double* arow = (lane < N) ? rec + L.o_a + lane * NV : rec + L.o_sa;
-        double s0 = 0.0, sx = 0.0, sy = 0.0;
-        for (int k = 0; k < NV; ++k) {
-          const double c = arow[k];
-          s0 = fma(c, sc->v0[k], s0);
-          sx = fma(c, sc->dx[k], sx);
-          sy = fma(c, sc->dy[k], sy);
-        }
-        if (lane < N) {
-          d_g0[lane] = s0; d_gx[lane] = sx; d_gy[lane] = sy;
-          // Occupations are bounded by the largest dot potential of the window (+1 for the ceil candidate, +2 on the
-          // tunnel path; the relaxed occupations never exceed max(g, 0) on an M-matrix).  uint8 charge maps and the
-          // packed latching keys hold 0..255: flag windows that could leave that range instead of saturating silently.
-          const double gmax = s0 + fmax(sx * (double)(sc->nx - 1), 0.0) + fmax(sy * (double)(sc->ny - 1), 0.0);
-          const bool replaced = (a.flags & QD_FLAG_RADIAL) && sc->rad_mode == 2;      // no occupations are computed there
-          if (ALG != QD_ALG_BRUTE_FORCE && !replaced && !(gmax < 252.0) && a.status)
-            *reinterpret_cast<volatile unsigned*>(a.status) = QD_STATUS_OCC_OVERFLOW;
-        }
-        else { d_us[0] = s0; d_us[1] = sx; d_us[2] = sy; }
-      }
-    }
+    if constexpr (!POINTS) item_affine_forms<N>(a, rec, sc, der, lane, ALG != QD_ALG_BRUTE_FORCE);
     __syncwarp();
     if constexpr (ALG == QD_ALG_BRUTE_FORCE) {
       // ---- tree order of this item (most negative potential at the item's centre first) and cdd_inv = U D U^T in it ----
@@ -857,15 +978,7 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
         const int ixc = valid ? ix : nx - 1;
         const long long pix = (long long)iy * nx + ixc;
         const unsigned vmask = __ballot_sync(0xffffffffu, valid);
-
-        // ---- random draws of this pixel ----
-        float z_white = 0.f, z_rad = 0.f, u_latch = 0.f, u_tele = 0.f;
-        if (need_rng) {
-          const Philox4 w = philox4x32_10(seed, (uint64_t)pix, 0u);
-          box_muller(w.w0, w.w1, z_white, z_rad);
-          u_latch = u24(w.w2);
-          u_tele = u24(w.w3);
-        }
+        const PixelDraws rnd = pixel_draws(need_rng, seed, pix);
 
         double nd[N];
         double g[N];
@@ -930,47 +1043,18 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
               todo &= ~1u;
               have_held = true;
             }
-            while (true) {
-              const unsigned diff = __ballot_sync(0xffffffffu, key != held_key) & todo;
-              if (!diff) break;
-              const int i = __ffs(diff) - 1;                 // first pixel whose ground state differs from the held one
-              const uint64_t ck = shfl_u64(key, i);
-              const uint64_t x = ck ^ held_key;
-              const uint64_t nz = (((x & 0x7f7f7f7f7f7f7f7fULL) + 0x7f7f7f7f7f7f7f7fULL) | x) & 0x8080808080808080ULL;
-              const int ndiff = __popcll(nz);
-              double p_acc = 2.0;                            // > every uniform: accept
-              if (ndiff == 1) {
-                p_acc = rec[L.o_pleads + ((__ffsll((long long)nz) - 1) >> 3)];
-              } else if (ndiff == 2) {
-                const int d0 = (__ffsll((long long)nz) - 1) >> 3;
-                const int d1 = (63 - __clzll((long long)nz)) >> 3;
-                p_acc = rec[L.o_pinter + d0 * 8 + d1];
-              }
-              // The pixels from i on that want the same new configuration form a run; every one of them faces the same
-              // (held -> ck) transition, so the first of them whose uniform is below p_acc accepts and the ones before
-              // it stay latched to the held configuration.
-              const unsigned from_i = ~((1u << i) - 1u);
-              const unsigned same = __ballot_sync(0xffffffffu, key == ck) & todo & from_i;
-              const unsigned run = same & ~((~same & from_i & todo) ? (~0u << (__ffs(~same & from_i & todo) - 1)) : 0u);
-              const unsigned acc = __ballot_sync(0xffffffffu, (double)u_latch < p_acc) & run;
-              const int a = acc ? __ffs(acc) - 1 : 32;       // accepting pixel (32: nobody in this run)
-              const unsigned rejected = run & ((a >= 32) ? ~0u : ((1u << a) - 1u));
-              if (rejected) {
-                if (!integral) {
-                  const int src = (i > 0) ? i - 1 : 0;
+            // a rejected pixel takes the occupations of lane i - 1 (the held configuration), or the carry of the last chunk
+            latch_chunk(key, held_key, todo, rnd.u_latch, rec, L, lane, [&](int i, unsigned rejected, int) {
+              if (rejected && !integral) {
+                const int src = (i > 0) ? i - 1 : 0;
 #pragma unroll
-                  for (int j = 0; j < N; ++j) {
-                    const double prev = shfl_f64(nd[j], src);
-                    const double held = (i > 0) ? prev : d_carry[j];
-                    if ((rejected >> lane) & 1u) nd[j] = held;
-                  }
+                for (int j = 0; j < N; ++j) {
+                  const double prev = shfl_f64(nd[j], src);
+                  const double held = (i > 0) ? prev : d_carry[j];
+                  if ((rejected >> lane) & 1u) nd[j] = held;
                 }
-                if ((rejected >> lane) & 1u) key = held_key;
               }
-              if (a < 32) held_key = ck;
-              const int done_to = (a < 32) ? a : (31 - __clz(run));
-              todo &= ~((2u << done_to) - 1u);
-            }
+            });
             if (integral) {
               if (key != key_free) {
 #pragma unroll
@@ -990,20 +1074,16 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
           // ---- sensor input noise: white + telegraph ----
           double noise_in = 0.0, noise_out = 0.0;
           if (f_noise) {
-            const double wn = par[QD_PAR_WHITE] * (double)z_white;
+            const double wn = par[QD_PAR_WHITE] * (double)rnd.z_white;
             if (f_white_out) noise_out = wn; else noise_in = wn;
             const double tamp = par[QD_PAR_TELE_AMP];
             if (tamp != 0.0) {
               if (!tele_init) {
-                if (f_carry) tele_state = 0u;
-                else {
-                  const Philox4 wr = philox4x32_10(seed, (uint64_t)iy, 1u);
-                  tele_state = ((double)u24(wr.w0) < par[QD_PAR_TELE_STAT]) ? 1u : 0u;
-                }
+                tele_state = tele_start(f_carry, seed, iy, par);
                 tele_init = true;
               }
-              const uint32_t flip0 = ((double)u_tele < par[QD_PAR_P01]) ? 1u : 0u;
-              const uint32_t flip1 = ((double)u_tele < par[QD_PAR_P10]) ? 1u : 0u;
+              const uint32_t flip0 = ((double)rnd.u_tele < par[QD_PAR_P01]) ? 1u : 0u;
+              const uint32_t flip1 = ((double)rnd.u_tele < par[QD_PAR_P10]) ? 1u : 0u;
               uint32_t fn = valid ? ((0u ^ flip0) | ((1u ^ flip1) << 1)) : 2u;   // invalid lanes: identity
 #pragma unroll
               for (int d = 1; d < 32; d <<= 1) {
@@ -1086,25 +1166,12 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
             }
             z = zs + noise_out;
           } else {
-            float zs = 0.f;
-#pragma unroll
-            for (int k = -5; k < 5; ++k) {
-              const float xk = (float)fma((double)k, xs, x0);
-              zs += rcp_approx(fmaf(xk, xk, 1.0f));
-            }
-            z = (double)zs + noise_out;
+            z = (double)sensor_lorentz10(x0, xs) + noise_out;
           }
-          if (f_radial && sc->rad_mode == 1) {
-            const float vx = (float)fma((double)ixc, sc->rad_dx, sc->rad_x0);
-            const float vy = (float)fma((double)iy, sc->rad_dy, sc->rad_y0);
-            const float dist = sqrtf(fmaf(vx, vx, vy * vy));
-            const float amp = fminf(fmaxf((float)sc->rad_alpha * (dist - (float)sc->rad_zero_radius), 0.0f),
-                                    (float)sc->rad_max_amp);
-            z = fma((double)z_rad, (double)amp, z);
-          }
+          if (f_radial && sc->rad_mode == 1) z = fma((double)rnd.z_rad, (double)radial_amp(sc, (double)ixc, (double)iy), z);
           zf = (float)z;
         } else {
-          zf = z_rad;
+          zf = rnd.z_rad;
 #pragma unroll
           for (int j = 0; j < N; ++j) nd[j] = 0.0;
         }
@@ -1151,8 +1218,8 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
 
 // ---------------------------------------------------------------------------------------------------------------
 // The HOT instantiation: default / thresholded search, hard argmin (kT = 0), affine scan windows -- config 4's kernel.
-// Same arithmetic as qd_scan_kernel<N, QD_ALG_DEFAULT, false, false> (the parity tests run both), restructured so that a
-// pixel never holds its occupations as doubles:
+// Same arithmetic as qd_scan_kernel<N, QD_ALG_DEFAULT, false, false> (the parity tests run both; the stages above are
+// shared), restructured so that a pixel never holds its occupations as doubles:
 //   * floor(n_c) is packed straight into the 8-bit-per-dot key the latching pass works on; the argmin adds its bits with
 //     one multiply (bit N-1-j -> byte j), and for N = 8 the uint8 charge map IS that key, stored with one STG.64;
 //   * the sensor's dot term sum_j w_j (n_j - g_j) splits into SN = sum_j w_j n_j, which travels with the key through the
@@ -1182,7 +1249,6 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
   const int warp = threadIdx.x >> 5;
   const int warps_per_cta = blockDim.x >> 5;
   const qd_layout& L = a.L;
-  const int NV = L.n_volt;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
   double* rec = reinterpret_cast<double*>(slot);
@@ -1230,58 +1296,16 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
     const int part = (int)(item - (long long)scan_id * a.items_per_scan);
     const qd_scan* gscan = a.scans + scan_id;
 
-    // ---- stage record + scan descriptor (TMA bulk, one mbarrier) ----
-    if (a.use_one) {
-      // the one descriptor of a single-scan call sits in the kernel parameters: lanes copy it, TMA brings the record
-      if (lane == 0) {
-        fence_proxy_async();
-        mbar_expect_tx(bar, rec_bytes);
-        tma_bulk_g2s(rec, a.records + (size_t)a.one.env_id * L.rec_doubles, rec_bytes, bar);
-      }
-      const double* src = reinterpret_cast<const double*>(&a.one);
-      double* dst = reinterpret_cast<double*>(sc);
-      for (int i = lane; i < (int)(sizeof(qd_scan) / 8); i += 32) dst[i] = src[i];
-      __syncwarp();
-    } else if (lane == 0) {
-      const int env = gscan->env_id;
-      fence_proxy_async();
-      mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
-      tma_bulk_g2s(rec, a.records + (size_t)env * L.rec_doubles, rec_bytes, bar);
-      tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1u;
+    stage_item(a, gscan, rec_bytes, rec, sc, bar, phase, lane, a.use_one);
     if (lane == 0) { pc.meta[0] = 0u; pc.meta[1] = 0u; }      // the projection cache belongs to one (env, window)
 
     const int nx = sc->nx, ny = sc->ny;
-    const int cparts = a.col_parts > 1 ? a.col_parts : 1;
-    const int rpart = part / cparts, cpart = part - rpart * cparts;
-    const int row0 = rpart * a.rows_per_item;
-    const int row1 = min(ny, row0 + a.rows_per_item);
-    // column range of this item: whole 32-pixel chunks, split evenly over the column parts
-    const int n_chunk_x = (nx + 31) >> 5;
-    const int cx0 = ((n_chunk_x * cpart) / cparts) << 5, cx1 = min(nx, ((n_chunk_x * (cpart + 1)) / cparts) << 5);
-    if (row0 >= ny || cx0 >= cx1) { __syncwarp(); continue; }
+    const ItemWindow w = item_window(a, part, nx, ny);
+    if (w.empty) { __syncwarp(); continue; }
+    const int row0 = w.row0, row1 = w.row1, cx0 = w.cx0, cx1 = w.cx1;
 
     // ---- per-item affine forms: dot potentials, sensor potential, sum_j w_j g_j; the two nibble tables of w ----
-    if (lane <= N) {
-      const double* arow = (lane < N) ? rec + L.o_a + lane * NV : rec + L.o_sa;
-      double s0 = 0.0, sx = 0.0, sy = 0.0;
-      for (int k = 0; k < NV; ++k) {
-        const double c = arow[k];
-        s0 = fma(c, sc->v0[k], s0);
-        sx = fma(c, sc->dx[k], sx);
-        sy = fma(c, sc->dy[k], sy);
-      }
-      if (lane < N) {
-        d_g0[lane] = s0; d_gx[lane] = sx; d_gy[lane] = sy;
-        // occupations <= largest dot potential of the window + 1 (qd_scan_kernel has the argument): flag windows that
-        // could leave the 0..255 range of the key bytes instead of saturating silently
-        const double gmax = s0 + fmax(sx * (double)(nx - 1), 0.0) + fmax(sy * (double)(ny - 1), 0.0);
-        const bool replaced = (a.flags & QD_FLAG_RADIAL) && sc->rad_mode == 2;        // no occupations are computed there
-        if (!replaced && !(gmax < 252.0) && a.status) *reinterpret_cast<volatile unsigned*>(a.status) = QD_STATUS_OCC_OVERFLOW;
-      } else { d_us[0] = s0; d_us[1] = sx; d_us[2] = sy; }
-    }
+    item_affine_forms<N>(a, rec, sc, der, lane);
     {
       double t = 0.0;
       const int h = lane & 15;
@@ -1323,15 +1347,7 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
         const long long pix = (long long)iy * nx + ixc;
         const unsigned vmask = __ballot_sync(0xffffffffu, valid);
         const double fx = (double)ixc, fy = (double)iy;
-
-        // ---- random draws of this pixel ----
-        float z_white = 0.f, z_rad = 0.f, u_latch = 0.f, u_tele = 0.f;
-        if (need_rng) {
-          const Philox4 w = philox4x32_10(seed, (uint64_t)pix, 0u);
-          box_muller(w.w0, w.w1, z_white, z_rad);
-          u_latch = u24(w.w2);
-          u_tele = u24(w.w3);
-        }
+        const PixelDraws rnd = pixel_draws(need_rng, seed, pix);
 
         uint64_t key = 0;
         float zf;
@@ -1431,54 +1447,26 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
               todo &= ~1u;
               have_held = true;
             }
-            while (true) {
-              const unsigned diff = __ballot_sync(0xffffffffu, key != held_key) & todo;
-              if (!diff) break;
-              const int i = __ffs(diff) - 1;                 // first pixel whose ground state differs from the held one
-              const uint64_t ck = shfl_u64(key, i);
-              const uint64_t x = ck ^ held_key;
-              const uint64_t nz = (((x & 0x7f7f7f7f7f7f7f7fULL) + 0x7f7f7f7f7f7f7f7fULL) | x) & 0x8080808080808080ULL;
-              const int ndiff = __popcll(nz);
-              double p_acc = 2.0;                            // > every uniform: accept
-              if (ndiff == 1) {
-                p_acc = rec[L.o_pleads + ((__ffsll((long long)nz) - 1) >> 3)];
-              } else if (ndiff == 2) {
-                const int d0 = (__ffsll((long long)nz) - 1) >> 3;
-                const int d1 = (63 - __clzll((long long)nz)) >> 3;
-                p_acc = rec[L.o_pinter + d0 * 8 + d1];
-              }
-              const unsigned from_i = ~((1u << i) - 1u);
-              const unsigned same = __ballot_sync(0xffffffffu, key == ck) & todo & from_i;
-              const unsigned brk = ~same & from_i & todo;
-              const unsigned run = same & ~(brk ? (~0u << (__ffs(brk) - 1)) : 0u);
-              const unsigned acc = __ballot_sync(0xffffffffu, (double)u_latch < p_acc) & run;
-              const int acl = acc ? __ffs(acc) - 1 : 32;     // accepting pixel (32: nobody in this run)
-              const unsigned rejected = run & ((acl >= 32) ? ~0u : ((1u << acl) - 1u));
-              if ((rejected >> lane) & 1u) { key = held_key; sn = held_sn; }
-              if (acl < 32) { held_key = ck; held_sn = shfl_f64(sn, acl); }
-              const int done_to = (acl < 32) ? acl : (31 - __clz(run));
-              todo &= ~((2u << done_to) - 1u);
-            }
+            latch_chunk(key, held_key, todo, rnd.u_latch, rec, L, lane, [&](int, unsigned rejected, int acl) {
+              if ((rejected >> lane) & 1u) sn = held_sn;
+              if (acl < 32) held_sn = shfl_f64(sn, acl);
+            });
           }
 
           // ---- sensor input noise: white + telegraph ----
           double noise_in = 0.0, noise_out = 0.0;
           if (f_noise) {
-            const double wn = par[QD_PAR_WHITE] * (double)z_white;
+            const double wn = par[QD_PAR_WHITE] * (double)rnd.z_white;
             if (f_white_out) noise_out = wn; else noise_in = wn;
             const double tamp = par[QD_PAR_TELE_AMP];
             if (tamp != 0.0) {
               if (!tele_init) {
-                if (f_carry) tele_state = 0u;
-                else {
-                  const Philox4 wr = philox4x32_10(seed, (uint64_t)iy, 1u);
-                  tele_state = ((double)u24(wr.w0) < par[QD_PAR_TELE_STAT]) ? 1u : 0u;
-                }
+                tele_state = tele_start(f_carry, seed, iy, par);
                 tele_init = true;
               }
               // lanes that flip when they are reached in state 0 / in state 1
-              const unsigned f0 = __ballot_sync(0xffffffffu, valid && (double)u_tele < par[QD_PAR_P01]);
-              const unsigned f1 = __ballot_sync(0xffffffffu, valid && (double)u_tele < par[QD_PAR_P10]);
+              const unsigned f0 = __ballot_sync(0xffffffffu, valid && (double)rnd.u_tele < par[QD_PAR_P01]);
+              const unsigned f1 = __ballot_sync(0xffffffffu, valid && (double)rnd.u_tele < par[QD_PAR_P10]);
               unsigned st_mask = 0u, rem = 0xffffffffu, cur = tele_state;
               while (true) {
                 const unsigned m = (cur ? f1 : f0) & rem;
@@ -1502,24 +1490,11 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
           const double t = (rint(us) + noise_in) - us;
           const double xs = 2.0 * css * inv_gamma;
           const double x0 = fma(css, fma(2.0, t, 1.0), base) * inv_gamma;
-          float zs = 0.f;
-#pragma unroll
-          for (int k = -5; k < 5; ++k) {
-            const float xk = (float)fma((double)k, xs, x0);
-            zs += rcp_approx(fmaf(xk, xk, 1.0f));
-          }
-          double z = (double)zs + noise_out;
-          if (f_radial && sc->rad_mode == 1) {
-            const float vx = (float)fma(fx, sc->rad_dx, sc->rad_x0);
-            const float vy = (float)fma(fy, sc->rad_dy, sc->rad_y0);
-            const float dist = sqrtf(fmaf(vx, vx, vy * vy));
-            const float amp = fminf(fmaxf((float)sc->rad_alpha * (dist - (float)sc->rad_zero_radius), 0.0f),
-                                    (float)sc->rad_max_amp);
-            z = fma((double)z_rad, (double)amp, z);
-          }
+          double z = (double)sensor_lorentz10(x0, xs) + noise_out;
+          if (f_radial && sc->rad_mode == 1) z = fma((double)rnd.z_rad, (double)radial_amp(sc, fx, fy), z);
           zf = (float)z;
         } else {
-          zf = z_rad;
+          zf = rnd.z_rad;
         }
 
         // ---- coalesced stores: the key IS the uint8 charge map ----

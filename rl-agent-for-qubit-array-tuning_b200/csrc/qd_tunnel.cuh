@@ -205,15 +205,7 @@ __global__ void __launch_bounds__(128, 3) qd_tunnel_gs_kernel(const KArgs a) {
     const int scan_id = (int)(item / a.items_per_scan);
     const int part = (int)(item - (long long)scan_id * a.items_per_scan);
     const qd_scan* gscan = a.scans + scan_id;
-    if (lane == 0) {
-      const int env = gscan->env_id;
-      fence_proxy_async();
-      mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
-      tma_bulk_g2s(rec, a.records + (size_t)env * L.rec_doubles, rec_bytes, bar);
-      tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1u;
+    stage_item(a, gscan, rec_bytes, rec, sc, bar, phase, lane);
 
     const int nx = sc->nx, ny = sc->ny;
     const long long npix = (long long)nx * ny;
@@ -958,25 +950,17 @@ __global__ void __launch_bounds__(128, 4) qd_tunnel_select_kernel(const KArgs a)
     const int scan_id = (int)(item / a.items_per_scan);
     const int part = (int)(item - (long long)scan_id * a.items_per_scan);
     const qd_scan* gscan = a.scans + scan_id;
-    if (a.topt & 16) {
+    if (a.fixup) {
       // fix-up mode: only the pixels qd_tunnel_select2_kernel marked (first key = QD_S2_MARK; item-level mark = a NaN in the
       // <n> scratch of the item's first pixel) are done here, each from a cold start
-      // (this launch uses shorter items than the marking kernel -- a.col_parts = its pixels per item -- so that an item
-      // whose pixels are all marked is shared by several warps)
+      // (this launch uses shorter items than the marking kernel, so that an item whose pixels are all marked is shared by
+      // several warps)
       const long long pb = (long long)part * a.rows_per_item;
       if (pb >= (long long)gscan->nx * gscan->ny) continue;
-      const double fl = a.nbar[(gscan->pix_offset + (pb / a.col_parts) * a.col_parts) * N];
+      const double fl = a.nbar[(gscan->pix_offset + (pb / a.mark_ppi) * a.mark_ppi) * N];
       if (fl == fl) continue;
     }
-    if (lane == 0) {
-      const int env = gscan->env_id;
-      fence_proxy_async();
-      mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
-      tma_bulk_g2s(rec, a.records + (size_t)env * L.rec_doubles, rec_bytes, bar);
-      tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1u;
+    stage_item(a, gscan, rec_bytes, rec, sc, bar, phase, lane);
 
     const int nx = sc->nx, ny = sc->ny;
     const long long npix = (long long)nx * ny;
@@ -1076,7 +1060,7 @@ __global__ void __launch_bounds__(128, 4) qd_tunnel_select_kernel(const KArgs a)
     for (long long pix = p_begin; pix < p_end; ++pix) {
       const int iy = (int)(pix / nx), ix = (int)(pix - (long long)iy * nx);
       const size_t tslot = (size_t)scan_id * a.tstride + pix;
-      if ((a.topt & 16) && a.tkeys[tslot * 32] != 0xfffffffffffffffeULL) { have_prev = false; continue; }
+      if (a.fixup && a.tkeys[tslot * 32] != 0xfffffffffffffffeULL) { have_prev = false; continue; }
       // ---------------- potentials, floor (from the relax kernel), r = f - g, h = C r ----------------
       if (lane < NV) {
         vv[lane] = (a.points == nullptr) ? fma((double)iy, sc->dy[lane], fma((double)ix, sc->dx[lane], sc->v0[lane]))
@@ -1345,23 +1329,15 @@ __global__ void __launch_bounds__(128, QD_TE_MIN_BLOCKS) qd_tunnel_eigen_kernel(
     const int scan_id = (int)(item / a.items_per_scan);
     const int part = (int)(item - (long long)scan_id * a.items_per_scan);
     const qd_scan* gscan = a.scans + scan_id;
-    if (a.topt & 8) {
-      // fix-up mode: qd_tunnel_eigen2_kernel left an item-level mark in the floor scratch of the item's first pixel (same
-      // item geometry in both launches); an item whose parent item holds no marked pixel is skipped before anything is staged
-      // (shorter items than the marking kernel's, a.col_parts = its pixels per item: see qd_tunnel_select_kernel)
+    if (a.fixup) {
+      // fix-up mode: qd_tunnel_eigen2_kernel left an item-level mark in the floor scratch of its item's first pixel; an
+      // item whose parent item holds no marked pixel is skipped before anything is staged (shorter items than the marking
+      // kernel's: see qd_tunnel_select_kernel)
       const long long pb = (long long)part * a.rows_per_item;
       if (pb >= (long long)gscan->nx * gscan->ny) continue;
-      if (a.tfloor[((size_t)scan_id * a.tstride + (pb / a.col_parts) * a.col_parts) * 8] != 0xff) continue;
+      if (a.tfloor[((size_t)scan_id * a.tstride + (pb / a.mark_ppi) * a.mark_ppi) * 8] != 0xff) continue;
     }
-    if (lane == 0) {
-      const int env = gscan->env_id;
-      fence_proxy_async();
-      mbar_expect_tx(bar, rec_bytes + (uint32_t)sizeof(qd_scan));
-      tma_bulk_g2s(rec, a.records + (size_t)env * L.rec_doubles, rec_bytes, bar);
-      tma_bulk_g2s(sc, gscan, (uint32_t)sizeof(qd_scan), bar);
-    }
-    mbar_wait(bar, phase);
-    phase ^= 1u;
+    stage_item(a, gscan, rec_bytes, rec, sc, bar, phase, lane);
 
     const int nx = sc->nx, ny = sc->ny;
     const long long npix = (long long)nx * ny;
@@ -1376,8 +1352,8 @@ __global__ void __launch_bounds__(128, QD_TE_MIN_BLOCKS) qd_tunnel_eigen_kernel(
     for (long long pix = p_begin; pix < p_end; ++pix) {
       const int iy = (int)(pix / nx), ix = (int)(pix - (long long)iy * nx);
       double nbar[N];
-      // fix-up mode (topt bit 3): only the pixels qd_tunnel_eigen2_kernel marked with a NaN are (re)done here
-      if ((a.topt & 8) && a.nbar[(pix0 + pix) * N] == a.nbar[(pix0 + pix) * N]) continue;
+      // fix-up mode: only the pixels qd_tunnel_eigen2_kernel marked with a NaN are (re)done here
+      if (a.fixup && a.nbar[(pix0 + pix) * N] == a.nbar[(pix0 + pix) * N]) continue;
       if (!replace) {
         uint64_t key = a.tkeys[((size_t)scan_id * a.tstride + pix) * 32 + lane];
         // ---------------- voltages, potentials, tunnel couplings ----------------
