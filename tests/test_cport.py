@@ -5,12 +5,19 @@ import pytest
 from util import oracle_batch
 
 
-@pytest.mark.parametrize("n_dot,alg,flag_names", [
-    (2, "default", ()), (4, "default", ("LATCH", "NOISE", "RADIAL")), (4, "default", ("LATCH", "NOISE", "CARRY_ROWS")),
-    (6, "default", ("LATCH",)), (5, "thresholded", ()), (3, "brute_force", ()), (4, "default", ("THERMAL",)),
-    (3, "default", ("NOISE", "WHITE_ON_OUTPUT")),
+# (n_dot, algorithm, max_charge_carriers, flags, offset_range).  The brute-force and 8-dot thermal cases use windows up
+# to 6 V off the set point, so that dots sit below 0 and above max_charge_carriers: the box edges of the search.
+@pytest.mark.parametrize("n_dot,alg,maxc,flag_names,offset_range", [
+    (2, "default", 4, (), 3.0), (4, "default", 4, ("LATCH", "NOISE", "RADIAL"), 3.0),
+    (4, "default", 4, ("LATCH", "NOISE", "CARRY_ROWS"), 3.0), (6, "default", 4, ("LATCH",), 3.0),
+    (5, "thresholded", 4, (), 3.0), (3, "brute_force", 4, (), 3.0), (4, "default", 4, ("THERMAL",), 3.0),
+    (3, "default", 4, ("NOISE", "WHITE_ON_OUTPUT"), 3.0),
+    (3, "brute_force", 15, ("THERMAL",), 6.0), (4, "brute_force", 0, (), 6.0),
+    (4, "brute_force", 1, ("THERMAL", "LATCH"), 6.0), (5, "brute_force", 4, ("THERMAL",), 6.0),
+    (8, "default", 4, ("THERMAL",), 6.0), (8, "thresholded", 4, ("THERMAL",), 6.0),
+    (3, "brute_force", 15, ("LATCH", "NOISE"), 6.0),
 ])
-def test_cport_matches_numpy_oracle(n_dot, alg, flag_names):
+def test_cport_matches_numpy_oracle(n_dot, alg, maxc, flag_names, offset_range):
     import qdsim
     from oracle import cport
     from qdsim import synth
@@ -18,9 +25,10 @@ def test_cport_matches_numpy_oracle(n_dot, alg, flag_names):
     for f in flag_names:
         flags |= getattr(qdsim, "FLAG_" + f)
     dev = synth.sample_devices(2, n_dot, seed=40 + n_dot)
-    mb = synth.model_batch(dev, algorithm=alg, thermal="THERMAL" in flag_names, threshold=0.6)
+    mb = synth.model_batch(dev, algorithm=alg, thermal="THERMAL" in flag_names, threshold=0.6, max_charge_carriers=maxc)
     mb.params["tele_p01"], mb.params["tele_p10"], mb.params["tele_amp"] = 0.04, 0.07, 0.01
-    scans = synth.env_step_scans(mb, dev, res=24, seed=5, offset_range=3.0)
+    res = 24 if n_dot < 8 else 12
+    scans = synth.env_step_scans(mb, dev, res=res, seed=5, offset_range=offset_range)
     scans["rad_zero_radius"], scans["rad_alpha"] = 1.0, 0.02
     z, n, _ = cport.run_scans(mb, scans, flags, threads=2)
     z_ref, n_ref, _ = oracle_batch(mb, scans, flags)

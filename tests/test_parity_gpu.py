@@ -99,7 +99,7 @@ def test_thresholded(engine):
     compare_charges(n, n_ref, margin)
 
 
-@pytest.mark.parametrize("n_dot", [2, 4])
+@pytest.mark.parametrize("n_dot", [2, 3, 4, 5])
 def test_brute_force(engine, n_dot):
     from qdsim import N_U8
     dev, mb, scans = _setup(engine, n_dot, n_env=2, algorithm="brute_force", res=32, latching=False, noise=False)
