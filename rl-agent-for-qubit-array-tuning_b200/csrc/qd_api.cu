@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <type_traits>
 #include <vector>
 
 #include "qd_kernels.cuh"
@@ -119,61 +120,12 @@ size_t n_elem_size(int n_type) {
 
 using kernel_fn = void (*)(const qd::KArgs);
 
-template <int ALG, bool THERMAL, bool POINTS>
-kernel_fn pick_n(int n) {
-  switch (n) {
-    case 1: return qd::qd_scan_kernel<1, ALG, THERMAL, POINTS>;
-    case 2: return qd::qd_scan_kernel<2, ALG, THERMAL, POINTS>;
-    case 3: return qd::qd_scan_kernel<3, ALG, THERMAL, POINTS>;
-    case 4: return qd::qd_scan_kernel<4, ALG, THERMAL, POINTS>;
-    case 5: return qd::qd_scan_kernel<5, ALG, THERMAL, POINTS>;
-    case 6: return qd::qd_scan_kernel<6, ALG, THERMAL, POINTS>;
-    case 7: return qd::qd_scan_kernel<7, ALG, THERMAL, POINTS>;
-    case 8: return qd::qd_scan_kernel<8, ALG, THERMAL, POINTS>;
-    default: return nullptr;
-  }
-}
-
-#define QD_PICK_N(NAME, KERNEL)                                  \
-  kernel_fn NAME(int n) {                                        \
-    switch (n) {                                                 \
-      case 2: return qd::KERNEL<2>;                              \
-      case 3: return qd::KERNEL<3>;                              \
-      case 4: return qd::KERNEL<4>;                              \
-      case 5: return qd::KERNEL<5>;                              \
-      case 6: return qd::KERNEL<6>;                              \
-      case 7: return qd::KERNEL<7>;                              \
-      case 8: return qd::KERNEL<8>;                              \
-      default: return nullptr;                                   \
-    }                                                            \
-  }
-QD_PICK_N(pick_tunnel_relax, qd_tunnel_relax_kernel)
-QD_PICK_N(pick_tunnel_select, qd_tunnel_select_kernel)
-QD_PICK_N(pick_tunnel_eigen, qd_tunnel_eigen_kernel)
-QD_PICK_N(pick_tunnel_eigen2, qd_tunnel_eigen2_kernel)
-kernel_fn pick_tunnel_select2(int n) {
-  switch (n) {
-    case 4: return qd::qd_tunnel_select2_kernel<4>;
-    case 5: return qd::qd_tunnel_select2_kernel<5>;
-    case 6: return qd::qd_tunnel_select2_kernel<6>;
-    case 7: return qd::qd_tunnel_select2_kernel<7>;
-    case 8: return qd::qd_tunnel_select2_kernel<8>;
-    default: return nullptr;      // fewer than 32 candidates can be valid below four dots: the block walk pads
-  }
-}
-
-kernel_fn pick_fast(int n) {
-  switch (n) {
-    case 1: return qd::qd_scan_fast_kernel<1>;
-    case 2: return qd::qd_scan_fast_kernel<2>;
-    case 3: return qd::qd_scan_fast_kernel<3>;
-    case 4: return qd::qd_scan_fast_kernel<4>;
-    case 5: return qd::qd_scan_fast_kernel<5>;
-    case 6: return qd::qd_scan_fast_kernel<6>;
-    case 7: return qd::qd_scan_fast_kernel<7>;
-    case 8: return qd::qd_scan_fast_kernel<8>;
-    default: return nullptr;
-  }
+// The instance of a kernel template for n_dot = n: `k` maps std::integral_constant<int, N> to the instance for N dots.
+// Only MIN_N..QD_MAX_DOTS are instantiated; any other n gives nullptr.
+template <int MIN_N, int N = QD_MAX_DOTS, typename F>
+kernel_fn pick_dots(int n, F k) {
+  if constexpr (N < MIN_N) return nullptr;
+  else return n == N ? k(std::integral_constant<int, N>{}) : pick_dots<MIN_N, N - 1>(n, k);
 }
 
 // default / thresholded search with a hard argmin on affine windows runs the restructured kernel (qd_scan_fast_kernel);
@@ -185,21 +137,11 @@ bool use_fast_kernel(const qd_layout& L, unsigned flags, bool points) {
   return !(e && e[0] == '1');
 }
 
-kernel_fn pick_tunnel_gs(int n) {
-  switch (n) {
-    case 2: return qd::qd_tunnel_gs_kernel<2>;
-    case 3: return qd::qd_tunnel_gs_kernel<3>;
-    case 4: return qd::qd_tunnel_gs_kernel<4>;
-    case 5: return qd::qd_tunnel_gs_kernel<5>;
-    case 6: return qd::qd_tunnel_gs_kernel<6>;
-    case 7: return qd::qd_tunnel_gs_kernel<7>;
-    case 8: return qd::qd_tunnel_gs_kernel<8>;
-    default: return nullptr;
-  }
-}
-
 template <int ALG, bool THERMAL>
-kernel_fn pick_p(int n, bool points) { return points ? pick_n<ALG, THERMAL, true>(n) : pick_n<ALG, THERMAL, false>(n); }
+kernel_fn pick_p(int n, bool points) {
+  if (points) return pick_dots<1>(n, [](auto k) { return qd::qd_scan_kernel<decltype(k)::value, ALG, THERMAL, true>; });
+  return pick_dots<1>(n, [](auto k) { return qd::qd_scan_kernel<decltype(k)::value, ALG, THERMAL, false>; });
+}
 
 kernel_fn pick_kernel(const qd_layout& L, unsigned flags, bool points) {
   const bool thermal = flags & QD_FLAG_THERMAL;
@@ -252,6 +194,20 @@ int configure_kernel(qd_ctx* ctx, const void* fn, size_t smem) {
   return QD_OK;
 }
 
+// Enqueue one kernel: configured first if it takes dynamic shared memory (the others keep the driver's defaults), the
+// grid clamped to what one launch takes, the launch checked and counted in ctx->launches.
+template <typename... P, typename... A>
+int issue(qd_ctx* ctx, void (*fn)(P...), long long grid, int threads, size_t smem, cudaStream_t stream, const A&... args) {
+  if (smem) {
+    const int rc = configure_kernel(ctx, (const void*)fn, smem);
+    if (rc) return rc;
+  }
+  fn<<<(unsigned)std::min(grid, 0x7fffffffLL), threads, smem, stream>>>(args...);
+  QD_CUDA(ctx, cudaGetLastError());
+  ctx->launches += 1;
+  return QD_OK;
+}
+
 // The context's scratch buffers (d_scans, d_nbar) are shared by all launches.  A launch on stream B that follows one on
 // stream A must not re-stage them before A's kernels are done with them: every launch records `last_launch`, and work
 // enqueued on a different stream waits for it first (same stream: already ordered, no call made).
@@ -266,179 +222,145 @@ int mark_launch(qd_ctx* ctx, cudaStream_t stream) {
   return QD_OK;
 }
 
+// Items of the warp-per-pixel tunnel kernels over a.n_scan scans of <= max_pix pixels: <= 64 consecutive pixels of one
+// scan each (the warm start runs along an item), about four per warp resident at `warps_per_sm` warps per SM; one warp
+// per CTA while four would leave SMs idle.  Sets a.rows_per_item (pixels per item) and a.items_per_scan.
+struct PixelItems { int warps; long long grid; };
+PixelItems plan_pixel_items(const qd_ctx* ctx, qd::KArgs& a, long long max_pix, int warps_per_sm) {
+  const long long want_items = (long long)ctx->sm_count * warps_per_sm * 4;
+  const long long ppi = std::min<long long>(std::max<long long>(((long long)a.n_scan * max_pix) / want_items, 1), 64);
+  a.rows_per_item = (int)ppi;
+  a.items_per_scan = (int)((max_pix + ppi - 1) / ppi);
+  const long long items = (long long)a.n_scan * a.items_per_scan;
+  const int warps = (items < (long long)ctx->sm_count * 4) ? 1 : 4;
+  return {warps, (items + warps - 1) / warps};
+}
+
+// One stage of the split tunnel pipeline: a primary kernel and the older kernel it falls back on.  `primary` (nullptr
+// when it does not apply or a switch turns it off) runs with the arguments `pa` and marks the pixels it could not do;
+// `fallback` then redoes only those (fix-up mode), or does every pixel when there is no primary.  fix = false skips
+// the second launch and leaves the marks in place.  `g` holds the items of plan_pixel_items.
+int primary_then_fixup(qd_ctx* ctx, const qd::KArgs& g, const PixelItems& p, kernel_fn primary, const qd::KArgs& pa,
+                       kernel_fn fallback, int fallback_slot_bytes, bool fix, cudaStream_t stream) {
+  if (primary) {
+    const int rc = issue(ctx, primary, p.grid, p.warps * 32, (size_t)pa.slot_bytes * p.warps, stream, pa);
+    if (rc) return rc;
+  }
+  if (!fix) return QD_OK;
+  qd::KArgs fa = g;
+  fa.slot_bytes = fallback_slot_bytes;
+  long long grid = p.grid;
+  if (primary) {
+    // items of 8 pixels (no state is carried between marked pixels), so that a stretch of marked pixels is spread over
+    // several warps; mark_ppi carries the marking kernel's item length to the mark look-up
+    fa.fixup = 1;
+    fa.mark_ppi = g.rows_per_item;
+    fa.rows_per_item = (g.rows_per_item % 8 == 0) ? 8 : g.rows_per_item;   // (must divide the marking kernel's item length)
+    fa.items_per_scan = (int)((ctx->up_max_pix + fa.rows_per_item - 1) / fa.rows_per_item);
+    grid = ((long long)fa.n_scan * fa.items_per_scan + p.warps - 1) / p.warps;
+    // (almost every item is skipped on its mark: a resident-size grid looping over the items instead of one CTA per four)
+    grid = std::min<long long>(grid, (long long)ctx->sm_count * 32);
+  }
+  return issue(ctx, fallback, grid, p.warps * 32, (size_t)fa.slot_bytes * p.warps, stream, fa);
+}
+
+// Path B: the tunnel-coupled ground state <n> of every pixel into d_nbar, for the scan kernel's latching / sensor / noise
+int tunnel_ground_state(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, const double* d_points, unsigned flags,
+                        cudaStream_t stream) {
+  const int N = ctx->L.n_dot;
+  const kernel_fn gs = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_gs_kernel<decltype(n)::value>; });
+  if (!gs) return fail(ctx, QD_ERR_UNSUPPORTED, "tunnel path needs 2..8 dots, got %d", N);
+  int rc = grow(ctx, &ctx->d_nbar, &ctx->nbar_cap, (size_t)ctx->up_pixels * N * sizeof(double));
+  if (rc) return rc;
+  qd::KArgs g;
+  memset(&g, 0, sizeof(g));
+  g.L = ctx->L; g.records = ctx->d_records; g.scans = d_scans; g.points = d_points; g.z_out = nullptr;
+  g.n_out = nullptr; g.nbar = ctx->d_nbar; g.n_scan = n_scan; g.n_type = QD_N_NONE; g.flags = flags;
+  g.status = ctx->d_status;
+  g.topt = 7;
+  if (const char* e = getenv("QDSIM_TUNNEL_OPT")) g.topt = atoi(e) & 7;
+  const long long max_pix = ctx->up_max_pix;
+  const char* mono_e = getenv("QDSIM_TUNNEL_MONO");
+  if (mono_e && mono_e[0] == '1') {
+    // the single-kernel form (one warp per pixel does everything): kept as the A/B reference of the split pipeline
+    g.slot_bytes = qd::qd_tunnel_slot_bytes(ctx->L);
+    const PixelItems p = plan_pixel_items(ctx, g, max_pix, 12);
+    return issue(ctx, gs, p.grid, p.warps * 32, (size_t)g.slot_bytes * p.warps, stream, g);
+  }
+  // split pipeline R -> S -> E over chunks of scans (8 + 128 + 256 bytes of scratch per pixel of a chunk)
+  const kernel_fn kr = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_relax_kernel<decltype(n)::value>; });
+  const kernel_fn ks = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_select_kernel<decltype(n)::value>; });
+  const kernel_fn ke = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen_kernel<decltype(n)::value>; });
+  // S: the lattice-enumeration kernel first (four dots and more: fewer than 32 candidates can be valid below four dots,
+  // and the block walk pads; QDSIM_SELECT=block skips it), then the block walk -- as the fix-up pass over the pixels the
+  // enumeration marked, or for everything
+  const char* sel_e = getenv("QDSIM_SELECT");
+  const kernel_fn ks2 = (sel_e && sel_e[0] == 'b')
+                            ? nullptr
+                            : pick_dots<4>(N, [](auto n) { return qd::qd_tunnel_select2_kernel<decltype(n)::value>; });
+  // E: the Noda-iteration kernel first (QDSIM_EIGEN=householder skips it); what it could not do (sectors of more
+  // than 16 states, no convergence) is marked with a NaN and redone by the Householder kernel in fix-up mode
+  const char* eig_e = getenv("QDSIM_EIGEN");
+  const bool no_fixup = eig_e && eig_e[0] == 'n';          // (measurement only: leaves the NaN marks in place)
+  const kernel_fn ke2 = (eig_e && eig_e[0] == 'h')
+                            ? nullptr
+                            : pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen2_kernel<decltype(n)::value>; });
+  long long chunk_pix = 8LL << 20;
+  if (const char* e = getenv("QDSIM_TUNNEL_CHUNK_PIX")) chunk_pix = atoll(e) > 0 ? atoll(e) : chunk_pix;
+  const long long spc = std::min<long long>(std::max<long long>(chunk_pix / max_pix, 1), n_scan);   // scans per chunk
+  rc = grow(ctx, &ctx->d_tfloor, &ctx->tfloor_cap, (size_t)spc * max_pix * 8);
+  if (rc) return rc;
+  rc = grow(ctx, &ctx->d_tkeys, &ctx->tkeys_cap, (size_t)spc * max_pix * 256);
+  if (rc) return rc;
+  rc = grow(ctx, &ctx->d_tpot, &ctx->tpot_cap, (size_t)spc * max_pix * 128);
+  if (rc) return rc;
+  g.tfloor = ctx->d_tfloor;
+  g.tpot = ctx->d_tpot;
+  g.tkeys = ctx->d_tkeys;
+  g.tstride = max_pix;
+  for (long long c0 = 0; c0 < n_scan; c0 += spc) {
+    g.scans = d_scans + c0;
+    g.n_scan = (int)std::min<long long>(spc, n_scan - c0);
+    // R: one thread per pixel, a CTA per <= 1024 pixels of one scan
+    qd::KArgs r = g;
+    r.rows_per_item = (int)std::min<long long>(1024, max_pix);
+    r.items_per_scan = (int)((max_pix + r.rows_per_item - 1) / r.rows_per_item);
+    rc = issue(ctx, kr, (long long)r.n_scan * r.items_per_scan, 128, qd::qd_tunnel_relax_smem_bytes(ctx->L), stream, r);
+    if (rc) return rc;
+    // S and E: one warp per pixel
+    const PixelItems p = plan_pixel_items(ctx, g, max_pix, 16);
+    qd::KArgs sa = g;
+    sa.slot_bytes = qd::qd_tunnel_select2_slot_bytes(ctx->L);
+    rc = primary_then_fixup(ctx, g, p, ks2, sa, ks, qd::qd_tunnel_select_slot_bytes(ctx->L), true, stream);
+    if (rc) return rc;
+    qd::KArgs ea = g;
+    ea.e2_kappa = 4.0f; ea.e2_qsafe = 4.0f; ea.e2_tol = 2e-10f;
+    if (const char* e = getenv("QDSIM_E2_KAPPA")) ea.e2_kappa = (float)atof(e);
+    if (const char* e = getenv("QDSIM_E2_QSAFE")) ea.e2_qsafe = (float)atof(e);
+    if (const char* e = getenv("QDSIM_E2_TOL")) ea.e2_tol = (float)atof(e);
+    ea.slot_bytes = qd::qd_tunnel_eigen2_slot_bytes(ctx->L);
+    rc = primary_then_fixup(ctx, g, p, ke2, ea, ke, qd::qd_tunnel_eigen_slot_bytes(ctx->L), !no_fixup, stream);
+    if (rc) return rc;
+  }
+  return QD_OK;
+}
+
 // enqueue one launch over device-resident descriptors
 int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const double* d_points, float* d_z, void* d_n,
            int n_type, unsigned flags, cudaStream_t stream, int rows_cap = 0, const qd_scan* h_one = nullptr) {
-  {
-    const int rc0 = order_after_last_launch(ctx, stream);     // the scratch of an earlier launch on another stream
-    if (rc0) return rc0;
-  }
+  int rc = order_after_last_launch(ctx, stream);     // the scratch of an earlier launch on another stream
+  if (rc) return rc;
   const bool fast = use_fast_kernel(ctx->L, flags, d_points != nullptr);
-  kernel_fn fn = fast ? pick_fast(ctx->L.n_dot) : pick_kernel(ctx->L, flags, d_points != nullptr);
+  const kernel_fn fn =
+      fast ? pick_dots<1>(ctx->L.n_dot, [](auto n) { return qd::qd_scan_fast_kernel<decltype(n)::value>; })
+           : pick_kernel(ctx->L, flags, d_points != nullptr);
   if (!fn) return fail(ctx, QD_ERR_UNSUPPORTED, "no kernel for n_dot=%d algorithm=%d", ctx->L.n_dot, ctx->L.algorithm);
   qd::KArgs a;
   memset(&a, 0, sizeof(a));
-  a.nbar = nullptr;
   if (ctx->L.algorithm == QD_ALG_TUNNEL) {
-    // tunnel-coupled ground state of every pixel into d_nbar, then (below) the scan kernel for latching / sensor / noise
-    const int N = ctx->L.n_dot;
-    kernel_fn gs = pick_tunnel_gs(N);
-    if (!gs) return fail(ctx, QD_ERR_UNSUPPORTED, "tunnel path needs 2..8 dots, got %d", N);
-    int rc = grow(ctx, &ctx->d_nbar, &ctx->nbar_cap, (size_t)ctx->up_pixels * N * sizeof(double));
+    // the tunnel-coupled ground state first; the scan kernel below reads it from d_nbar
+    rc = tunnel_ground_state(ctx, n_scan, d_scans, d_points, flags, stream);
     if (rc) return rc;
-    qd::KArgs g;
-    memset(&g, 0, sizeof(g));
-    g.L = ctx->L; g.records = ctx->d_records; g.scans = d_scans; g.points = d_points; g.z_out = nullptr;
-    g.n_out = nullptr; g.nbar = ctx->d_nbar; g.n_scan = n_scan; g.n_type = QD_N_NONE; g.flags = flags;
-    g.status = ctx->d_status;
-    g.topt = 7;
-    if (const char* e = getenv("QDSIM_TUNNEL_OPT")) g.topt = atoi(e) & 7;
-    const long long max_pix = ctx->up_max_pix;
-    const char* mono_e = getenv("QDSIM_TUNNEL_MONO");
-    const bool mono = mono_e && mono_e[0] == '1';
-    if (mono) {
-      // the single-kernel form (one warp per pixel does everything): kept as the A/B reference of the split pipeline
-      g.slot_bytes = qd::qd_tunnel_slot_bytes(ctx->L);
-      const long long want_items = (long long)ctx->sm_count * 12 * 4;
-      long long ppi = ((long long)n_scan * max_pix) / want_items;          // pixels per item
-      if (ppi < 1) ppi = 1;
-      if (ppi > 64) ppi = 64;
-      g.rows_per_item = (int)ppi;
-      g.items_per_scan = (int)((max_pix + ppi - 1) / ppi);
-      const long long items = (long long)n_scan * g.items_per_scan;
-      const int gw = (items < (long long)ctx->sm_count * 4) ? 1 : 4;
-      long long ggrid = (items + gw - 1) / gw;
-      if (ggrid > 0x7fffffffLL) ggrid = 0x7fffffffLL;
-      const size_t gsmem = (size_t)g.slot_bytes * gw;
-      rc = configure_kernel(ctx, (const void*)gs, gsmem);
-      if (rc) return rc;
-      gs<<<(unsigned)ggrid, gw * 32, gsmem, stream>>>(g);
-      QD_CUDA(ctx, cudaGetLastError());
-      ctx->launches += 1;
-    } else {
-      // split pipeline R -> S -> E over chunks of scans (8 + 256 bytes of scratch per pixel of a chunk)
-      kernel_fn kr = pick_tunnel_relax(N), ks = pick_tunnel_select(N), ke = pick_tunnel_eigen(N);
-      long long chunk_pix = 8LL << 20;
-      if (const char* e = getenv("QDSIM_TUNNEL_CHUNK_PIX")) chunk_pix = atoll(e) > 0 ? atoll(e) : chunk_pix;
-      long long spc = chunk_pix / max_pix;                                 // scans per chunk
-      if (spc < 1) spc = 1;
-      if (spc > n_scan) spc = n_scan;
-      rc = grow(ctx, &ctx->d_tfloor, &ctx->tfloor_cap, (size_t)spc * max_pix * 8);
-      if (rc) return rc;
-      rc = grow(ctx, &ctx->d_tkeys, &ctx->tkeys_cap, (size_t)spc * max_pix * 256);
-      if (rc) return rc;
-      rc = grow(ctx, &ctx->d_tpot, &ctx->tpot_cap, (size_t)spc * max_pix * 128);
-      if (rc) return rc;
-      g.tfloor = ctx->d_tfloor;
-      g.tpot = ctx->d_tpot;
-      g.tkeys = ctx->d_tkeys;
-      g.tstride = max_pix;
-      for (long long c0 = 0; c0 < n_scan; c0 += spc) {
-        const int nc = (int)std::min<long long>(spc, n_scan - c0);
-        g.scans = d_scans + c0;
-        g.n_scan = nc;
-        // R: one thread per pixel, a CTA per <= 1024 pixels of one scan
-        {
-          qd::KArgs r = g;
-          r.rows_per_item = (int)std::min<long long>(1024, max_pix);
-          r.items_per_scan = (int)((max_pix + r.rows_per_item - 1) / r.rows_per_item);
-          long long grid = (long long)nc * r.items_per_scan;
-          if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
-          const size_t smem = (size_t)qd::qd_tunnel_relax_smem_bytes(ctx->L);
-          rc = configure_kernel(ctx, (const void*)kr, smem);
-          if (rc) return rc;
-          kr<<<(unsigned)grid, 128, smem, stream>>>(r);
-          QD_CUDA(ctx, cudaGetLastError());
-        }
-        // S and E: one warp per pixel, items of <= 64 consecutive pixels (the warm start runs along an item)
-        const long long want_items = (long long)ctx->sm_count * 16 * 4;
-        long long ppi = ((long long)nc * max_pix) / want_items;
-        if (ppi < 1) ppi = 1;
-        if (ppi > 64) ppi = 64;
-        g.rows_per_item = (int)ppi;
-        g.items_per_scan = (int)((max_pix + ppi - 1) / ppi);
-        const long long items = (long long)nc * g.items_per_scan;
-        const int gw = (items < (long long)ctx->sm_count * 4) ? 1 : 4;
-        long long ggrid = (items + gw - 1) / gw;
-        if (ggrid > 0x7fffffffLL) ggrid = 0x7fffffffLL;
-        // S: the lattice-enumeration kernel first (four dots and more; QDSIM_SELECT=block skips it), then the block walk --
-        // as the fix-up pass over the pixels the enumeration marked, or for everything
-        const char* sel_e = getenv("QDSIM_SELECT");
-        kernel_fn ks2 = (sel_e && sel_e[0] == 'b') ? nullptr : pick_tunnel_select2(N);
-        if (ks2) {
-          qd::KArgs sa = g;
-          sa.slot_bytes = qd::qd_tunnel_select2_slot_bytes(ctx->L);
-          const size_t smem = (size_t)sa.slot_bytes * gw;
-          rc = configure_kernel(ctx, (const void*)ks2, smem);
-          if (rc) return rc;
-          ks2<<<(unsigned)ggrid, gw * 32, smem, stream>>>(sa);
-          QD_CUDA(ctx, cudaGetLastError());
-          ctx->launches += 1;
-        }
-        // fix-up launches: items of 8 pixels (no state is carried between marked pixels), so that a stretch of marked pixels
-        // is spread over several warps; mark_ppi carries the marking kernel's item length to the mark look-up
-        const int fix_ppi = (ppi % 8 == 0) ? 8 : (int)ppi;          // (must divide the marking kernel's item length)
-        const int fix_ips = (int)((max_pix + fix_ppi - 1) / fix_ppi);
-        long long fix_grid = ((long long)nc * fix_ips + gw - 1) / gw;
-        // (almost every item is skipped on its mark: a resident-size grid looping over the items instead of one CTA per four)
-        fix_grid = std::min<long long>(fix_grid, (long long)ctx->sm_count * 32);
-        {
-          qd::KArgs sa = g;
-          long long sgrid = ggrid;
-          if (ks2) {
-            sa.fixup = 1;
-            sa.mark_ppi = (int)ppi;
-            sa.rows_per_item = fix_ppi;
-            sa.items_per_scan = fix_ips;
-            sgrid = fix_grid;
-          }
-          sa.slot_bytes = qd::qd_tunnel_select_slot_bytes(ctx->L);
-          const size_t smem = (size_t)sa.slot_bytes * gw;
-          rc = configure_kernel(ctx, (const void*)ks, smem);
-          if (rc) return rc;
-          ks<<<(unsigned)sgrid, gw * 32, smem, stream>>>(sa);
-          QD_CUDA(ctx, cudaGetLastError());
-        }
-        // E: the Noda-iteration kernel first (QDSIM_EIGEN=householder skips it); what it could not do (sectors of more
-        // than 16 states, no convergence) is marked with a NaN and redone by the Householder kernel in fix-up mode
-        const char* eig_e = getenv("QDSIM_EIGEN");
-        const bool householder_only = eig_e && eig_e[0] == 'h';
-        const bool no_fixup = eig_e && eig_e[0] == 'n';          // (measurement only: leaves the NaN marks in place)
-        if (!householder_only) {
-          kernel_fn ke2 = pick_tunnel_eigen2(N);
-          qd::KArgs ea = g;
-          ea.e2_kappa = 4.0f; ea.e2_qsafe = 4.0f; ea.e2_tol = 2e-10f;
-          if (const char* e = getenv("QDSIM_E2_KAPPA")) ea.e2_kappa = (float)atof(e);
-          if (const char* e = getenv("QDSIM_E2_QSAFE")) ea.e2_qsafe = (float)atof(e);
-          if (const char* e = getenv("QDSIM_E2_TOL")) ea.e2_tol = (float)atof(e);
-          ea.slot_bytes = qd::qd_tunnel_eigen2_slot_bytes(ctx->L);
-          const size_t smem = (size_t)ea.slot_bytes * gw;
-          rc = configure_kernel(ctx, (const void*)ke2, smem);
-          if (rc) return rc;
-          ke2<<<(unsigned)ggrid, gw * 32, smem, stream>>>(ea);
-          QD_CUDA(ctx, cudaGetLastError());
-          ctx->launches += 1;
-        }
-        if (!no_fixup) {
-          qd::KArgs ea = g;
-          long long egrid = ggrid;
-          if (!householder_only) {
-            ea.fixup = 1;
-            ea.mark_ppi = (int)ppi;
-            ea.rows_per_item = fix_ppi;
-            ea.items_per_scan = fix_ips;
-            egrid = fix_grid;
-          }
-          ea.slot_bytes = qd::qd_tunnel_eigen_slot_bytes(ctx->L);
-          const size_t smem = (size_t)ea.slot_bytes * gw;
-          rc = configure_kernel(ctx, (const void*)ke, smem);
-          if (rc) return rc;
-          ke<<<(unsigned)egrid, gw * 32, smem, stream>>>(ea);
-          QD_CUDA(ctx, cudaGetLastError());
-        }
-        ctx->launches += 3;
-      }
-    }
     a.nbar = ctx->d_nbar;
   }
   a.L = ctx->L;
@@ -482,17 +404,17 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
   // one warp per CTA and lets the hardware scheduler balance (16 CTAs of 11.9 KB per SM).  QDSIM_WPC overrides (A/B).
   int wpc = (total_items < (long long)ctx->sm_count * 4) ? 1 : (fast ? 1 : QD_CTA_WARPS);
   if (const char* e = getenv("QDSIM_WPC")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4) wpc = v; }
-  long long grid = (total_items + wpc - 1) / wpc;
-  if (grid > 0x7fffffffLL) grid = 0x7fffffffLL;
-  const size_t smem = (size_t)a.slot_bytes * wpc;
-  {
-    const int rc2 = configure_kernel(ctx, (const void*)fn, smem);
-    if (rc2) return rc2;
-  }
-  fn<<<(unsigned)grid, wpc * 32, smem, stream>>>(a);
-  QD_CUDA(ctx, cudaGetLastError());
-  ctx->launches += 1;
+  rc = issue(ctx, fn, (total_items + wpc - 1) / wpc, wpc * 32, (size_t)a.slot_bytes * wpc, stream, a);
+  if (rc) return rc;
   return mark_launch(ctx, stream);
+}
+
+int check_scan(qd_ctx* ctx, int i, const qd_scan& s) {
+  if (s.env_id < 0 || s.env_id >= ctx->n_env)
+    return fail(ctx, QD_ERR_INVALID, "scan %d: env_id %d out of range [0,%d)", i, s.env_id, ctx->n_env);
+  if (s.nx <= 0 || s.ny <= 0) return fail(ctx, QD_ERR_INVALID, "scan %d: nx, ny must be positive", i);
+  if (s.pix_offset < 0) return fail(ctx, QD_ERR_INVALID, "scan %d: negative pix_offset", i);
+  return QD_OK;
 }
 
 int stage_scans(qd_ctx* ctx, int n_scan, const qd_scan* scans, cudaStream_t stream, int* max_ny,
@@ -544,10 +466,8 @@ int stage_scans(qd_ctx* ctx, int n_scan, const qd_scan* scans, cudaStream_t stre
     const long long np_ = (long long)s.nx * s.ny;
     if (s.pix_offset + np_ > ext) ext = s.pix_offset + np_;
     if (np_ > mpix) mpix = np_;
-    if (s.env_id < 0 || s.env_id >= ctx->n_env)
-      return fail(ctx, QD_ERR_INVALID, "scan %d: env_id %d out of range [0,%d)", i, s.env_id, ctx->n_env);
-    if (s.nx <= 0 || s.ny <= 0) return fail(ctx, QD_ERR_INVALID, "scan %d: nx, ny must be positive", i);
-    if (s.pix_offset < 0) return fail(ctx, QD_ERR_INVALID, "scan %d: negative pix_offset", i);
+    rc = check_scan(ctx, i, s);
+    if (rc) return rc;
     if (s.ny > mny) mny = s.ny;
   }
   *max_ny = mny;
@@ -843,10 +763,9 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
     const long long total = (long long)desc->n_env << N;
     long long blocks = (total + 255) / 256;
     if (blocks > 65535) blocks = 65535;
-    qd::qd_build_q_kernel<<<(unsigned)blocks, 256>>>(L, ctx->d_records, desc->n_env);
-    QD_CUDA(ctx, cudaGetLastError());
+    rc = issue(ctx, qd::qd_build_q_kernel, blocks, 256, 0, nullptr, L, ctx->d_records, desc->n_env);
+    if (rc) return rc;
     QD_CUDA(ctx, cudaDeviceSynchronize());
-    ctx->launches += 1;
   }
   ctx->have_models = true;
   return QD_OK;
@@ -892,9 +811,8 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
                    (long long)scans[0].nx * scans[0].ny * (4 + ctx->L.n_dot * (long long)n_elem_size(n_type)) <= (1 << 20);
   if (one) {
     const qd_scan& s0 = scans[0];
-    if (s0.env_id < 0 || s0.env_id >= ctx->n_env)
-      return fail(ctx, QD_ERR_INVALID, "scan 0: env_id %d out of range [0,%d)", s0.env_id, ctx->n_env);
-    if (s0.nx <= 0 || s0.ny <= 0) return fail(ctx, QD_ERR_INVALID, "scan 0: nx, ny must be positive");
+    rc = check_scan(ctx, 0, s0);
+    if (rc) return rc;
     rc = order_after_last_launch(ctx, ctx->s_compute);
     if (rc) return rc;
     max_ny = s0.ny;
@@ -964,9 +882,7 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
     if (esz) QD_CUDA(ctx, cudaMemsetAsync(ctx->d_n, 0, (size_t)pixels * N * esz, ctx->s_compute));
   }
   const int rows_cap = pipe_rows_cap();
-  const long long all_pixels = ctx->up_pixels;
   for (int c = 0; c < P.n_chunk; ++c) {
-    ctx->up_pixels = all_pixels;      // the tunnel scratch is addressed with the scans' own pixel offsets
     rc = launch(ctx, P.cut[c + 1] - P.cut[c], ctx->d_scans + P.cut[c], max_ny, nullptr, ctx->d_z, ctx->d_n, n_type, flags,
                 ctx->s_compute, P.n_chunk > 1 ? rows_cap : 0);
     if (rc) return rc;
@@ -994,21 +910,15 @@ template <typename OUT>
 int normalise_launch(qd_ctx* ctx, const float* z, OUT* out, int64_t per_env, int n_env, double ql, double qh, double* stats,
                      cudaStream_t stream) {
   const size_t need = (size_t)per_env * sizeof(float);
+  auto fn = qd::qd_normalise_kernel<OUT, false>;
+  size_t smem = 0;
   if (per_env <= 32 * 1024) {        // the env's image fits in the registers of one CTA: one HBM read per pixel
-    qd::qd_normalise_reg_kernel<OUT><<<n_env, 1024, 0, stream>>>(z, out, per_env, n_env, ql, qh, stats);
+    fn = qd::qd_normalise_reg_kernel<OUT>;
   } else if (need <= 200 * 1024) {   // ... or in its shared memory
-    auto fn = qd::qd_normalise_kernel<OUT, true>;
-    if (need > 40 * 1024) {
-      int rc = configure_kernel(ctx, (const void*)fn, need);
-      if (rc) return rc;
-    }
-    fn<<<n_env, 1024, need, stream>>>(z, out, per_env, n_env, ql, qh, stats);
-  } else {
-    qd::qd_normalise_kernel<OUT, false><<<n_env, 1024, 0, stream>>>(z, out, per_env, n_env, ql, qh, stats);
+    fn = qd::qd_normalise_kernel<OUT, true>;
+    smem = need;
   }
-  QD_CUDA(ctx, cudaGetLastError());
-  ctx->launches += 1;
-  return QD_OK;
+  return issue(ctx, fn, n_env, 1024, smem, stream, z, out, per_env, n_env, ql, qh, stats);
 }
 
 int normalise_typed(qd_ctx* ctx, const float* z, void* out, int z_type, int64_t per_env, int n_env, double q_low_pct,
@@ -1062,9 +972,7 @@ int qd_scan_obs_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, int scans_pe
   }
   const ChunkPlan P = plan_chunks(ctx, n_scan, scans, scans_per_env);
   const int rows_cap = pipe_rows_cap();
-  const long long all_pixels = ctx->up_pixels;
   for (int c = 0; c < P.n_chunk; ++c) {
-    ctx->up_pixels = all_pixels;
     rc = launch(ctx, P.cut[c + 1] - P.cut[c], ctx->d_scans + P.cut[c], max_ny, nullptr, ctx->d_z, nullptr, QD_N_NONE, flags,
                 ctx->s_compute, P.n_chunk > 1 ? rows_cap : 0);
     if (rc) return rc;
@@ -1079,9 +987,9 @@ int qd_scan_obs_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, int scans_pe
     } else if (z_type == QD_Z_F16) {
       long long blocks = (hi - lo + 2047) / 2048;
       if (blocks > 8 * (long long)ctx->sm_count) blocks = 8 * (long long)ctx->sm_count;
-      qd::qd_to_half_kernel<<<(unsigned)blocks, 256, 0, ctx->s_compute>>>(ctx->d_z + lo, (__half*)ctx->d_obs + lo, hi - lo);
-      QD_CUDA(ctx, cudaGetLastError());
-      ctx->launches += 1;
+      rc = issue(ctx, qd::qd_to_half_kernel, blocks, 256, 0, ctx->s_compute, ctx->d_z + lo, (__half*)ctx->d_obs + lo,
+                 hi - lo);
+      if (rc) return rc;
       src = (const char*)ctx->d_obs + (size_t)lo * zsz;
     }
     QD_CUDA(ctx, cudaEventRecord(ctx->chunk_done[c], ctx->s_compute));
