@@ -190,8 +190,9 @@ int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const 
 int qd_normalise_obs(qd_ctx* ctx, const float* z, float* out, int64_t per_env, int n_env, double q_low_pct,
                      double q_high_pct, double* stats, void* stream);
 
-/* qd_normalise_obs with a typed output (enum qd_ztype): out holds n_env * per_env elements of z_type; QD_Z_U8 stores
- * rint(255 * x).  z, out, stats are DEVICE pointers. */
+/* qd_normalise_obs with a typed output (enum qd_ztype): out holds n_env * per_env elements of z_type, each the fp64
+ * value x above rounded as QD_Z_F32 = (float)x, QD_Z_F16 = half((float)x), QD_Z_U8 = rint(255 * x).  z, out, stats
+ * are DEVICE pointers. */
 int qd_normalise_obs_typed(qd_ctx* ctx, const float* z, void* out, int z_type, int64_t per_env, int n_env,
                            double q_low_pct, double q_high_pct, double* stats, void* stream);
 

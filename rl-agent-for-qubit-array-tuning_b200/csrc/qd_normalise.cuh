@@ -246,27 +246,21 @@ __global__ void __launch_bounds__(1024) qd_normalise_reg_kernel(const float* __r
   const bool ok = p_high > p_low;
   const double span = p_high - p_low;
   OUT* __restrict__ dst = out + (size_t)env * per_env;
-  if constexpr (sizeof(OUT) == 4) {
-    // fp32 output: the reference's fp64 expression, bit for bit (tests/test_obs.py)
+  // The reference's fp64 quotient (x - p_low) / span, correctly rounded, for every output type: the same values as
+  // qd_normalise_kernel's division, whichever kernel the env's size picks (tests/test_normalise_gpu.py).  Without a
+  // division per pixel: q0 = d * RN(1 / span) is within an ulp and one exact residual step rounds it correctly
+  // (Markstein), as long as nothing underflows -- d is 0 or >= ~2^-202 for fp32 pixels.  (An fp32 multiply-add by
+  // 1 / span instead loses about log2(p_low / span) bits: 8 LSB of uint8 at p_low / span = 1e6.)
+  const double rcp = ok ? 1.0 / span : 0.0;
 #pragma unroll
-    for (int e = 0; e < EPT; ++e) {
-      const long long i = (long long)e * 1024 + tid;
-      if (i < per_env) {
-        double v = ok ? ((double)key_f32(key[e]) - p_low) / span : 0.0;
-        v = fmin(fmax(v, 0.0), 1.0);
-        store_norm(dst + i, v);
-      }
-    }
-  } else {
-    // half / uint8 output (declared +-1 LSB): one fp32 multiply-add per pixel instead of an fp64 division
-    const float sc = ok ? (float)(1.0 / span) : 0.0f, of = ok ? (float)(-p_low / span) : 0.0f;
-#pragma unroll
-    for (int e = 0; e < EPT; ++e) {
-      const long long i = (long long)e * 1024 + tid;
-      if (i < per_env) {
-        const float v = fminf(fmaxf(fmaf(key_f32(key[e]), sc, of), 0.0f), 1.0f);
-        store_norm(dst + i, (double)v);
-      }
+  for (int e = 0; e < EPT; ++e) {
+    const long long i = (long long)e * 1024 + tid;
+    if (i < per_env) {
+      const double d = __dsub_rn((double)key_f32(key[e]), p_low);
+      const double q0 = __dmul_rn(d, rcp);
+      double v = ok ? __fma_rn(__fma_rn(-q0, span, d), rcp, q0) : 0.0;
+      v = fmin(fmax(v, 0.0), 1.0);
+      store_norm(dst + i, v);
     }
   }
 }
