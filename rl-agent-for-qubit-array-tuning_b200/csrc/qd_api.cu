@@ -22,6 +22,37 @@
 static_assert(sizeof(qd_scan) == 480, "qd_scan must be 480 bytes (multiple of 16 for the TMA bulk copy)");
 static_assert(sizeof(qd_scan) % 16 == 0, "qd_scan size");
 
+// The slot layouts of the kernels, for every algorithm, dot count and voltage / gate count: the TMA destinations
+// (record, descriptor) 16-byte aligned and the record a multiple of 16 bytes, the mbarrier 8-byte aligned, the regions
+// read as double2 (projection-cache matrices and affine forms, Q rows of the record, vq) 16-byte aligned, and the slots
+// of the most warps a launch gives a CTA (4; the relax kernel: one slot per CTA) within the 227 KB a block may have.
+constexpr bool slot_layouts_hold() {
+  constexpr int W = 4, SMEM = 227 * 1024;
+  const auto staged = [](const auto& S) {          // a slot that stages the record and the descriptor by TMA
+    return S.rec_bytes % 16 == 0 && (S.rec_bytes + S.scan) % 16 == 0 && (S.rec_bytes + S.bar) % 8 == 0 &&
+           S.bytes * W <= SMEM;
+  };
+  const auto at16 = [](const auto& S, int region) { return (S.rec_bytes + region) % 16 == 0; };
+  for (int alg = QD_ALG_DEFAULT; alg <= QD_ALG_TUNNEL; ++alg)
+    for (int n = 1; n <= QD_MAX_DOTS; ++n)
+      for (int g = 1; g <= QD_MAX_VOLT; ++g)
+        for (int nv = g; nv <= QD_MAX_VOLT; ++nv) {
+          const qd_layout L = qd_make_layout(n, nv, g, alg, 32, 1);
+          const qd::ScanSlot a = qd::qd_scan_slot(L);
+          const qd::FastSlot f = qd::qd_fast_slot(L);
+          const qd::TunnelSlot t = qd::qd_tunnel_slot(L);
+          const qd::EigenSlot e = qd::qd_tunnel_eigen_slot(L);
+          if (!(L.o_q % 2 == 0 && staged(a) && at16(a, a.pc_mats) && at16(a, a.pc_aff) && staged(f) &&
+                at16(f, f.pc_mats) && at16(f, f.pc_aff) && staged(t) && at16(t, t.vq) &&
+                staged(qd::qd_tunnel_select_slot(L)) && staged(e) && at16(e, e.vq) &&
+                qd::qd_tunnel_relax_slot(L).bytes <= SMEM && qd::qd_tunnel_select2_slot().bytes * W <= SMEM &&
+                qd::qd_tunnel_eigen2_slot(n).bytes * W <= SMEM))
+            return false;
+        }
+  return true;
+}
+static_assert(slot_layouts_hold(), "a shared-memory slot layout breaks an alignment or size invariant");
+
 struct qd_ctx {
   int device = 0;
   int sm_count = 0;
@@ -236,21 +267,29 @@ PixelItems plan_pixel_items(const qd_ctx* ctx, qd::KArgs& a, long long max_pix, 
   return {warps, (items + warps - 1) / warps};
 }
 
-// One stage of the split tunnel pipeline: a primary kernel and the older kernel it falls back on.  `primary` (nullptr
+// A kernel that gives each warp a slot of dynamic shared memory, with the size of that slot (its layout's `bytes`).
+struct SlotKernel { kernel_fn fn; int slot_bytes; };
+
+// Enqueue a SlotKernel with `warps` warps per CTA: its warps' stride is its own slot size.
+int issue_slots(qd_ctx* ctx, const SlotKernel& k, long long grid, int warps, cudaStream_t stream, qd::KArgs a) {
+  a.slot_bytes = k.slot_bytes;
+  return issue(ctx, k.fn, grid, warps * 32, (size_t)k.slot_bytes * warps, stream, a);
+}
+
+// One stage of the split tunnel pipeline: a primary kernel and the older kernel it falls back on.  `primary` (no fn
 // when it does not apply or a switch turns it off) runs with the arguments `pa` and marks the pixels it could not do;
 // `fallback` then redoes only those (fix-up mode), or does every pixel when there is no primary.  fix = false skips
 // the second launch and leaves the marks in place.  `g` holds the items of plan_pixel_items.
-int primary_then_fixup(qd_ctx* ctx, const qd::KArgs& g, const PixelItems& p, kernel_fn primary, const qd::KArgs& pa,
-                       kernel_fn fallback, int fallback_slot_bytes, bool fix, cudaStream_t stream) {
-  if (primary) {
-    const int rc = issue(ctx, primary, p.grid, p.warps * 32, (size_t)pa.slot_bytes * p.warps, stream, pa);
+int primary_then_fixup(qd_ctx* ctx, const qd::KArgs& g, const PixelItems& p, const SlotKernel& primary,
+                       const qd::KArgs& pa, const SlotKernel& fallback, bool fix, cudaStream_t stream) {
+  if (primary.fn) {
+    const int rc = issue_slots(ctx, primary, p.grid, p.warps, stream, pa);
     if (rc) return rc;
   }
   if (!fix) return QD_OK;
   qd::KArgs fa = g;
-  fa.slot_bytes = fallback_slot_bytes;
   long long grid = p.grid;
-  if (primary) {
+  if (primary.fn) {
     // items of 8 pixels (no state is carried between marked pixels), so that a stretch of marked pixels is spread over
     // several warps; mark_ppi carries the marking kernel's item length to the mark look-up
     fa.fixup = 1;
@@ -261,15 +300,16 @@ int primary_then_fixup(qd_ctx* ctx, const qd::KArgs& g, const PixelItems& p, ker
     // (almost every item is skipped on its mark: a resident-size grid looping over the items instead of one CTA per four)
     grid = std::min<long long>(grid, (long long)ctx->sm_count * 32);
   }
-  return issue(ctx, fallback, grid, p.warps * 32, (size_t)fa.slot_bytes * p.warps, stream, fa);
+  return issue_slots(ctx, fallback, grid, p.warps, stream, fa);
 }
 
 // Path B: the tunnel-coupled ground state <n> of every pixel into d_nbar, for the scan kernel's latching / sensor / noise
 int tunnel_ground_state(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, const double* d_points, unsigned flags,
                         cudaStream_t stream) {
   const int N = ctx->L.n_dot;
-  const kernel_fn gs = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_gs_kernel<decltype(n)::value>; });
-  if (!gs) return fail(ctx, QD_ERR_UNSUPPORTED, "tunnel path needs 2..8 dots, got %d", N);
+  const SlotKernel gs{pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_gs_kernel<decltype(n)::value>; }),
+                      qd::qd_tunnel_slot(ctx->L).bytes};
+  if (!gs.fn) return fail(ctx, QD_ERR_UNSUPPORTED, "tunnel path needs 2..8 dots, got %d", N);
   int rc = grow(ctx, &ctx->d_nbar, &ctx->nbar_cap, (size_t)ctx->up_pixels * N * sizeof(double));
   if (rc) return rc;
   qd::KArgs g;
@@ -283,28 +323,31 @@ int tunnel_ground_state(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, const d
   const char* mono_e = getenv("QDSIM_TUNNEL_MONO");
   if (mono_e && mono_e[0] == '1') {
     // the single-kernel form (one warp per pixel does everything): kept as the A/B reference of the split pipeline
-    g.slot_bytes = qd::qd_tunnel_slot_bytes(ctx->L);
     const PixelItems p = plan_pixel_items(ctx, g, max_pix, 12);
-    return issue(ctx, gs, p.grid, p.warps * 32, (size_t)g.slot_bytes * p.warps, stream, g);
+    return issue_slots(ctx, gs, p.grid, p.warps, stream, g);
   }
   // split pipeline R -> S -> E over chunks of scans (8 + 128 + 256 bytes of scratch per pixel of a chunk)
   const kernel_fn kr = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_relax_kernel<decltype(n)::value>; });
-  const kernel_fn ks = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_select_kernel<decltype(n)::value>; });
-  const kernel_fn ke = pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen_kernel<decltype(n)::value>; });
+  const SlotKernel ks{pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_select_kernel<decltype(n)::value>; }),
+                      qd::qd_tunnel_select_slot(ctx->L).bytes};
+  const SlotKernel ke{pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen_kernel<decltype(n)::value>; }),
+                      qd::qd_tunnel_eigen_slot(ctx->L).bytes};
   // S: the lattice-enumeration kernel first (four dots and more: fewer than 32 candidates can be valid below four dots,
   // and the block walk pads; QDSIM_SELECT=block skips it), then the block walk -- as the fix-up pass over the pixels the
   // enumeration marked, or for everything
   const char* sel_e = getenv("QDSIM_SELECT");
-  const kernel_fn ks2 = (sel_e && sel_e[0] == 'b')
-                            ? nullptr
-                            : pick_dots<4>(N, [](auto n) { return qd::qd_tunnel_select2_kernel<decltype(n)::value>; });
+  const SlotKernel ks2{(sel_e && sel_e[0] == 'b')
+                           ? nullptr
+                           : pick_dots<4>(N, [](auto n) { return qd::qd_tunnel_select2_kernel<decltype(n)::value>; }),
+                       qd::qd_tunnel_select2_slot().bytes};
   // E: the Noda-iteration kernel first (QDSIM_EIGEN=householder skips it); what it could not do (sectors of more
   // than 16 states, no convergence) is marked with a NaN and redone by the Householder kernel in fix-up mode
   const char* eig_e = getenv("QDSIM_EIGEN");
   const bool no_fixup = eig_e && eig_e[0] == 'n';          // (measurement only: leaves the NaN marks in place)
-  const kernel_fn ke2 = (eig_e && eig_e[0] == 'h')
-                            ? nullptr
-                            : pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen2_kernel<decltype(n)::value>; });
+  const SlotKernel ke2{(eig_e && eig_e[0] == 'h')
+                           ? nullptr
+                           : pick_dots<2>(N, [](auto n) { return qd::qd_tunnel_eigen2_kernel<decltype(n)::value>; }),
+                       qd::qd_tunnel_eigen2_slot(N).bytes};
   long long chunk_pix = 8LL << 20;
   if (const char* e = getenv("QDSIM_TUNNEL_CHUNK_PIX")) chunk_pix = atoll(e) > 0 ? atoll(e) : chunk_pix;
   const long long spc = std::min<long long>(std::max<long long>(chunk_pix / max_pix, 1), n_scan);   // scans per chunk
@@ -325,21 +368,18 @@ int tunnel_ground_state(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, const d
     qd::KArgs r = g;
     r.rows_per_item = (int)std::min<long long>(1024, max_pix);
     r.items_per_scan = (int)((max_pix + r.rows_per_item - 1) / r.rows_per_item);
-    rc = issue(ctx, kr, (long long)r.n_scan * r.items_per_scan, 128, qd::qd_tunnel_relax_smem_bytes(ctx->L), stream, r);
+    rc = issue(ctx, kr, (long long)r.n_scan * r.items_per_scan, 128, qd::qd_tunnel_relax_slot(ctx->L).bytes, stream, r);
     if (rc) return rc;
     // S and E: one warp per pixel
     const PixelItems p = plan_pixel_items(ctx, g, max_pix, 16);
-    qd::KArgs sa = g;
-    sa.slot_bytes = qd::qd_tunnel_select2_slot_bytes(ctx->L);
-    rc = primary_then_fixup(ctx, g, p, ks2, sa, ks, qd::qd_tunnel_select_slot_bytes(ctx->L), true, stream);
+    rc = primary_then_fixup(ctx, g, p, ks2, g, ks, true, stream);
     if (rc) return rc;
     qd::KArgs ea = g;
     ea.e2_kappa = 4.0f; ea.e2_qsafe = 4.0f; ea.e2_tol = 2e-10f;
     if (const char* e = getenv("QDSIM_E2_KAPPA")) ea.e2_kappa = (float)atof(e);
     if (const char* e = getenv("QDSIM_E2_QSAFE")) ea.e2_qsafe = (float)atof(e);
     if (const char* e = getenv("QDSIM_E2_TOL")) ea.e2_tol = (float)atof(e);
-    ea.slot_bytes = qd::qd_tunnel_eigen2_slot_bytes(ctx->L);
-    rc = primary_then_fixup(ctx, g, p, ke2, ea, ke, qd::qd_tunnel_eigen_slot_bytes(ctx->L), !no_fixup, stream);
+    rc = primary_then_fixup(ctx, g, p, ke2, ea, ke, !no_fixup, stream);
     if (rc) return rc;
   }
   return QD_OK;
@@ -351,10 +391,12 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
   int rc = order_after_last_launch(ctx, stream);     // the scratch of an earlier launch on another stream
   if (rc) return rc;
   const bool fast = use_fast_kernel(ctx->L, flags, d_points != nullptr);
-  const kernel_fn fn =
-      fast ? pick_dots<1>(ctx->L.n_dot, [](auto n) { return qd::qd_scan_fast_kernel<decltype(n)::value>; })
-           : pick_kernel(ctx->L, flags, d_points != nullptr);
-  if (!fn) return fail(ctx, QD_ERR_UNSUPPORTED, "no kernel for n_dot=%d algorithm=%d", ctx->L.n_dot, ctx->L.algorithm);
+  const SlotKernel k =
+      fast ? SlotKernel{pick_dots<1>(ctx->L.n_dot, [](auto n) { return qd::qd_scan_fast_kernel<decltype(n)::value>; }),
+                        qd::qd_fast_slot(ctx->L).bytes}
+           : SlotKernel{pick_kernel(ctx->L, flags, d_points != nullptr), qd::qd_scan_slot(ctx->L).bytes};
+  if (!k.fn)
+    return fail(ctx, QD_ERR_UNSUPPORTED, "no kernel for n_dot=%d algorithm=%d", ctx->L.n_dot, ctx->L.algorithm);
   qd::KArgs a;
   memset(&a, 0, sizeof(a));
   if (ctx->L.algorithm == QD_ALG_TUNNEL) {
@@ -374,7 +416,6 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
   a.flags = flags;
   a.status = ctx->d_status;
   if (h_one && ctx->L.algorithm != QD_ALG_TUNNEL) { a.use_one = 1; a.one = *h_one; }
-  a.slot_bytes = fast ? qd::qd_fast_slot_bytes(ctx->L) : qd::qd_slot_bytes(ctx->L);
   // item = block of rows of one scan handled by one warp.  Large batches: one scan per warp (staging amortised over
   // the whole scan).  Small batches: split rows so that every SM gets work.  A flat (carry-rows) pass is sequential
   // over the whole scan by definition.
@@ -404,7 +445,7 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
   // one warp per CTA and lets the hardware scheduler balance (16 CTAs of 11.9 KB per SM).  QDSIM_WPC overrides (A/B).
   int wpc = (total_items < (long long)ctx->sm_count * 4) ? 1 : (fast ? 1 : QD_CTA_WARPS);
   if (const char* e = getenv("QDSIM_WPC")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4) wpc = v; }
-  rc = issue(ctx, fn, (total_items + wpc - 1) / wpc, wpc * 32, (size_t)a.slot_bytes * wpc, stream, a);
+  rc = issue_slots(ctx, k, (total_items + wpc - 1) / wpc, wpc, stream, a);
   if (rc) return rc;
   return mark_launch(ctx, stream);
 }

@@ -57,22 +57,21 @@ struct KArgs {
   unsigned flags;
   int rows_per_item;
   int items_per_scan;
-  int slot_bytes;
+  int slot_bytes;                      // warps' stride in dynamic shared memory: `bytes` of the kernel's slot layout
   int col_parts;                       // items per row block along x (> 1 only when nothing is carried along a row: no
                                        // latching, telegraph or 1/f chain) -- small launches spread over more SMs
 };
 
-constexpr int QD_DER_DOUBLES = 48;  // derived per-item block: g0[8] gx[8] gy[8] us0 usx usy pad[5] carry[8] + spare
-constexpr int QD_PC_DOUBLES = 8 * 64 + 8 * 16 + 8 + 8 * 32 + 8 * 24;   // projection cache: 8 matrices, inversion scratch, keys + meta; per-lane lin[8]; affine forms
-
-constexpr int QD_BF_DOUBLES = 8 + 64 + 8;   // brute force, per item: d[8], U[64] of the PERMUTED cdd_inv, perm / inverse perm (16 ints)
-
-__host__ __device__ inline int qd_slot_bytes(const qd_layout& L) {
-  int b = L.rec_doubles * 8 + (int)sizeof(qd_scan) + QD_DER_DOUBLES * 8 + 16;
-  if (L.algorithm == QD_ALG_DEFAULT || L.algorithm == QD_ALG_THRESHOLDED) b += QD_PC_DOUBLES * 8;
-  if (L.algorithm == QD_ALG_BRUTE_FORCE) b += QD_BF_DOUBLES * 8;
-  return (b + 127) & ~127;
-}
+// Each kernel that gives every warp (the relax kernel: every CTA) its own slot of dynamic shared memory describes the
+// slot in ONE layout function, qd_scan_slot, qd_fast_slot or qd_tunnel_*_slot.  A slot starts with the part of the
+// env's record the kernel stages, the one region whose size is known at run time only; every other region has a fixed
+// size.  The layout gives the record's length `rec_bytes`, the byte offset of every other region from the END of the
+// record, and `bytes`, the slot's size (rounded up to 128 bytes where warps share a CTA), which the launch multiplies
+// by the warps of a CTA and passes as KArgs.slot_bytes, the warps' stride.  A kernel's region pointers are
+// slot + rec_bytes + offset: the offsets are compile-time constants there, so the kernel does the address arithmetic of
+// a hand-written carve.  Only `bytes` depends on the algorithm, and only the host reads it.  qd_api.cu checks every
+// layout at compile time.
+__host__ __device__ constexpr int qd_slot_round(size_t bytes) { return (int)((bytes + 127) & ~(size_t)127); }
 
 // ---------------------------------------------------------------------------------------------------------------
 // Exact continuous relaxation: min (n-g)^T cdd^{-1} (n-g), n >= 0  (monotone active set on the M-matrix cdd;
@@ -846,6 +845,47 @@ __device__ __forceinline__ float radial_amp(const qd_scan* sc, double fx, double
   return fminf(fmaxf((float)sc->rad_alpha * (dist - (float)sc->rad_zero_radius), 0.0f), (float)sc->rad_max_amp);
 }
 
+// Slot of qd_scan_kernel.  The projection cache (default / thresholded) and the brute-force block start at the same
+// offset: an instance has one of them, or neither (QD_ALG_TUNNEL), and `bytes` counts only the one it has.
+struct ScanSlot {
+  size_t rec_bytes;   // [rec_doubles] the env's record (TMA destination); the offsets below count from its end
+  int scan;           // qd_scan, the descriptor (TMA destination)
+  int der;            // [48] per item: g0[8] gx[8] gy[8] us0 usx usy pad[5] | carry[8] | 1/f chain states[4] pad[4]
+  int bar;            // mbarrier of the two copies (16 bytes)
+  int pc_mats;        // projection cache: [QD_PC_WAYS][64] P_S matrices (mat_stride = 64), read as double2
+  int pc_aug;         // [8][16] scratch of the cooperative inversion
+  int pc_keys;        // u32 keys[QD_PC_WAYS], then u32 meta[2] (entries in use, next victim): 8 doubles reserved
+  int pc_meta;
+  int pc_lin;         // [8][32] per-lane copy of the linear coefficients
+  int pc_aff;         // [QD_PC_WAYS][24] affine forms P_S g0, P_S gx, P_S gy, read as double2
+  int bf_ud;          // brute force, per item: d[8] and U[64] of the PERMUTED cdd_inv
+  int bf_pm;          // int[16] perm / inverse perm: 8 doubles reserved
+  int bytes;
+};
+__host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L) {
+  ScanSlot S{};
+  S.rec_bytes = (size_t)L.rec_doubles * 8;
+  int o = 0;
+  S.scan = o;     o += (int)sizeof(qd_scan);
+  S.der = o;      o += 48 * 8;
+  S.bar = o;      o += 16;
+  const int pc_or_bf = o;             // QD_ALG_TUNNEL has neither: its slot ends here
+  S.pc_mats = o;  o += QD_PC_WAYS * 64 * 8;
+  S.pc_aug = o;   o += 8 * 16 * 8;
+  S.pc_keys = o;  S.pc_meta = o + QD_PC_WAYS * 4;   o += 8 * 8;
+  S.pc_lin = o;   o += 8 * 32 * 8;
+  S.pc_aff = o;   o += QD_PC_WAYS * 24 * 8;
+  const int pc_end = o;
+  o = pc_or_bf;
+  S.bf_ud = o;    o += 72 * 8;
+  S.bf_pm = o;    o += 8 * 8;
+  const int bf_end = o;
+  const bool has_pc = L.algorithm == QD_ALG_DEFAULT || L.algorithm == QD_ALG_THRESHOLDED;
+  const bool has_bf = L.algorithm == QD_ALG_BRUTE_FORCE;
+  S.bytes = qd_slot_round(S.rec_bytes + (has_pc ? pc_end : has_bf ? bf_end : pc_or_bf));
+  return S;
+}
+
 // THERMAL = false instantiations carry no Boltzmann-average code at all (the hard-argmin kernels are the hot ones; the
 // launch picks THERMAL = true only when QD_FLAG_THERMAL is set).
 // POINTS = true: explicit voltage list (a.points) instead of the affine descriptor -- the single-device entry points.
@@ -859,24 +899,26 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   const int NV = L.n_volt;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  const ScanSlot S = qd_scan_slot(L);
+  unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(slot + (size_t)L.rec_doubles * 8);
-  double* der = reinterpret_cast<double*>(slot + (size_t)L.rec_doubles * 8 + sizeof(qd_scan));
-  uint64_t* bar = reinterpret_cast<uint64_t*>(der + QD_DER_DOUBLES);
+  qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
+  double* der = reinterpret_cast<double*>(tail + S.der);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(tail + S.bar);
   double* d_g0 = der;
   double* d_gx = der + 8;
   double* d_gy = der + 16;
   double* d_us = der + 24;      // us0, usx, usy
   double* d_carry = der + 32;   // latched configuration of the last pixel of the previous chunk
   ProjCache pc;
-  double* bf_ud = reinterpret_cast<double*>(bar + 2);            // brute force: per-item factor of the permuted cdd_inv
-  int* bf_pm = reinterpret_cast<int*>(bf_ud + 72);
-  pc.mats = reinterpret_cast<double*>(bar + 2);
-  pc.aug = pc.mats + 8 * 64;
-  pc.keys = reinterpret_cast<uint32_t*>(pc.aug + 8 * 16);
-  pc.meta = pc.keys + QD_PC_WAYS;
-  pc.lin_s = pc.aug + 8 * 16 + 8;
-  pc.aff = pc.lin_s + 8 * 32;
+  double* bf_ud = reinterpret_cast<double*>(tail + S.bf_ud);     // brute force: per-item factor of the permuted cdd_inv
+  int* bf_pm = reinterpret_cast<int*>(tail + S.bf_pm);
+  pc.mats = reinterpret_cast<double*>(tail + S.pc_mats);
+  pc.aug = reinterpret_cast<double*>(tail + S.pc_aug);
+  pc.keys = reinterpret_cast<uint32_t*>(tail + S.pc_keys);
+  pc.meta = reinterpret_cast<uint32_t*>(tail + S.pc_meta);
+  pc.lin_s = reinterpret_cast<double*>(tail + S.pc_lin);
+  pc.aff = reinterpret_cast<double*>(tail + S.pc_aff);
   pc.gsrc = POINTS ? nullptr : der;
   pc.mat_stride = 64;
 
@@ -1234,12 +1276,37 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
 #ifndef QD_FAST_MIN_BLOCKS
 #define QD_FAST_MIN_BLOCKS 4
 #endif
-constexpr int QD_FAST_DER = 32;     // g0[8] gx[8] gy[8] us[3] sg[3] pad[2]
-constexpr int QD_FAST_PC = 64 + 8 * 16 + 8 + 8 * 32 + QD_PC_WAYS * 24;   // scratch P, inversion scratch, keys/meta, lin, affine forms
-
-__host__ __device__ inline int qd_fast_slot_bytes(const qd_layout& L) {
-  const int b = L.rec_doubles * 8 + (int)sizeof(qd_scan) + (QD_FAST_DER + 32 + QD_FAST_PC) * 8 + 16;
-  return (b + 127) & ~127;
+// Slot of qd_scan_fast_kernel.  Its projection cache keeps the affine forms only: ONE scratch matrix for building them
+// (mat_stride = 0), not QD_PC_WAYS matrices as in qd_scan_slot.
+struct FastSlot {
+  size_t rec_bytes;   // [rec_doubles] the env's record (TMA destination); the offsets below count from its end
+  int scan;           // qd_scan, the descriptor (TMA destination)
+  int der;            // [32] derived per-item block: g0[8] gx[8] gy[8] us[3] sg[3] pad[2]
+  int swt;            // [32] sum of w over the set LOW bits (dots N-1 .. N-4) [0..15], over the set HIGH bits [16..31]
+  int pc_mats;        // projection cache: [64] one scratch matrix, read as double2
+  int pc_aug;         // [8][16] scratch of the cooperative inversion
+  int pc_keys;        // u32 keys[QD_PC_WAYS], then u32 meta[2] (entries in use, next victim): 8 doubles reserved
+  int pc_meta;
+  int pc_lin;         // [8][32] per-lane copy of the linear coefficients
+  int pc_aff;         // [QD_PC_WAYS][24] affine forms P_S g0, P_S gx, P_S gy, read as double2
+  int bar;            // mbarrier of the two copies (16 bytes)
+  int bytes;
+};
+__host__ __device__ constexpr FastSlot qd_fast_slot(const qd_layout& L) {
+  FastSlot S{};
+  S.rec_bytes = (size_t)L.rec_doubles * 8;
+  int o = 0;
+  S.scan = o;     o += (int)sizeof(qd_scan);
+  S.der = o;      o += 32 * 8;
+  S.swt = o;      o += 32 * 8;
+  S.pc_mats = o;  o += 64 * 8;
+  S.pc_aug = o;   o += 8 * 16 * 8;
+  S.pc_keys = o;  S.pc_meta = o + QD_PC_WAYS * 4;   o += 8 * 8;
+  S.pc_lin = o;   o += 8 * 32 * 8;
+  S.pc_aff = o;   o += QD_PC_WAYS * 24 * 8;
+  S.bar = o;      o += 16;
+  S.bytes = qd_slot_round(S.rec_bytes + o);
+  return S;
 }
 
 template <int N>
@@ -1251,25 +1318,27 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_FAST_MIN_BLOCKS) qd_scan
   const qd_layout& L = a.L;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  const FastSlot S = qd_fast_slot(L);
+  unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(slot + (size_t)L.rec_doubles * 8);
-  double* der = reinterpret_cast<double*>(slot + (size_t)L.rec_doubles * 8 + sizeof(qd_scan));
+  qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
+  double* der = reinterpret_cast<double*>(tail + S.der);
   double* d_g0 = der;
   double* d_gx = der + 8;
   double* d_gy = der + 16;
   double* d_us = der + 24;      // us0, usx, usy
   double* d_sg = der + 27;      // sum_j w_j g_j: sg0, sgx, sgy
-  double* swt = der + QD_FAST_DER;     // [0..15]: sum of w over the set LOW bits (dots N-1 .. N-4); [16..31]: HIGH bits
+  double* swt = reinterpret_cast<double*>(tail + S.swt);
   ProjCache pc;
-  pc.mats = swt + 32;
-  pc.aug = pc.mats + 64;
-  pc.keys = reinterpret_cast<uint32_t*>(pc.aug + 8 * 16);
-  pc.meta = pc.keys + QD_PC_WAYS;
-  pc.lin_s = pc.aug + 8 * 16 + 8;
-  pc.aff = pc.lin_s + 8 * 32;
+  pc.mats = reinterpret_cast<double*>(tail + S.pc_mats);
+  pc.aug = reinterpret_cast<double*>(tail + S.pc_aug);
+  pc.keys = reinterpret_cast<uint32_t*>(tail + S.pc_keys);
+  pc.meta = reinterpret_cast<uint32_t*>(tail + S.pc_meta);
+  pc.lin_s = reinterpret_cast<double*>(tail + S.pc_lin);
+  pc.aff = reinterpret_cast<double*>(tail + S.pc_aff);
   pc.gsrc = der;
   pc.mat_stride = 0;
-  uint64_t* bar = reinterpret_cast<uint64_t*>(pc.aff + QD_PC_WAYS * 24);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(tail + S.bar);
 
   if (lane == 0) mbar_init(bar, 1);
   __syncwarp();

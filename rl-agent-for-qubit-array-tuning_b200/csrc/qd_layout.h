@@ -47,8 +47,8 @@ struct qd_layout {
   int32_t rec_doubles;  // total, multiple of 2 (16 bytes)
 };
 
-static inline qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int algorithm, int num_states, int chunk) {
-  qd_layout L;
+static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int algorithm, int num_states, int chunk) {
+  qd_layout L{};
   L.n_dot = n_dot; L.n_volt = n_volt; L.n_gate = n_gate; L.algorithm = algorithm;
   L.num_states = num_states; L.chunk = chunk;
   int o = 0;

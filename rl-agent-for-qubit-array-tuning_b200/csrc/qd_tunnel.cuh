@@ -28,12 +28,51 @@
 namespace qd {
 
 constexpr int QD_T_HS = 33;                       // row stride of H in shared memory (bank-conflict free)
-constexpr int QD_T_TAB = 64 + 16 + 256 + 16;      // per-item: permuted Cinv, Schur block, Qll, perm / inverse perm
-constexpr int QD_T_WORK = 32 * QD_T_HS + 9 * 32 + 64 + QD_T_TAB;   // H, dd, ee, e2, qi, ll, yy, vq | small vectors | tables
 
-__host__ __device__ inline int qd_tunnel_slot_bytes(const qd_layout& L) {
-  int b = L.gs_doubles * 8 + (int)sizeof(qd_scan) + QD_T_WORK * 8 + 16;     // record PREFIX only (qd_layout.h)
-  return (b + 127) & ~127;
+// Slot of qd_tunnel_gs_kernel (qd_kernels.cuh: slot layouts).  It stages the record's gs_doubles PREFIX only
+// (qd_layout.h).
+struct TunnelSlot {
+  size_t rec_bytes;   // [gs_doubles] the record prefix (TMA destination); the offsets below count from its end
+  int scan;           // qd_scan, the descriptor (TMA destination)
+  int H;              // [32][QD_T_HS] the Hamiltonian
+  int dd, ee, e2, qi, ll, yy;   // [32] each
+  int vq;             // [64] interleaved (v_j, q_j) of the current Householder step, read as double2, + spare row [32]
+  int vv;             // [16]
+  int gs, ns, fs, hs, ts, nb;   // [8] each
+  int Cp;             // [64] Cinv with rows / columns permuted so that the stiffest dots come first
+  int Sp;             // [16] Schur complement of the permuted high block
+  int Ql;             // [256] y^T Cp_ll y over the low digit combinations
+  int pm;             // int[16] pm[j]: dot at permuted position j, pm[8 + d]: position of dot d (16 doubles reserved)
+  int bar;            // mbarrier of the two copies (16 bytes)
+  int bytes;
+};
+__host__ __device__ constexpr TunnelSlot qd_tunnel_slot(const qd_layout& L) {
+  TunnelSlot S{};
+  S.rec_bytes = (size_t)L.gs_doubles * 8;
+  int o = 0;
+  S.scan = o;     o += (int)sizeof(qd_scan);
+  S.H = o;        o += 32 * QD_T_HS * 8;
+  S.dd = o;       o += 32 * 8;
+  S.ee = o;       o += 32 * 8;
+  S.e2 = o;       o += 32 * 8;
+  S.qi = o;       o += 32 * 8;
+  S.ll = o;       o += 32 * 8;
+  S.yy = o;       o += 32 * 8;
+  S.vq = o;       o += 96 * 8;
+  S.vv = o;       o += 16 * 8;
+  S.gs = o;       o += 8 * 8;
+  S.ns = o;       o += 8 * 8;
+  S.fs = o;       o += 8 * 8;
+  S.hs = o;       o += 8 * 8;
+  S.ts = o;       o += 8 * 8;
+  S.nb = o;       o += 8 * 8;
+  S.Cp = o;       o += 64 * 8;
+  S.Sp = o;       o += 16 * 8;
+  S.Ql = o;       o += 256 * 8;
+  S.pm = o;       o += 16 * 8;
+  S.bar = o;      o += 16;
+  S.bytes = qd_slot_round(S.rec_bytes + o);
+  return S;
 }
 
 // Scales of the voltage-dependent capacitance models (voltage_dependent_capacitance.py:78-125; include/qdsim.h enum
@@ -166,30 +205,30 @@ __global__ void __launch_bounds__(128, 3) qd_tunnel_gs_kernel(const KArgs a) {
   __syncthreads();
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  const TunnelSlot S = qd_tunnel_slot(L);
+  unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(slot + (size_t)L.gs_doubles * 8);
-  double* wk = reinterpret_cast<double*>(slot + (size_t)L.gs_doubles * 8 + sizeof(qd_scan));
-  double* H = wk;
-  double* dd = wk + 32 * QD_T_HS;
-  double* ee = dd + 32;
-  double* e2 = ee + 32;
-  double* qi = e2 + 32;
-  double* ll = qi + 32;
-  double* yy = ll + 32;
-  double* vq = yy + 32;          // interleaved (v_j, q_j) of the current Householder step, 64 doubles
-  double* sv = vq + 96;          // (one spare row) small vectors: vv[16] gs[8] ns[8] fs[8] hs[8] ts[8] nb[8]
-  double* vv = sv;
-  double* gs = sv + 16;
-  double* ns = sv + 24;
-  double* fs = sv + 32;
-  double* hs = sv + 40;
-  double* ts = sv + 48;
-  double* nb = sv + 56;
-  double* Cp = sv + 64;          // Cinv with rows / columns permuted so that the stiffest dots come first
-  double* Sp = Cp + 64;          // Schur complement of the permuted high block
-  double* Ql = Sp + 16;          // y^T Cp_ll y over the low digit combinations
-  int* pm = reinterpret_cast<int*>(Ql + 256);   // pm[j]: dot at permuted position j;  pm[8 + d]: position of dot d
-  uint64_t* bar = reinterpret_cast<uint64_t*>(wk + QD_T_WORK);
+  qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
+  double* H = reinterpret_cast<double*>(tail + S.H);
+  double* dd = reinterpret_cast<double*>(tail + S.dd);
+  double* ee = reinterpret_cast<double*>(tail + S.ee);
+  double* e2 = reinterpret_cast<double*>(tail + S.e2);
+  double* qi = reinterpret_cast<double*>(tail + S.qi);
+  double* ll = reinterpret_cast<double*>(tail + S.ll);
+  double* yy = reinterpret_cast<double*>(tail + S.yy);
+  double* vq = reinterpret_cast<double*>(tail + S.vq);
+  double* vv = reinterpret_cast<double*>(tail + S.vv);
+  double* gs = reinterpret_cast<double*>(tail + S.gs);
+  double* ns = reinterpret_cast<double*>(tail + S.ns);
+  double* fs = reinterpret_cast<double*>(tail + S.fs);
+  double* hs = reinterpret_cast<double*>(tail + S.hs);
+  double* ts = reinterpret_cast<double*>(tail + S.ts);
+  double* nb = reinterpret_cast<double*>(tail + S.nb);
+  double* Cp = reinterpret_cast<double*>(tail + S.Cp);
+  double* Sp = reinterpret_cast<double*>(tail + S.Sp);
+  double* Ql = reinterpret_cast<double*>(tail + S.Ql);
+  int* pm = reinterpret_cast<int*>(tail + S.pm);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(tail + S.bar);
 
   const double* __restrict__ C = rec + L.o_cinv;
   const double INF = __longlong_as_double(0x7ff0000000000000LL);
@@ -771,18 +810,83 @@ __global__ void __launch_bounds__(128, 3) qd_tunnel_gs_kernel(const KArgs a) {
 //   E  qd_tunnel_eigen_kernel   one warp per pixel: Hamiltonian in total-charge sectors, ground eigenvector, <n>
 // Scratch between them: 8 + 256 bytes per pixel of the current chunk of scans (the launcher cuts large batches).
 // =====================================================================================================================
-constexpr int QD_TS_SMALL = 16 + 8 + 8 + 8 + 8 + 16;     // vv[16] gs[8] ns[8] fs[8] hs[8] pad (select kernel)
-constexpr int QD_TS_WORK = QD_TS_SMALL + QD_T_TAB;
-constexpr int QD_TE_WORK = 32 * QD_T_HS + 6 * 32 + 72 + 32;   // H | dd ee e2 qi ll yy | vq | vv[16] gs[8] ts[8] (eigen kernel)
+// Slots of the three kernels (qd_kernels.cuh: slot layouts).  Each stages the record's gs_doubles prefix only.
+struct RelaxSlot {    // one per CTA
+  size_t rec_bytes;   // [gs_doubles] the record prefix; the offsets below count from its end
+  int scan;           // qd_scan, the descriptor
+  int bytes;          // (not rounded)
+};
+__host__ __device__ constexpr RelaxSlot qd_tunnel_relax_slot(const qd_layout& L) {
+  RelaxSlot S{};
+  S.rec_bytes = (size_t)L.gs_doubles * 8;
+  S.scan = 0;
+  S.bytes = (int)(S.rec_bytes + sizeof(qd_scan));
+  return S;
+}
 
-__host__ __device__ inline int qd_tunnel_select_slot_bytes(const qd_layout& L) {
-  return (L.gs_doubles * 8 + (int)sizeof(qd_scan) + QD_TS_WORK * 8 + 16 + 127) & ~127;
+struct SelectSlot {
+  size_t rec_bytes;   // [gs_doubles] the record prefix (TMA destination); the offsets below count from its end
+  int scan;           // qd_scan, the descriptor (TMA destination)
+  int vv;             // [16]
+  int gs, ns, fs, hs; // [8] each
+  int Mi;             // [9] inverse of rows / columns 1..3 of the low 4 x 4 block of Cp (NLO = 4): 16 doubles reserved
+  int Cp;             // [64] Cinv with rows / columns permuted so that the stiffest dots come first
+  int Sp;             // [16] Schur complement of the permuted high block
+  int Ql;             // [256] y^T Cp_ll y over the low digit combinations
+  int pm;             // int[16] pm[j]: dot at permuted position j, pm[8 + d]: position of dot d (16 doubles reserved)
+  int bar;            // mbarrier of the two copies (16 bytes)
+  int bytes;
+};
+__host__ __device__ constexpr SelectSlot qd_tunnel_select_slot(const qd_layout& L) {
+  SelectSlot S{};
+  S.rec_bytes = (size_t)L.gs_doubles * 8;
+  int o = 0;
+  S.scan = o;     o += (int)sizeof(qd_scan);
+  S.vv = o;       o += 16 * 8;
+  S.gs = o;       o += 8 * 8;
+  S.ns = o;       o += 8 * 8;
+  S.fs = o;       o += 8 * 8;
+  S.hs = o;       o += 8 * 8;
+  S.Mi = o;       o += 16 * 8;
+  S.Cp = o;       o += 64 * 8;
+  S.Sp = o;       o += 16 * 8;
+  S.Ql = o;       o += 256 * 8;
+  S.pm = o;       o += 16 * 8;
+  S.bar = o;      o += 16;
+  S.bytes = qd_slot_round(S.rec_bytes + o);
+  return S;
 }
-__host__ __device__ inline int qd_tunnel_eigen_slot_bytes(const qd_layout& L) {
-  return (L.gs_doubles * 8 + (int)sizeof(qd_scan) + QD_TE_WORK * 8 + 16 + 127) & ~127;
-}
-__host__ __device__ inline int qd_tunnel_relax_smem_bytes(const qd_layout& L) {
-  return L.gs_doubles * 8 + (int)sizeof(qd_scan);
+
+struct EigenSlot {
+  size_t rec_bytes;   // [gs_doubles] the record prefix (TMA destination); the offsets below count from its end
+  int scan;           // qd_scan, the descriptor (TMA destination)
+  int H;              // [32][QD_T_HS] the Hamiltonian
+  int dd, ee, e2, qi, ll, yy;   // [32] each
+  int vq;             // [64] interleaved (v_j, q_j) of the current Householder step, read as double2; + 8 spare
+  int vv;             // [16]
+  int gs, ts;         // [8] each
+  int bar;            // mbarrier of the two copies (16 bytes)
+  int bytes;
+};
+__host__ __device__ constexpr EigenSlot qd_tunnel_eigen_slot(const qd_layout& L) {
+  EigenSlot S{};
+  S.rec_bytes = (size_t)L.gs_doubles * 8;
+  int o = 0;
+  S.scan = o;     o += (int)sizeof(qd_scan);
+  S.H = o;        o += 32 * QD_T_HS * 8;
+  S.dd = o;       o += 32 * 8;
+  S.ee = o;       o += 32 * 8;
+  S.e2 = o;       o += 32 * 8;
+  S.qi = o;       o += 32 * 8;
+  S.ll = o;       o += 32 * 8;
+  S.yy = o;       o += 32 * 8;
+  S.vq = o;       o += 72 * 8;
+  S.vv = o;       o += 16 * 8;
+  S.gs = o;       o += 8 * 8;
+  S.ts = o;       o += 8 * 8;
+  S.bar = o;      o += 16;
+  S.bytes = qd_slot_round(S.rec_bytes + o);
+  return S;
 }
 
 // ---- R: relaxation, one thread per pixel ------------------------------------------------------------------------------
@@ -791,8 +895,9 @@ __global__ void __launch_bounds__(128) qd_tunnel_relax_kernel(const KArgs a) {
   extern __shared__ __align__(128) unsigned char qd_smem[];
   const qd_layout& L = a.L;
   const int NV = L.n_volt;
+  const RelaxSlot S = qd_tunnel_relax_slot(L);
   double* rec = reinterpret_cast<double*>(qd_smem);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(qd_smem + (size_t)L.gs_doubles * 8);
+  qd_scan* sc = reinterpret_cast<qd_scan*>(qd_smem + S.rec_bytes + S.scan);
   const double* __restrict__ C = rec + L.o_cinv;
   const long long total_items = (long long)a.n_scan * a.items_per_scan;
   for (long long item = blockIdx.x; item < total_items; item += gridDim.x) {
@@ -922,19 +1027,21 @@ __global__ void __launch_bounds__(128, 4) qd_tunnel_select_kernel(const KArgs a)
   const int NV = L.n_volt;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  const SelectSlot S = qd_tunnel_select_slot(L);
+  unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(slot + (size_t)L.gs_doubles * 8);
-  double* sv = reinterpret_cast<double*>(slot + (size_t)L.gs_doubles * 8 + sizeof(qd_scan));
-  double* vv = sv;
-  double* gs = sv + 16;
-  double* ns = sv + 24;
-  double* fs = sv + 32;
-  double* hs = sv + 40;
-  double* Cp = sv + QD_TS_SMALL;  // Cinv with rows / columns permuted so that the stiffest dots come first
-  double* Sp = Cp + 64;           // Schur complement of the permuted high block
-  double* Ql = Sp + 16;           // y^T Cp_ll y over the low digit combinations
-  int* pm = reinterpret_cast<int*>(Ql + 256);   // pm[j]: dot at permuted position j;  pm[8 + d]: position of dot d
-  uint64_t* bar = reinterpret_cast<uint64_t*>(sv + QD_TS_WORK);
+  qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
+  double* vv = reinterpret_cast<double*>(tail + S.vv);
+  double* gs = reinterpret_cast<double*>(tail + S.gs);
+  double* ns = reinterpret_cast<double*>(tail + S.ns);
+  double* fs = reinterpret_cast<double*>(tail + S.fs);
+  double* hs = reinterpret_cast<double*>(tail + S.hs);
+  double* mi = reinterpret_cast<double*>(tail + S.Mi);
+  double* Cp = reinterpret_cast<double*>(tail + S.Cp);
+  double* Sp = reinterpret_cast<double*>(tail + S.Sp);
+  double* Ql = reinterpret_cast<double*>(tail + S.Ql);
+  int* pm = reinterpret_cast<int*>(tail + S.pm);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(tail + S.bar);
 
   const double* __restrict__ C = rec + L.o_cinv;
   const double INF = __longlong_as_double(0x7ff0000000000000LL);
@@ -1041,7 +1148,7 @@ __global__ void __launch_bounds__(128, 4) qd_tunnel_select_kernel(const KArgs a)
           const double c11 = a22 * a33 - a23 * a23, c12 = a13 * a23 - a12 * a33, c13 = a12 * a23 - a13 * a22;
           const double c22 = a11 * a33 - a13 * a13, c23 = a12 * a13 - a11 * a23, c33 = a11 * a22 - a12 * a12;
           const double idet = 1.0 / (a11 * c11 + a12 * c12 + a13 * c13);
-          double* Mi = sv + 48;
+          double* Mi = mi;
           Mi[0] = c11 * idet; Mi[1] = c12 * idet; Mi[2] = c13 * idet;
           Mi[3] = c12 * idet; Mi[4] = c22 * idet; Mi[5] = c23 * idet;
           Mi[6] = c13 * idet; Mi[7] = c23 * idet; Mi[8] = c33 * idet;
@@ -1210,7 +1317,7 @@ __global__ void __launch_bounds__(128, 4) qd_tunnel_select_kernel(const KArgs a)
         const double base_lane = tunnel_lane_part<NLO>(base, c, lane);      // lane part, once per block
         double alpha_b = 0.0, beta_b = 0.0, gamma_b = 0.0;
         if constexpr (NLO == 4) {
-          const double* __restrict__ Mi = sv + 48;
+          const double* __restrict__ Mi = mi;
           const double u0 = fma(Mi[0], c[1], fma(Mi[1], c[2], Mi[2] * c[3]));
           const double u1 = fma(Mi[3], c[1], fma(Mi[4], c[2], Mi[5] * c[3]));
           const double u2 = fma(Mi[6], c[1], fma(Mi[7], c[2], Mi[8] * c[3]));
@@ -1301,21 +1408,22 @@ __global__ void __launch_bounds__(128, QD_TE_MIN_BLOCKS) qd_tunnel_eigen_kernel(
   __syncthreads();
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  const EigenSlot S = qd_tunnel_eigen_slot(L);
+  unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
-  qd_scan* sc = reinterpret_cast<qd_scan*>(slot + (size_t)L.gs_doubles * 8);
-  double* wk = reinterpret_cast<double*>(slot + (size_t)L.gs_doubles * 8 + sizeof(qd_scan));
-  double* H = wk;
-  double* dd = wk + 32 * QD_T_HS;
-  double* ee = dd + 32;
-  double* e2 = ee + 32;
-  double* qi = e2 + 32;
-  double* ll = qi + 32;
-  double* yy = ll + 32;
-  double* vq = yy + 32;          // interleaved (v_j, q_j) of the current Householder step, 64 doubles (+ pad)
-  double* vv = vq + 72;
-  double* gs = vv + 16;
-  double* ts = gs + 8;
-  uint64_t* bar = reinterpret_cast<uint64_t*>(wk + QD_TE_WORK);
+  qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
+  double* H = reinterpret_cast<double*>(tail + S.H);
+  double* dd = reinterpret_cast<double*>(tail + S.dd);
+  double* ee = reinterpret_cast<double*>(tail + S.ee);
+  double* e2 = reinterpret_cast<double*>(tail + S.e2);
+  double* qi = reinterpret_cast<double*>(tail + S.qi);
+  double* ll = reinterpret_cast<double*>(tail + S.ll);
+  double* yy = reinterpret_cast<double*>(tail + S.yy);
+  double* vq = reinterpret_cast<double*>(tail + S.vq);
+  double* vv = reinterpret_cast<double*>(tail + S.vv);
+  double* gs = reinterpret_cast<double*>(tail + S.gs);
+  double* ts = reinterpret_cast<double*>(tail + S.ts);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(tail + S.bar);
   const double* __restrict__ C = rec + L.o_cinv;
 
   if (lane == 0) mbar_init(bar, 1);

@@ -22,13 +22,39 @@
 namespace qd {
 
 constexpr int QD_S2_CAP = 320;                    // nodes per level list (two lists); leaves share them
-// (16 spare) rem[8] r[8] rcm[8] rc[8] dd[8] Mt[72] | Lc[64] | listP[2][CAP] | listD[2][CAP] (u32) | outk[32] (u64)
-constexpr int QD_S2_SMALL = 56 + 72;                 // + Mt[8][9]: L^T with zeros below the diagonal (row k: L_jk, j > k)
-constexpr int QD_S2_WORK = QD_S2_SMALL + 64 + 2 * QD_S2_CAP + QD_S2_CAP + 32;
 constexpr unsigned long long QD_S2_MARK = 0xfffffffffffffffeULL;      // first key of a pixel left to the fix-up pass
 
-__host__ __device__ inline int qd_tunnel_select2_slot_bytes(const qd_layout&) {
-  return (QD_S2_WORK * 8 + 127) & ~127;
+// Slot of qd_tunnel_select2_kernel (qd_kernels.cuh: slot layouts).  Nothing is staged: the potentials come from the
+// relax kernel, cdd_inv is read once per item for the factorisation, the four scalars of the scan descriptor straight
+// from global memory.  The offsets count from the start of the slot.
+struct Select2Slot {
+  int rem;            // [8] rem[k]: lower bound of the levels below k
+  int rs;             // [8] r = floor - g
+  int rcm;            // [8]
+  int rc;             // [8] rc_k = r_k + sum_{j>k} L_jk r_j
+  int dd;             // [8]
+  int Mt;             // [8][9] L^T with zeros below the diagonal: Mt[k * 9 + j] = L_jk for j > k, else 0
+  int Lc;             // [64] Lc[j * N + k] = L_jk (j > k)
+  int listP;          // [2][QD_S2_CAP]
+  int listD;          // u32 [2][QD_S2_CAP]: QD_S2_CAP doubles
+  int outk;           // u64 [32]
+  int bytes;
+};
+__host__ __device__ constexpr Select2Slot qd_tunnel_select2_slot() {
+  Select2Slot S{};
+  int o = 16 * 8;                     // (the first 16 doubles are not used)
+  S.rem = o;      o += 8 * 8;
+  S.rs = o;       o += 8 * 8;
+  S.rcm = o;      o += 8 * 8;
+  S.rc = o;       o += 8 * 8;
+  S.dd = o;       o += 8 * 8;
+  S.Mt = o;       o += 72 * 8;
+  S.Lc = o;       o += 64 * 8;
+  S.listP = o;    o += 2 * QD_S2_CAP * 8;
+  S.listD = o;    o += QD_S2_CAP * 8;
+  S.outk = o;     o += 32 * 8;
+  S.bytes = qd_slot_round(o);
+  return S;
 }
 
 // One term of the energy, the same rounded operations wherever it is formed.  Digits enter as codes c = delta + 1 in
@@ -47,19 +73,19 @@ __global__ void __launch_bounds__(128, 5) qd_tunnel_select2_kernel(const KArgs a
   const int warps_per_cta = blockDim.x >> 5;
   const qd_layout& L = a.L;
 
-  // nothing is staged: the potentials come from the relax kernel, cdd_inv is read once per item for the factorisation,
-  // the four scalars of the scan descriptor straight from global memory (9.5 KB per warp -> five CTAs per SM)
-  double* sv = reinterpret_cast<double*>(qd_smem + (size_t)warp * a.slot_bytes);
-  double* gs = sv + 16;             // rem[k]: lower bound of the levels below k
-  double* rs = sv + 24;             // r = floor - g
-  double* fs = sv + 32;             // rcm
-  double* rc = sv + 40;             // rc_k = r_k + sum_{j>k} L_jk r_j
-  double* dd = sv + 48;
-  double* Mt = sv + 56;             // Mt[k * 9 + j] = L_jk for j > k, else 0
-  double* Lc = sv + QD_S2_SMALL;    // Lc[j * N + k] = L_jk (j > k)
-  double* listP = Lc + 64;          // [2][CAP]
-  unsigned* listD = reinterpret_cast<unsigned*>(listP + 2 * QD_S2_CAP);   // [2][CAP]
-  uint64_t* outk = reinterpret_cast<uint64_t*>(listP + 2 * QD_S2_CAP + QD_S2_CAP);
+  // (9.5 KB per warp -> five CTAs per SM)
+  constexpr Select2Slot S = qd_tunnel_select2_slot();
+  unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  double* gs = reinterpret_cast<double*>(slot + S.rem);
+  double* rs = reinterpret_cast<double*>(slot + S.rs);
+  double* fs = reinterpret_cast<double*>(slot + S.rcm);
+  double* rc = reinterpret_cast<double*>(slot + S.rc);
+  double* dd = reinterpret_cast<double*>(slot + S.dd);
+  double* Mt = reinterpret_cast<double*>(slot + S.Mt);
+  double* Lc = reinterpret_cast<double*>(slot + S.Lc);
+  double* listP = reinterpret_cast<double*>(slot + S.listP);
+  unsigned* listD = reinterpret_cast<unsigned*>(slot + S.listD);
+  uint64_t* outk = reinterpret_cast<uint64_t*>(slot + S.outk);
   const double INF = __longlong_as_double(0x7ff0000000000000LL);
 
   const long long total_items = (long long)a.n_scan * a.items_per_scan;

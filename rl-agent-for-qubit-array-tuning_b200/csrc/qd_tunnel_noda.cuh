@@ -26,18 +26,40 @@
 namespace qd {
 
 constexpr int QD_E2_LS = 17;                         // row stride of the sector-local matrices (odd: conflict free)
-// Shared memory per warp: cinv[N^2] | Lm[32][17] | H17[32][17] | hash keys[64] | hash x[64].  Nothing else is staged: the
-// per-pixel potentials come from the relax kernel, the four scalars of the scan descriptor are read from global memory.
-// Lm comes FIRST: the loops of the factorisation run to a warp-uniform bound and read up to 271 doubles past a short
-// sector's rows -- with this order they land in H17 (finite numbers), and no padding is needed.  Small per-pixel vectors
-// alias the head of Lm (dead before the first factorisation): gs[8] at +16, ts[8] at +24, the sort permutation at +32,
-// the start vector of the first mat-vec at +64 (48 entries).  10.1 KB at 8 dots -> five CTAs of four warps per SM.
-constexpr int QD_E2_WORK = 2 * 32 * QD_E2_LS + 128;
 constexpr int QD_E2_MAXIT = 12;
 
-__host__ __device__ inline int qd_tunnel_eigen2_slot_bytes(const qd_layout& L) {
-  const int cinv_doubles = (L.n_dot * L.n_dot + 1) & ~1;
-  return ((cinv_doubles + QD_E2_WORK) * 8 + 127) & ~127;
+// Slot of qd_tunnel_eigen2_kernel for n_dot dots (qd_kernels.cuh: slot layouts).  Only cdd_inv is staged (by the lanes,
+// from the record): the per-pixel potentials come from the relax kernel, the four scalars of the scan descriptor are
+// read from global memory.  The offsets count from the start of the slot.  10.1 KB at 8 dots -> five CTAs of four warps
+// per SM.
+// Lm comes BEFORE H: the loops of the factorisation run to a warp-uniform bound and read up to 271 doubles past a short
+// sector's rows -- with this order they land in H (finite numbers), and no padding is needed.  Small per-pixel vectors
+// alias the head of Lm (dead before the first factorisation).
+struct Eigen2Slot {
+  int cinv;           // [n_dot^2], rounded up to an even count
+  int Lm;             // [32][QD_E2_LS] the factorisation, in place
+  int gs, ts;         // [8] each, at Lm + 16 and Lm + 24 doubles (aliases)
+  int perm;           // int[32] the sort permutation, at Lm + 32 doubles (alias)
+  int colbuf;         // [48] start vector of the first mat-vec, at Lm + 64 doubles (alias)
+  int H;              // [32][QD_E2_LS] row `lane`, columns of the lane's own sector
+  int hkey;           // u64 [64] hash keys
+  int hx;             // [64] hash values
+  int bytes;
+};
+__host__ __device__ constexpr Eigen2Slot qd_tunnel_eigen2_slot(int n_dot) {
+  Eigen2Slot S{};
+  int o = 0;
+  S.cinv = o;     o += ((n_dot * n_dot + 1) & ~1) * 8;
+  S.Lm = o;       o += 32 * QD_E2_LS * 8;
+  S.gs = S.Lm + 16 * 8;
+  S.ts = S.Lm + 24 * 8;
+  S.perm = S.Lm + 32 * 8;
+  S.colbuf = S.Lm + 64 * 8;
+  S.H = o;        o += 32 * QD_E2_LS * 8;
+  S.hkey = o;     o += 64 * 8;
+  S.hx = o;       o += 64 * 8;
+  S.bytes = qd_slot_round(o);
+  return S;
 }
 
 // 1 / x for a positive normal x: MUFU.RCP64H seed (20 bits) + two Newton steps
@@ -198,16 +220,17 @@ __global__ void __launch_bounds__(128, QD_E2_MIN_BLOCKS) qd_tunnel_eigen2_kernel
   for (int k = threadIdx.x; k < 258; k += blockDim.x) sq_tab[k] = sqrt((double)k);
   __syncthreads();
 
-  constexpr int CINV_DOUBLES = (N * N + 1) & ~1;
-  double* Csm = reinterpret_cast<double*>(qd_smem + (size_t)warp * a.slot_bytes);
-  double* Lm = Csm + CINV_DOUBLES;                  // [32][17]: the factorisation, in place
-  double* H = Lm + 32 * QD_E2_LS;                   // [32][17]: row `lane`, columns of the lane's own sector
-  double* gs = Lm + 16;                             // (aliases, dead before the first factorisation: see QD_E2_WORK)
-  double* ts = Lm + 24;
-  int* perm = reinterpret_cast<int*>(Lm + 32);
-  double* colbuf = Lm + 64;                         // start vector of the first mat-vec, [48]
-  uint64_t* hkey = reinterpret_cast<uint64_t*>(H + 32 * QD_E2_LS);       // [64]
-  double* hx = reinterpret_cast<double*>(hkey + 64);                     // [64]
+  constexpr Eigen2Slot S = qd_tunnel_eigen2_slot(N);
+  unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
+  double* Csm = reinterpret_cast<double*>(slot + S.cinv);
+  double* Lm = reinterpret_cast<double*>(slot + S.Lm);
+  double* H = reinterpret_cast<double*>(slot + S.H);
+  double* gs = reinterpret_cast<double*>(slot + S.gs);
+  double* ts = reinterpret_cast<double*>(slot + S.ts);
+  int* perm = reinterpret_cast<int*>(slot + S.perm);
+  double* colbuf = reinterpret_cast<double*>(slot + S.colbuf);
+  uint64_t* hkey = reinterpret_cast<uint64_t*>(slot + S.hkey);
+  double* hx = reinterpret_cast<double*>(slot + S.hx);
   const double* __restrict__ C = Csm;
 
   const long long total_items = (long long)a.n_scan * a.items_per_scan;
