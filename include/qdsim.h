@@ -181,6 +181,29 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
 int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const double* v, float* z_out_host,
                         void* n_out_host, int n_type, unsigned flags);
 
+/* Closed arrays: a fixed total number of carriers per scan, n_charge = sum of the dot occupations (ChargeSensedDotArray's
+ * closed methods, qarray 1.6.0).  The ground state is the closed form of the model set's algorithm: the minimiser of the
+ * free energy over the charge configurations with sum n = n_charge -- `default`: floor of the exact closed relaxation
+ * (n >= 0, sum n = n_charge) plus {0,1}^N, kept where the sum is n_charge; `brute_force`: every n in {0..n_charge}^N of that
+ * sum (max_charge_carriers unused).  Latching, sensor, noise and radial noise are those of the open path.  Same model set
+ * as the open entry points (qd_set_models); QD_ERR_UNSUPPORTED for QD_ALG_THRESHOLDED and QD_ALG_TUNNEL, QD_ERR_INVALID for
+ * an n_charge outside 0..251 (default) / 0..15 (brute_force).
+ *   n_charge  HOST, [n_scan]: total charge of each scan; copied to the device next to the descriptors (stream-ordered) */
+
+/* Replaces, per scan, ChargeSensedDotArray.do2d_closed (+ QarrayBaseClass._apply_radial_noise).  Asynchronous, DEVICE
+ * outputs, as qd_scan_open. */
+int qd_scan_closed(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out, void* n_out,
+                   int n_type, unsigned flags, void* stream);
+
+/* ChargeSensedDotArray.do2d_closed with HOST outputs, as qd_scan_open_host. */
+int qd_scan_closed_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out_host,
+                        void* n_out_host, int n_type, unsigned flags);
+
+/* ChargeSensedDotArray.ground_state_closed / charge_sensor_closed / do1d_closed on an explicit voltage list, as
+ * qd_points_open_host, with the one total charge n_charge. */
+int qd_points_closed_host(qd_ctx* ctx, const qd_scan* scan, int32_t n_charge, int ny, int nx, const double* v,
+                          float* z_out_host, void* n_out_host, int n_type, unsigned flags);
+
 /* Percentile normalisation of the observation images, per env (K8; replaces QuantumDeviceEnv._normalise_obs,
  * src/qadapt/environment/env.py:471-509): for each of n_env consecutive blocks of per_env floats,
  *   p_low, p_high = np.percentile(block, q_low_pct), np.percentile(block, q_high_pct)   (numpy 'linear' method)

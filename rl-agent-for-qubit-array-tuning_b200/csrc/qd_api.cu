@@ -39,10 +39,12 @@ constexpr bool slot_layouts_hold() {
         for (int nv = g; nv <= QD_MAX_VOLT; ++nv) {
           const qd_layout L = qd_make_layout(n, nv, g, alg, 32, 1);
           const qd::ScanSlot a = qd::qd_scan_slot(L);
+          const qd::ScanSlot ac = qd::qd_scan_slot(L, true);
           const qd::FastSlot f = qd::qd_fast_slot(L);
           const qd::TunnelSlot t = qd::qd_tunnel_slot(L);
           const qd::EigenSlot e = qd::qd_tunnel_eigen_slot(L);
-          if (!(L.o_q % 2 == 0 && staged(a) && at16(a, a.pc_mats) && at16(a, a.pc_aff) && staged(f) &&
+          if (!(L.o_q % 2 == 0 && staged(a) && at16(a, a.pc_mats) && at16(a, a.pc_aff) && staged(ac) &&
+                at16(ac, ac.pc_mats) && at16(ac, ac.pc_aff) && staged(f) &&
                 at16(f, f.pc_mats) && at16(f, f.pc_aff) && staged(t) && at16(t, t.vq) &&
                 staged(qd::qd_tunnel_select_slot(L)) && staged(e) && at16(e, e.vq) &&
                 qd::qd_tunnel_relax_slot(L).bytes <= SMEM && qd::qd_tunnel_select2_slot().bytes * W <= SMEM &&
@@ -74,6 +76,8 @@ struct qd_ctx {
   size_t n_cap = 0;
   double* d_pts = nullptr;
   size_t pts_cap = 0;
+  int32_t* d_ncharge = nullptr;   // closed launches: total charge per scan, next to d_scans (same ordering rules)
+  size_t ncharge_cap = 0;
   double* d_nbar = nullptr;       // tunnel path: <n> of every pixel between the two launches
   size_t nbar_cap = 0;
   unsigned char* d_tfloor = nullptr;   // tunnel path, split pipeline: floor(n_c) of the current chunk, 8 bytes per pixel
@@ -160,9 +164,9 @@ kernel_fn pick_dots(int n, F k) {
 }
 
 // default / thresholded search with a hard argmin on affine windows runs the restructured kernel (qd_scan_fast_kernel);
-// QDSIM_GENERIC_SCAN=1 keeps the generic one (A/B timing, and the parity tests run both)
-bool use_fast_kernel(const qd_layout& L, unsigned flags, bool points) {
-  if (points || (flags & (QD_FLAG_THERMAL | QD_FLAG_PINK))) return false;
+// QDSIM_GENERIC_SCAN=1 keeps the generic one (A/B timing, and the parity tests run both).  Closed arrays: generic only.
+bool use_fast_kernel(const qd_layout& L, unsigned flags, bool points, bool closed) {
+  if (closed || points || (flags & (QD_FLAG_THERMAL | QD_FLAG_PINK))) return false;
   if (L.algorithm != QD_ALG_DEFAULT && L.algorithm != QD_ALG_THRESHOLDED) return false;
   const char* e = getenv("QDSIM_GENERIC_SCAN");
   return !(e && e[0] == '1');
@@ -174,8 +178,14 @@ kernel_fn pick_p(int n, bool points) {
   return pick_dots<1>(n, [](auto k) { return qd::qd_scan_kernel<decltype(k)::value, ALG, THERMAL, false>; });
 }
 
-kernel_fn pick_kernel(const qd_layout& L, unsigned flags, bool points) {
+kernel_fn pick_kernel(const qd_layout& L, unsigned flags, bool points, bool closed) {
   const bool thermal = flags & QD_FLAG_THERMAL;
+  if (closed) {
+    constexpr int DC = QD_ALG_DEFAULT | qd::QD_CLOSED, BC = QD_ALG_BRUTE_FORCE | qd::QD_CLOSED;
+    if (L.algorithm == QD_ALG_BRUTE_FORCE) return thermal ? pick_p<BC, true>(L.n_dot, points) : pick_p<BC, false>(L.n_dot, points);
+    if (L.algorithm == QD_ALG_DEFAULT) return thermal ? pick_p<DC, true>(L.n_dot, points) : pick_p<DC, false>(L.n_dot, points);
+    return nullptr;
+  }
   if (L.algorithm == QD_ALG_TUNNEL) return pick_p<QD_ALG_TUNNEL, false>(L.n_dot, points);
   if (L.algorithm == QD_ALG_BRUTE_FORCE)
     return thermal ? pick_p<QD_ALG_BRUTE_FORCE, true>(L.n_dot, points) : pick_p<QD_ALG_BRUTE_FORCE, false>(L.n_dot, points);
@@ -202,6 +212,33 @@ int validate_launch(qd_ctx* ctx, int n_type, unsigned flags, const void* n_out) 
     return fail(ctx, QD_ERR_INVALID, "the tunnel path yields non-integer occupations <n>: use QD_N_F32/F64 or QD_N_NONE");
   return QD_OK;
 }
+
+// The closed entry points: supported algorithms and the range of the total charge.  default: q <= 251 keeps every dot
+// below the 252 carriers of the uint8 charge map and the latching keys; brute_force: 4 bits per dot in the walk's codes.
+int validate_closed(qd_ctx* ctx, int n_scan, const int32_t* n_charge) {
+  if (!n_charge) return fail(ctx, QD_ERR_INVALID, "n_charge is NULL");
+  const int alg = ctx->L.algorithm;
+  if (alg != QD_ALG_DEFAULT && alg != QD_ALG_BRUTE_FORCE)
+    return fail(ctx, QD_ERR_UNSUPPORTED, "closed arrays: algorithm %d is not supported (default and brute_force are)", alg);
+  const int qmax = alg == QD_ALG_BRUTE_FORCE ? 15 : 251;
+  for (int i = 0; i < n_scan; ++i)
+    if (n_charge[i] < 0 || n_charge[i] > qmax)
+      return fail(ctx, QD_ERR_INVALID, "scan %d: n_charge %d outside 0..%d", i, n_charge[i], qmax);
+  return QD_OK;
+}
+
+// Copy the total charges of a closed launch next to the descriptors (stream-ordered; the caller has already ordered
+// `stream` after the context's last launch).
+int stage_ncharge(qd_ctx* ctx, int n_scan, const int32_t* n_charge, cudaStream_t stream) {
+  int rc = grow(ctx, &ctx->d_ncharge, &ctx->ncharge_cap, (size_t)n_scan * sizeof(int32_t));
+  if (rc) return rc;
+  QD_CUDA(ctx, cudaMemcpyAsync(ctx->d_ncharge, n_charge, (size_t)n_scan * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
+  return QD_OK;
+}
+
+// Total charge of the scans of a closed launch: d_q = device array of the launch's scans, or (single-scan path, d_q
+// unused) `one` for its one scan.
+struct ClosedArgs { const int32_t* d_q; int one; };
 
 // shared-memory attributes of a kernel: set once per context (two driver calls saved per launch)
 // Function attributes belong to the CUDA context of a device, not to a qd_ctx: the table is process-wide, keyed by
@@ -387,14 +424,16 @@ int tunnel_ground_state(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, const d
 
 // enqueue one launch over device-resident descriptors
 int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const double* d_points, float* d_z, void* d_n,
-           int n_type, unsigned flags, cudaStream_t stream, int rows_cap = 0, const qd_scan* h_one = nullptr) {
+           int n_type, unsigned flags, cudaStream_t stream, int rows_cap = 0, const qd_scan* h_one = nullptr,
+           const ClosedArgs* closed = nullptr) {
   int rc = order_after_last_launch(ctx, stream);     // the scratch of an earlier launch on another stream
   if (rc) return rc;
-  const bool fast = use_fast_kernel(ctx->L, flags, d_points != nullptr);
+  const bool fast = use_fast_kernel(ctx->L, flags, d_points != nullptr, closed != nullptr);
   const SlotKernel k =
       fast ? SlotKernel{pick_dots<1>(ctx->L.n_dot, [](auto n) { return qd::qd_scan_fast_kernel<decltype(n)::value>; }),
                         qd::qd_fast_slot(ctx->L).bytes}
-           : SlotKernel{pick_kernel(ctx->L, flags, d_points != nullptr), qd::qd_scan_slot(ctx->L).bytes};
+           : SlotKernel{pick_kernel(ctx->L, flags, d_points != nullptr, closed != nullptr),
+                        qd::qd_scan_slot(ctx->L, closed != nullptr).bytes};
   if (!k.fn)
     return fail(ctx, QD_ERR_UNSUPPORTED, "no kernel for n_dot=%d algorithm=%d", ctx->L.n_dot, ctx->L.algorithm);
   qd::KArgs a;
@@ -416,6 +455,7 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
   a.flags = flags;
   a.status = ctx->d_status;
   if (h_one && ctx->L.algorithm != QD_ALG_TUNNEL) { a.use_one = 1; a.one = *h_one; }
+  if (closed) { a.n_charge = closed->d_q; a.one_n_charge = closed->one; }
   // item = block of rows of one scan handled by one warp.  Large batches: one scan per warp (staging amortised over
   // the whole scan).  Small batches: split rows so that every SM gets work.  A flat (carry-rows) pass is sequential
   // over the whole scan by definition.
@@ -683,6 +723,7 @@ void qd_destroy(qd_ctx* ctx) {
   if (ctx->d_z) cudaFree(ctx->d_z);
   if (ctx->d_n) cudaFree(ctx->d_n);
   if (ctx->d_pts) cudaFree(ctx->d_pts);
+  if (ctx->d_ncharge) cudaFree(ctx->d_ncharge);
   if (ctx->d_nbar) cudaFree(ctx->d_nbar);
   if (ctx->d_tfloor) cudaFree(ctx->d_tfloor);
   if (ctx->d_tpot) cudaFree(ctx->d_tpot);
@@ -812,15 +853,34 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
   return QD_OK;
 }
 
-int qd_scan_open(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_out, void* n_out, int n_type, unsigned flags,
-                 void* stream) {
+// qd_scan_open, and qd_scan_closed when n_charge (HOST, [n_scan]) is given
+static int scan_device(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out, void* n_out,
+                       int n_type, unsigned flags, void* stream) {
   int rc = validate_launch(ctx, n_type, flags, n_out);
   if (rc) return rc;
+  if (n_charge && (rc = validate_closed(ctx, n_scan, n_charge))) return rc;
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
   int max_ny = 0;
   rc = stage_scans(ctx, n_scan, scans, (cudaStream_t)stream, &max_ny);
   if (rc) return rc;
-  return launch(ctx, n_scan, ctx->d_scans, max_ny, nullptr, z_out, n_out, n_type, flags, (cudaStream_t)stream);
+  if (!n_charge)
+    return launch(ctx, n_scan, ctx->d_scans, max_ny, nullptr, z_out, n_out, n_type, flags, (cudaStream_t)stream);
+  rc = stage_ncharge(ctx, n_scan, n_charge, (cudaStream_t)stream);
+  if (rc) return rc;
+  const ClosedArgs cl{ctx->d_ncharge, 0};
+  return launch(ctx, n_scan, ctx->d_scans, max_ny, nullptr, z_out, n_out, n_type, flags, (cudaStream_t)stream, 0, nullptr,
+                &cl);
+}
+
+int qd_scan_open(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_out, void* n_out, int n_type, unsigned flags,
+                 void* stream) {
+  return scan_device(ctx, n_scan, scans, nullptr, z_out, n_out, n_type, flags, stream);
+}
+
+int qd_scan_closed(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out, void* n_out,
+                   int n_type, unsigned flags, void* stream) {
+  if (ctx && !n_charge) return fail(ctx, QD_ERR_INVALID, "n_charge is NULL");
+  return scan_device(ctx, n_scan, scans, n_charge, z_out, n_out, n_type, flags, stream);
 }
 
 int qd_scan_upload(qd_ctx* ctx, int n_scan, const qd_scan* scans, void* stream) {
@@ -840,10 +900,12 @@ int qd_scan_launch(qd_ctx* ctx, float* z_out, void* n_out, int n_type, unsigned 
                 (cudaStream_t)stream);
 }
 
-int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_out_host, void* n_out_host, int n_type,
-                      unsigned flags) {
+// qd_scan_open_host, and qd_scan_closed_host when n_charge (HOST, [n_scan]) is given
+static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out_host,
+                     void* n_out_host, int n_type, unsigned flags) {
   int rc = validate_launch(ctx, n_type, flags, n_out_host);
   if (rc) return rc;
+  if (n_charge && (rc = validate_closed(ctx, n_scan, n_charge))) return rc;
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
   *ctx->h_status = 0u;      // report what THIS call's kernels raise (a caller of the async entries polls qd_status itself)
   int max_ny = 0;
@@ -863,7 +925,11 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
   } else {
     rc = stage_scans(ctx, n_scan, scans, ctx->s_compute, &max_ny, true);
     if (rc) return rc;
+    if (n_charge && (rc = stage_ncharge(ctx, n_scan, n_charge, ctx->s_compute))) return rc;
   }
+  // closed: the launch over scans [c0, ...) reads d_ncharge + c0; the single-scan path carries the one total charge
+  const auto closed_from = [&](int c0) { return ClosedArgs{ctx->d_ncharge + c0, one ? n_charge[0] : 0}; };
+  const ClosedArgs cl_all = n_charge ? closed_from(0) : ClosedArgs{};
   const long long pixels = ctx->up_pixels;
   const int N = ctx->L.n_dot;
   const size_t esz = n_elem_size(n_type);
@@ -887,7 +953,7 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
     using clk = std::chrono::steady_clock;
     const auto t0 = clk::now();
     rc = launch(ctx, n_scan, ctx->d_scans, max_ny, nullptr, z_out_host ? (float*)ctx->d_small : nullptr,
-                ctx->d_small + zoff, n_type, flags, ctx->s_compute, 0, one ? scans : nullptr);
+                ctx->d_small + zoff, n_type, flags, ctx->s_compute, 0, one ? scans : nullptr, n_charge ? &cl_all : nullptr);
     if (rc) return rc;
     const auto t1 = clk::now();
     // a latency-bound call: poll the stream instead of cudaStreamSynchronize (whose wake-up costs microseconds); bounded,
@@ -924,8 +990,9 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
   }
   const int rows_cap = pipe_rows_cap();
   for (int c = 0; c < P.n_chunk; ++c) {
+    const ClosedArgs cl = n_charge ? closed_from(P.cut[c]) : ClosedArgs{};
     rc = launch(ctx, P.cut[c + 1] - P.cut[c], ctx->d_scans + P.cut[c], max_ny, nullptr, ctx->d_z, ctx->d_n, n_type, flags,
-                ctx->s_compute, P.n_chunk > 1 ? rows_cap : 0);
+                ctx->s_compute, P.n_chunk > 1 ? rows_cap : 0, nullptr, n_charge ? &cl : nullptr);
     if (rc) return rc;
     QD_CUDA(ctx, cudaEventRecord(ctx->chunk_done[c], ctx->s_compute));
     QD_CUDA(ctx, cudaStreamWaitEvent(ctx->s_copy, ctx->chunk_done[c], 0));
@@ -941,6 +1008,17 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
   QD_CUDA(ctx, cudaStreamSynchronize(ctx->s_compute));
   ctx->staged_pending = false;
   return check_status(ctx);
+}
+
+int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_out_host, void* n_out_host, int n_type,
+                      unsigned flags) {
+  return scan_host(ctx, n_scan, scans, nullptr, z_out_host, n_out_host, n_type, flags);
+}
+
+int qd_scan_closed_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_t* n_charge, float* z_out_host,
+                        void* n_out_host, int n_type, unsigned flags) {
+  if (ctx && !n_charge) return fail(ctx, QD_ERR_INVALID, "n_charge is NULL");
+  return scan_host(ctx, n_scan, scans, n_charge, z_out_host, n_out_host, n_type, flags);
 }
 
 extern "C++" {
@@ -1049,11 +1127,13 @@ int qd_scan_obs_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, int scans_pe
   return check_status(ctx);
 }
 
-int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const double* v, float* z_out_host,
-                        void* n_out_host, int n_type, unsigned flags) {
+// qd_points_open_host, and qd_points_closed_host when n_charge (HOST, one value) is given
+static int points_host(qd_ctx* ctx, const qd_scan* scan, const int32_t* n_charge, int ny, int nx, const double* v,
+                       float* z_out_host, void* n_out_host, int n_type, unsigned flags) {
   int rc = validate_launch(ctx, n_type, flags, n_out_host);
   if (rc) return rc;
-  if (!scan || !v) return fail(ctx, QD_ERR_INVALID, "NULL argument to qd_points_open_host");
+  if (n_charge && (rc = validate_closed(ctx, 1, n_charge))) return rc;
+  if (!scan || !v) return fail(ctx, QD_ERR_INVALID, "NULL argument to qd_points_%s_host", n_charge ? "closed" : "open");
   if (nx <= 0 || ny <= 0) return fail(ctx, QD_ERR_INVALID, "nx, ny must be positive");
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
   *ctx->h_status = 0u;
@@ -1076,7 +1156,10 @@ int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const 
     if (rc) return rc;
   }
   QD_CUDA(ctx, cudaMemcpyAsync(ctx->d_pts, v, (size_t)pixels * NV * sizeof(double), cudaMemcpyHostToDevice, nullptr));
-  rc = launch(ctx, 1, ctx->d_scans, max_ny, ctx->d_pts, ctx->d_z, ctx->d_n, n_type, flags, nullptr);
+  if (n_charge && (rc = stage_ncharge(ctx, 1, n_charge, nullptr))) return rc;
+  const ClosedArgs cl{ctx->d_ncharge, 0};
+  rc = launch(ctx, 1, ctx->d_scans, max_ny, ctx->d_pts, ctx->d_z, ctx->d_n, n_type, flags, nullptr, 0, nullptr,
+              n_charge ? &cl : nullptr);
   if (rc) return rc;
   if (z_out_host)
     QD_CUDA(ctx, cudaMemcpyAsync(z_out_host, ctx->d_z, (size_t)pixels * sizeof(float), cudaMemcpyDeviceToHost, nullptr));
@@ -1084,6 +1167,16 @@ int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const 
   QD_CUDA(ctx, cudaStreamSynchronize(nullptr));
   ctx->staged_pending = false;
   return check_status(ctx);
+}
+
+int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const double* v, float* z_out_host,
+                        void* n_out_host, int n_type, unsigned flags) {
+  return points_host(ctx, scan, nullptr, ny, nx, v, z_out_host, n_out_host, n_type, flags);
+}
+
+int qd_points_closed_host(qd_ctx* ctx, const qd_scan* scan, int32_t n_charge, int ny, int nx, const double* v,
+                          float* z_out_host, void* n_out_host, int n_type, unsigned flags) {
+  return points_host(ctx, scan, &n_charge, ny, nx, v, z_out_host, n_out_host, n_type, flags);
 }
 
 int qd_normalise_obs_typed(qd_ctx* ctx, const float* z, void* out, int z_type, int64_t per_env, int n_env,

@@ -60,6 +60,10 @@ struct KArgs {
   int slot_bytes;                      // warps' stride in dynamic shared memory: `bytes` of the kernel's slot layout
   int col_parts;                       // items per row block along x (> 1 only when nothing is carried along a row: no
                                        // latching, telegraph or 1/f chain) -- small launches spread over more SMs
+  // closed arrays (qd_scan_kernel<N, ALG | QD_CLOSED, ...>): total charge of every scan, [n_scan]; with use_one the one
+  // scan's in one_n_charge
+  const int32_t* n_charge;
+  int one_n_charge;
 };
 
 // Each kernel that gives every warp (the relax kernel: every CTA) its own slot of dynamic shared memory describes the
@@ -126,6 +130,12 @@ struct ProjCache {
   double* mats;     // [QD_PC_WAYS][64]  (mat_stride = 64), or one scratch matrix (mat_stride = 0: affine forms only)
   double* aug;      // [8][16] scratch of the cooperative inversion
   int mat_stride;
+};
+// Closed arrays only (relax_lcp<..., SHIFT = true>): c = cdd 1 of the env, and P_S c of every way of the ProjCache.  Kept
+// out of ProjCache, which proj_cache_build (not inlined) takes from the stack.
+struct ShiftCache {
+  const double* cvec;  // [8]
+  double* caff;        // [QD_PC_WAYS][8]
 };
 
 template <int N>
@@ -198,15 +208,29 @@ __device__ __noinline__ int proj_cache_build(const ProjCache& pc, const double* 
   return slot;
 }
 
-template <int N, bool AFFINE>
+// SHIFT (closed arrays): the relaxation at the shifted potentials h = g + nu c, c = sh.cvec.  P_S h = P_S g + nu P_S c, so
+// the cache serves it with one more vector per way (sh.caff).  `on` = false: the lane only takes part in the warp's votes.
+// Out: *set = the final clamped set S, sums[0] = sum_i (P_S g)_i, sums[1] = sum_i (P_S c)_i (left as they are when the lane
+// clamps nothing).
+template <int N, bool AFFINE, bool SHIFT = false>
 __device__ __forceinline__ void relax_lcp(const double (&g)[N], const double* __restrict__ cdd, const ProjCache& pc,
-                                          int lane, double fx, double fy, double (&nc)[N]) {
+                                          int lane, double fx, double fy, double (&nc)[N], const ShiftCache* sh = nullptr,
+                                          double nu = 0.0, bool on = true, unsigned* set = nullptr, double* sums = nullptr) {
   unsigned act = 0;
 #pragma unroll
   for (int j = 0; j < N; ++j) act |= ((unsigned)__double2hiint(g[j]) >> 31) << j;     // sign bits (a -0.0 clamps to 0 too)
   bool need = act != 0;
 #pragma unroll
   for (int j = 0; j < N; ++j) nc[j] = g[j];
+  if constexpr (SHIFT) {
+    act = 0;
+#pragma unroll
+    for (int j = 0; j < N; ++j) {
+      nc[j] = fma(nu, sh->cvec[j], g[j]);
+      act |= ((unsigned)__double2hiint(nc[j]) >> 31) << j;
+    }
+    need = on && act != 0;
+  }
 #pragma unroll 1
   for (int round = 0; round <= N; ++round) {
     unsigned pend = __ballot_sync(0xffffffffu, need);
@@ -220,6 +244,17 @@ __device__ __forceinline__ void relax_lcp(const double (&g)[N], const double* __
       const unsigned hit = __ballot_sync(0xffffffffu, lane < (int)pc.meta[0] && pc.keys[lane & (QD_PC_WAYS - 1)] == S &&
                                                           lane < QD_PC_WAYS);
       const int slot = hit ? __ffs(hit) - 1 : proj_cache_build<N>(pc, cdd, S, lane);
+      if constexpr (SHIFT) {
+        if (!hit) {                                   // the new way's P_S c
+          if (lane < N) {
+            const double* __restrict__ P = pc.mats + slot * pc.mat_stride + lane * N;
+            double acc = 0.0;
+            for (int j = 0; j < N; ++j) acc = fma(P[j], sh->cvec[j], acc);
+            sh->caff[slot * 8 + lane] = acc;
+          }
+          __syncwarp();
+        }
+      }
       if (member) {
         const double* __restrict__ P = pc.mats + slot * pc.mat_stride;
         unsigned neu = act;
@@ -242,6 +277,18 @@ __device__ __forceinline__ void relax_lcp(const double (&g)[N], const double* __
         } else {
           matvec_smem<N>(P, g, wv);
         }
+        if constexpr (SHIFT) {
+          const double* __restrict__ Pc = sh->caff + slot * 8;
+          double sg = 0.0, sc = 0.0;
+#pragma unroll
+          for (int i = 0; i < N; ++i) {
+            sg += wv[i];
+            sc += Pc[i];
+            wv[i] = fma(nu, Pc[i], wv[i]);
+          }
+          sums[0] = sg;
+          sums[1] = sc;
+        }
 #pragma unroll
         for (int i = 0; i < N; ++i) {
           const double sacc = ((act >> i) & 1u) ? 0.0 : wv[i];
@@ -256,6 +303,61 @@ __device__ __forceinline__ void relax_lcp(const double (&g)[N], const double* __
     need = changed;
   }
   // (a lane leaves the loop only after a round that produced no negative entry, so nc >= 0 here)
+  if constexpr (SHIFT) *set = act;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Closed arrays: min (n-g)^T cdd^{-1} (n-g) over n >= 0, sum n = Q.  Since cdd^{-1} c = 1 for c = cdd 1, the KKT conditions
+// of the closed problem are those of the open one at h = g + nu c, with nu such that sum n = Q: the solution is the open
+// relaxation (relax_lcp) at g + nu* c.  On the segment of nu where the open relaxation clamps the set S it is
+// P_S g + nu P_S c, so sum n(nu) = Sg + nu Sc is linear there and its root nu_S = (Q - Sg) / Sc is exact.  Newton's method on
+// these segments, kept inside a bracket [lo, hi] of sum n(lo) < Q <= sum n(hi) (bisection when a root falls outside):
+// it stops when the relaxation at the root nu_S clamps S again, i.e. the root lies on its own segment.
+//   start: nu of the segment that clamps nothing, sum (g + nu c) = Q;
+//   bracket: at nu_bot = min_j -g_j / c_j every h_j <= 0 and n = 0; at nu_top = max_j -g_j / c_j nothing is clamped, and
+//            sum n = sum h >= Q unless the start already lies above nu_top (then it is the answer).
+// Q = 0 has the single feasible point n = 0.
+// ---------------------------------------------------------------------------------------------------------------
+template <int N, bool AFFINE>
+__device__ __forceinline__ void relax_closed(const double (&g)[N], const double* __restrict__ cdd, const ProjCache& pc,
+                                             const ShiftCache& sh, int lane, double fx, double fy, double q,
+                                             double (&nc)[N]) {
+  const double* __restrict__ c = sh.cvec;
+  double sg0 = 0.0, sc0 = 0.0, nu_bot = 0.0, nu_top = 0.0;
+#pragma unroll
+  for (int j = 0; j < N; ++j) {
+    sg0 += g[j];
+    sc0 += c[j];
+    const double t = -g[j] / c[j];
+    nu_bot = j ? fmin(nu_bot, t) : t;
+    nu_top = j ? fmax(nu_top, t) : t;
+  }
+  double nu = (q - sg0) / sc0;
+  double lo = nu_bot, hi = fmax(nu_top, nu);
+  unsigned root_of = 0u;                 // the clamped set whose segment root nu is (~0u: a bisection point)
+  bool done = !(q > 0.0);
+#pragma unroll
+  for (int j = 0; j < N; ++j) nc[j] = 0.0;
+#pragma unroll 1
+  for (int it = 0; it < 64; ++it) {
+    if (!__any_sync(0xffffffffu, !done)) break;
+    double w[N], sums[2] = {sg0, sc0};
+    unsigned S = 0u;
+    relax_lcp<N, AFFINE, true>(g, cdd, pc, lane, fx, fy, w, &sh, nu, !done, &S, sums);
+    if (!done) {
+      double s = 0.0;
+#pragma unroll
+      for (int j = 0; j < N; ++j) { nc[j] = w[j]; s += w[j]; }
+      if (S == root_of || s == q) {
+        done = true;
+      } else {
+        if (s < q) lo = nu; else hi = nu;
+        const double r = (q - sums[0]) / sums[1];       // (S clamps every dot: sums[1] = 0, r = +-inf or NaN)
+        if (r > lo && r < hi) { nu = r; root_of = S; }
+        else { nu = 0.5 * (lo + hi); root_of = ~0u; }
+      }
+    }
+  }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -538,6 +640,79 @@ __device__ __forceinline__ void ground_state_box(const double (&g)[N], const dou
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// default ground state of a closed array (total charge q).  Candidates floor(n_c) + delta, delta in {0,1}^N, with
+// sum = q: since k = q - sum floor(n_c) lies in [0, N], these are the C(N, k) deltas of weight k, walked in ascending
+// order (Gosper's next-combination step) with the energy E(delta) = sum_j delta_j lin_j + Q[delta] (+ const) of
+// ground_state_box; strict < keeps the first minimum.  kT > 0: Boltzmann average over the same candidates, cut at 40 kT.
+// ---------------------------------------------------------------------------------------------------------------
+template <int N, bool THERMAL, bool AFFINE>
+__device__ __forceinline__ void ground_state_closed_box(const double (&g)[N], const double* __restrict__ rec,
+                                                        const qd_layout& L, const ProjCache& pc, const ShiftCache& sh,
+                                                        int lane, int q, double kT, double fx, double fy, double (&nd)[N]) {
+  const double* __restrict__ cinv = rec + L.o_cinv;
+  const double* __restrict__ Q = rec + L.o_q;
+  double nc[N];
+  relax_closed<N, AFFINE>(g, rec + L.o_cdd, pc, sh, lane, fx, fy, (double)q, nc);
+  double f[N], r[N], lin[N];
+  int fsum = 0;
+#pragma unroll
+  for (int j = 0; j < N; ++j) {
+    f[j] = floor(nc[j]);
+    r[j] = f[j] - g[j];
+    fsum += (int)f[j];
+  }
+  matvec_smem<N>(cinv, r, lin);
+  double lb[N];                                         // linear coefficient of candidate bit p (dot N-1-p)
+#pragma unroll
+  for (int p = 0; p < N; ++p) lb[p] = 2.0 * lin[N - 1 - p];
+  const int k = min(max(q - fsum, 0), N);
+  const unsigned first = (1u << k) - 1u, end = 1u << N;
+  const auto energy = [&](unsigned idx) {
+    double e = Q[idx];
+#pragma unroll
+    for (int p = 0; p < N; ++p) e += ((idx >> p) & 1u) ? lb[p] : 0.0;
+    return e;
+  };
+  const auto next = [](unsigned idx) {                  // next larger index of the same weight (idx != 0)
+    const unsigned low = idx & (0u - idx), up = idx + low;
+    return up | (((idx ^ up) >> 2) >> (__ffs(low) - 1));
+  };
+  const double INF = __longlong_as_double(0x7ff0000000000000LL);
+  double best = INF;
+  unsigned bidx = first;
+#pragma unroll 1
+  for (unsigned idx = first; idx < end; idx = next(idx)) {
+    const double e = energy(idx);
+    if (e < best) { best = e; bidx = idx; }
+    if (idx == 0u) break;
+  }
+  if (THERMAL && kT > 0.0) {
+    const double inv_kT = 1.0 / kT;
+    double Z = 0.0, acc[N];
+#pragma unroll
+    for (int p = 0; p < N; ++p) acc[p] = 0.0;
+#pragma unroll 1
+    for (unsigned idx = first; idx < end; idx = next(idx)) {
+      const double d = (energy(idx) - best) * inv_kT;
+      if (d < 40.0) {
+        const double wgt = exp(-d);
+        Z += wgt;
+#pragma unroll
+        for (int p = 0; p < N; ++p)
+          if ((idx >> p) & 1u) acc[p] += wgt;
+      }
+      if (idx == 0u) break;
+    }
+    const double invZ = 1.0 / Z;
+#pragma unroll
+    for (int j = 0; j < N; ++j) nd[j] = f[j] + acc[N - 1 - j] * invZ;
+  } else {
+#pragma unroll
+    for (int j = 0; j < N; ++j) nd[j] = f[j] + (double)((bidx >> (N - 1 - j)) & 1u);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // brute_force ground state: the minimum over ALL n in {0..maxc}^N (dot 0 slowest, first minimum wins), found by exact
 // branch and bound instead of visiting the (maxc+1)^N candidates (15 625 at N = 6, 390 625 at N = 8).
 //   cdd_inv = U D U^T (U unit upper triangular, D > 0; factored once per env on the host), so with z = n - g
@@ -551,20 +726,23 @@ __device__ __forceinline__ void ground_state_box(const double (&g)[N], const dou
 template <int N, int LVL>
 struct BruteLevel {
   // PASS 0: argmin.  PASS 1: Boltzmann accumulation over candidates with E < cut = Emin + 40 kT.
-  template <int PASS>
+  // CLOSED: `rem` carriers are left for levels LVL..N-1: this level takes 0..rem, the last one exactly rem.
+  template <int PASS, bool CLOSED = false>
   static __device__ __forceinline__ void run(const double* __restrict__ ud, const double (&g)[N], int maxc, double p_prev,
                                              const double (&s)[N], unsigned code, double& best, unsigned& bcode,
-                                             double emin, double inv_kT, double& Z, double (&acc)[N]) {
+                                             double emin, double inv_kT, double& Z, double (&acc)[N], int rem = 0) {
     const double dl = ud[LVL];
     const double ctr = g[LVL] - s[LVL];                     // continuous minimiser of this level's term
+    const int vlo = (CLOSED && LVL == N - 1) ? rem : 0;
+    const int vhi = CLOSED ? rem : maxc;
     // children in order of increasing distance from the centre (Schnorr-Euchner zig-zag): the first leaf reached is the
     // sequentially rounded point -- a strong incumbent -- and a level is left at its FIRST child that fails the bound,
     // since every later child is farther from the centre
-    int up = (int)fmin(fmax(ceil(ctr), 0.0), (double)(maxc + 1));
+    int up = (int)fmin(fmax(ceil(ctr), (double)vlo), (double)(vhi + 1));
     int dn = up - 1;
 #pragma unroll 1
-    while (dn >= 0 || up <= maxc) {
-      const bool take_up = dn < 0 || (up <= maxc && ((double)up - ctr) < (ctr - (double)dn));
+    while (dn >= vlo || up <= vhi) {
+      const bool take_up = dn < vlo || (up <= vhi && ((double)up - ctr) < (ctr - (double)dn));
       const int v = take_up ? up : dn;
       if (take_up) ++up; else --dn;
       const double y = (double)v - ctr;
@@ -586,16 +764,16 @@ struct BruteLevel {
         double s2[N];
 #pragma unroll
         for (int k = 0; k < N; ++k) s2[k] = (k > LVL) ? fma(ud[8 + LVL * N + k], zl, s[k]) : 0.0;
-        BruteLevel<N, LVL + 1>::template run<PASS>(ud, g, maxc, p, s2, c2, best, bcode, emin, inv_kT, Z, acc);
+        BruteLevel<N, LVL + 1>::template run<PASS, CLOSED>(ud, g, maxc, p, s2, c2, best, bcode, emin, inv_kT, Z, acc, rem - v);
       }
     }
   }
 };
 template <int N>
 struct BruteLevel<N, N> {
-  template <int PASS>
+  template <int PASS, bool CLOSED = false>
   static __device__ __forceinline__ void run(const double*, const double (&)[N], int, double, const double (&)[N], unsigned,
-                                             double&, unsigned&, double, double, double&, double (&)[N]) {}
+                                             double&, unsigned&, double, double, double&, double (&)[N], int = 0) {}
 };
 
 // `ud`: d[8] | U[64] of cdd_inv with rows / columns permuted by `pm` (pm[l] = dot at tree level l, pm[8 + j] = level of dot
@@ -605,12 +783,13 @@ struct BruteLevel<N, N> {
 // pinned to the upper face).  (With such dots at the bottom the
 // unconstrained completion the bound assumes is far below anything the box allows, and the walk degenerates.)
 // Exact energy ties (measure zero; the parity tests skip margins <= 1e-9) resolve in tree order.
-template <int N, bool THERMAL>
+// CLOSED (total charge q): every n in {0..q}^N with sum n = q; the walk starts without an incumbent (best = +inf).
+template <int N, bool THERMAL, bool CLOSED = false>
 __device__ __forceinline__ void ground_state_brute(const double (&gp)[N], const double* __restrict__ rec,
                                                    const qd_layout& L, const double* __restrict__ ud,
-                                                   const int* __restrict__ pm, double kT, double (&nd)[N]) {
+                                                   const int* __restrict__ pm, double kT, double (&nd)[N], int q = 0) {
   const double (&g)[N] = gp;
-  const int maxc = (int)rec[L.o_par + QD_PAR_MAXC];
+  const int maxc = CLOSED ? q : (int)rec[L.o_par + QD_PAR_MAXC];
   double Z = 0.0;
   double s[N], acc[N];
 #pragma unroll
@@ -618,7 +797,9 @@ __device__ __forceinline__ void ground_state_brute(const double (&gp)[N], const 
   // starting incumbent: the potentials rounded and clipped to the box
   unsigned bcode = 0;
   double best = 0.0;
-  {
+  if constexpr (CLOSED) {
+    best = __longlong_as_double(0x7ff0000000000000LL);
+  } else {
     double sk[N];
 #pragma unroll
     for (int k = 0; k < N; ++k) sk[k] = 0.0;
@@ -635,11 +816,11 @@ __device__ __forceinline__ void ground_state_brute(const double (&gp)[N], const 
     }
     best += 1e-9;
   }
-  BruteLevel<N, 0>::template run<0>(ud, g, maxc, 0.0, s, 0u, best, bcode, 0.0, 0.0, Z, acc);
+  BruteLevel<N, 0>::template run<0, CLOSED>(ud, g, maxc, 0.0, s, 0u, best, bcode, 0.0, 0.0, Z, acc, q);
   if (THERMAL && kT > 0.0) {
     double cut = best + 40.0 * kT;
     unsigned dummy = 0;
-    BruteLevel<N, 0>::template run<1>(ud, g, maxc, 0.0, s, 0u, cut, dummy, best, 1.0 / kT, Z, acc);
+    BruteLevel<N, 0>::template run<1, CLOSED>(ud, g, maxc, 0.0, s, 0u, cut, dummy, best, 1.0 / kT, Z, acc, q);
     const double invZ = 1.0 / Z;
     double np_[N];
 #pragma unroll
@@ -846,7 +1027,8 @@ __device__ __forceinline__ float radial_amp(const qd_scan* sc, double fx, double
 }
 
 // Slot of qd_scan_kernel.  The projection cache (default / thresholded) and the brute-force block start at the same
-// offset: an instance has one of them, or neither (QD_ALG_TUNNEL), and `bytes` counts only the one it has.
+// offset: an instance has one of them, or neither (QD_ALG_TUNNEL), and `bytes` counts only the one it has.  The closed
+// default instances (qd_scan_slot(L, true)) have one more region after the projection cache.
 struct ScanSlot {
   size_t rec_bytes;   // [rec_doubles] the env's record (TMA destination); the offsets below count from its end
   int scan;           // qd_scan, the descriptor (TMA destination)
@@ -860,9 +1042,11 @@ struct ScanSlot {
   int pc_aff;         // [QD_PC_WAYS][24] affine forms P_S g0, P_S gx, P_S gy, read as double2
   int bf_ud;          // brute force, per item: d[8] and U[64] of the PERMUTED cdd_inv
   int bf_pm;          // int[16] perm / inverse perm: 8 doubles reserved
+  int cl_c;           // closed default: [8] c = cdd 1 of the env, then [QD_PC_WAYS][8] P_S c of every cache way
+  int cl_caff;
   int bytes;
 };
-__host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L) {
+__host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L, bool closed = false) {
   ScanSlot S{};
   S.rec_bytes = (size_t)L.rec_doubles * 8;
   int o = 0;
@@ -876,21 +1060,31 @@ __host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L) {
   S.pc_lin = o;   o += 8 * 32 * 8;
   S.pc_aff = o;   o += QD_PC_WAYS * 24 * 8;
   const int pc_end = o;
+  S.cl_c = o;     o += 8 * 8;
+  S.cl_caff = o;  o += QD_PC_WAYS * 8 * 8;
+  const int closed_end = o;
   o = pc_or_bf;
   S.bf_ud = o;    o += 72 * 8;
   S.bf_pm = o;    o += 8 * 8;
   const int bf_end = o;
   const bool has_pc = L.algorithm == QD_ALG_DEFAULT || L.algorithm == QD_ALG_THRESHOLDED;
   const bool has_bf = L.algorithm == QD_ALG_BRUTE_FORCE;
-  S.bytes = qd_slot_round(S.rec_bytes + (has_pc ? pc_end : has_bf ? bf_end : pc_or_bf));
+  S.bytes = qd_slot_round(S.rec_bytes + (has_pc ? (closed ? closed_end : pc_end) : has_bf ? bf_end : pc_or_bf));
   return S;
 }
+
+// ALG of the closed-array instances of qd_scan_kernel: QD_ALG_DEFAULT | QD_CLOSED, QD_ALG_BRUTE_FORCE | QD_CLOSED.  They
+// swap the ground-state stage for its closed form (total charge per scan: KArgs.n_charge / one_n_charge).
+constexpr int QD_CLOSED = 0x10;
 
 // THERMAL = false instantiations carry no Boltzmann-average code at all (the hard-argmin kernels are the hot ones; the
 // launch picks THERMAL = true only when QD_FLAG_THERMAL is set).
 // POINTS = true: explicit voltage list (a.points) instead of the affine descriptor -- the single-device entry points.
-template <int N, int ALG, bool THERMAL, bool POINTS>
+// ALG may carry QD_CLOSED (closed arrays, QD_ALG_DEFAULT and QD_ALG_BRUTE_FORCE only).
+template <int N, int ALG_, bool THERMAL, bool POINTS>
 __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kernel(const KArgs a) {
+  constexpr bool CLOSED = (ALG_ & QD_CLOSED) != 0;
+  constexpr int ALG = ALG_ & ~QD_CLOSED;
   extern __shared__ __align__(128) unsigned char qd_smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -899,7 +1093,7 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   const int NV = L.n_volt;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
-  const ScanSlot S = qd_scan_slot(L);
+  const ScanSlot S = qd_scan_slot(L, CLOSED);
   unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
   qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
@@ -921,6 +1115,8 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   pc.aff = reinterpret_cast<double*>(tail + S.pc_aff);
   pc.gsrc = POINTS ? nullptr : der;
   pc.mat_stride = 64;
+  double* cl_c = reinterpret_cast<double*>(tail + S.cl_c);
+  const ShiftCache sh{cl_c, reinterpret_cast<double*>(tail + S.cl_caff)};
 
   if (lane == 0) mbar_init(bar, 1);
   __syncwarp();
@@ -947,20 +1143,31 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
     if constexpr (ALG == QD_ALG_DEFAULT) {
       if (lane == 0) { pc.meta[0] = 0u; pc.meta[1] = 0u; }    // the projection cache belongs to one env
     }
+    int qn = 0;                                               // closed: total charge of this scan
+    if constexpr (CLOSED) {
+      qn = a.use_one ? a.one_n_charge : a.n_charge[scan_id];
+      if constexpr (ALG == QD_ALG_DEFAULT) {
+        if (lane < N) {
+          double t = 0.0;
+          for (int j = 0; j < N; ++j) t += rec[L.o_cdd + lane * N + j];
+          cl_c[lane] = t;
+        }
+      }
+    }
 
     const int nx = sc->nx, ny = sc->ny;
     const ItemWindow w = item_window(a, part, nx, ny);
     if (w.empty) { __syncwarp(); continue; }
     const int row0 = w.row0, row1 = w.row1, cx0 = w.cx0, cx1 = w.cx1;
 
-    if constexpr (!POINTS) item_affine_forms<N>(a, rec, sc, der, lane, ALG != QD_ALG_BRUTE_FORCE);
+    if constexpr (!POINTS) item_affine_forms<N>(a, rec, sc, der, lane, ALG != QD_ALG_BRUTE_FORCE && !CLOSED);
     __syncwarp();
     if constexpr (ALG == QD_ALG_BRUTE_FORCE) {
       // ---- tree order of this item (most negative potential at the item's centre first) and cdd_inv = U D U^T in it ----
       if (lane == 0) {
         int ord[N];
         double gc[N];
-        const double maxc_d = rec[L.o_par + QD_PAR_MAXC];
+        const double maxc_d = CLOSED ? (double)qn : rec[L.o_par + QD_PAR_MAXC];
         for (int j = 0; j < N; ++j) {
           ord[j] = j;
           // sort key: how far INSIDE the box [0, maxc] the potential at the item's centre lies (negative: outside, pinned to
@@ -1044,7 +1251,7 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
               for (int j = 0; j < N; ++j) g[j] = fma(rec[L.o_a + j * NV + k], vk, g[j]);
               us = fma(rec[L.o_sa + k], vk, us);
             }
-            if constexpr (ALG != QD_ALG_BRUTE_FORCE) {
+            if constexpr (ALG != QD_ALG_BRUTE_FORCE && !CLOSED) {
               bool big = false;
 #pragma unroll
               for (int j = 0; j < N; ++j) big |= !(g[j] < 252.0);
@@ -1068,7 +1275,9 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
 #pragma unroll
               for (int l = 0; l < N; ++l) gp[l] = g[l];           // explicit voltage lists keep the identity order
             }
-            ground_state_brute<N, THERMAL>(gp, rec, L, bf_ud, bf_pm, kT, nd);
+            ground_state_brute<N, THERMAL, CLOSED>(gp, rec, L, bf_ud, bf_pm, kT, nd, qn);
+          } else if constexpr (CLOSED) {
+            ground_state_closed_box<N, THERMAL, !POINTS>(g, rec, L, pc, sh, lane, qn, kT, (double)ixc, (double)iy, nd);
           }
           else ground_state_box<N, THERMAL, !POINTS>(g, rec, L, pc, lane, L.algorithm == QD_ALG_THRESHOLDED, kT, (double)ixc, (double)iy, nd);
 

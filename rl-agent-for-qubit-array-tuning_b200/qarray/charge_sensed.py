@@ -7,6 +7,7 @@ from __future__ import annotations
 import numpy as np
 
 from qdsim import FLAG_LATCH, FLAG_NOISE, FLAG_THERMAL, N_F64, N_U8, maxwell
+from qdsim._lib import CLOSED_MAX_CHARGE
 from qdsim.composer import GateVoltageComposer
 from qdsim.engine import ModelBatch, new_scans
 from qdsim.runtime import engine_for, fresh_seed
@@ -193,11 +194,61 @@ class ChargeSensedDotArray:
         self.gate_voltage_composer.virtual_gate_matrix = vgm
         return vgm
 
-    # closed arrays are not on the hot path (SURVEY.md section 8a: dead code in the reference's fork)
-    def ground_state_closed(self, vg, n_charge):
-        raise NotImplementedError("closed arrays are outside the accelerated path")
+    # ---- closed arrays: n_charges carriers in total on the dots ----------------------------------------------
+    def _n_charge(self, n_charges) -> int:
+        """The total charge as an int; NotImplementedError for ``thresholded``, ValueError for a non-integer or an
+        out-of-range value (0..251 for ``default``, 0..15 for ``brute_force``)."""
+        if self.algorithm not in CLOSED_MAX_CHARGE:
+            raise NotImplementedError(f"closed arrays: the {self.algorithm} algorithm is not supported (its candidate set "
+                                      "can be empty under the sum constraint); use default or brute_force")
+        if isinstance(n_charges, (bool, np.bool_)) or not isinstance(n_charges, (int, np.integer, float, np.floating)) \
+                or not float(n_charges).is_integer():
+            raise ValueError(f"n_charges must be an integer, got {n_charges!r}")
+        q = int(n_charges)
+        if not 0 <= q <= CLOSED_MAX_CHARGE[self.algorithm]:
+            raise ValueError(f"n_charges must be in 0..{CLOSED_MAX_CHARGE[self.algorithm]} for {self.algorithm}, got {q}")
+        return q
 
-    charge_sensor_closed = do1d_closed = do2d_closed = ground_state_closed
+    def _points_closed(self, vg, n_charges, sensor: bool):
+        q = self._n_charge(n_charges)
+        vg = np.asarray(vg, dtype=np.float64)
+        if vg.shape[-1] != self.n_gate:
+            raise ValueError(f"The shape of vg is in correct it should be of shape (..., n_gate) = (...,{self.n_gate})")
+        lead = vg.shape[:-1]
+        nx = lead[-1] if lead else 1
+        ny = int(np.prod(lead[:-1])) if len(lead) > 1 else 1
+        z, n = engine_for(self, self.device).points_closed_host(
+            self._scan_record(), q, vg.reshape(ny, nx, self.n_gate), n_type=N_F64, flags=self._flags(sensor),
+            want_z=sensor)
+        n = n.reshape(*lead, self.n_dot)
+        if sensor:
+            return z.astype(np.float64).reshape(*lead, 1), n
+        return n
+
+    def ground_state_closed(self, vg, n_charges):
+        """Ground-state occupations of the closed array, (..., n_gate) -> (..., n_dot), summing to ``n_charges``."""
+        return self._points_closed(vg, n_charges, sensor=False)
+
+    def charge_sensor_closed(self, vg, n_charges):
+        """Sensor signal and occupations of the closed array, (..., n_gate) -> ((..., n_sensor), (..., n_dot))."""
+        return self._points_closed(vg, n_charges, sensor=True)
+
+    def do1d_closed(self, gate, min, max, points, n_charges):  # noqa: A002
+        """1-d sweep, closed array.  Returns ``(z (points, n_sensor), n (points, n_dot))``."""
+        q = self._n_charge(n_charges)
+        return self.charge_sensor_closed(self.gate_voltage_composer.do1d(gate, min, max, points), q)
+
+    def do2d_closed(self, x_gate, x_min, x_max, x_points, y_gate, y_min, y_max, y_points, n_charges):
+        """2-d sweep, closed array.  Returns ``(z (y, x, n_sensor), n (y, x, n_dot))``."""
+        q = self._n_charge(n_charges)
+        s = self._scan_record()
+        v0, dx, dy = self.gate_voltage_composer.affine2d(x_gate, x_min, x_max, x_points, y_gate, y_min, y_max, y_points)
+        s["v0"][0, :self.n_gate], s["dx"][0, :self.n_gate], s["dy"][0, :self.n_gate] = v0, dx, dy
+        s["nx"], s["ny"] = x_points, y_points
+        flags = self._flags(True)
+        z, n = engine_for(self, self.device).scan_closed_host(s, q, N_F64 if flags & FLAG_THERMAL else N_U8, flags)
+        return (z.astype(np.float64).reshape(y_points, x_points, 1),
+                n.astype(np.float64).reshape(y_points, x_points, self.n_dot))
 
     def _assert_shape(self):
         assert self.Cdd.shape == (self.n_dot, self.n_dot), "Cdd must be square"

@@ -21,6 +21,8 @@ N_DTYPES = {N_U8: np.uint8, N_F32: np.float32, N_F64: np.float64}
 Z_F32, Z_F16, Z_U8 = 0, 1, 2
 Z_DTYPES = {Z_F32: np.float32, Z_F16: np.float16, Z_U8: np.uint8}
 STATUS_OCC_OVERFLOW = 0x1
+# closed entry points (qd_scan_closed ...): largest total charge per algorithm (QD_ERR_INVALID above it)
+CLOSED_MAX_CHARGE = {"default": 251, "brute_force": 15}
 # flags
 FLAG_LATCH, FLAG_NOISE, FLAG_RADIAL, FLAG_THERMAL = 0x01, 0x02, 0x04, 0x08
 FLAG_CARRY_ROWS, FLAG_LATCH_EXACT, FLAG_WHITE_ON_OUTPUT, FLAG_PINK = 0x10, 0x20, 0x40, 0x80
@@ -67,7 +69,7 @@ def lib_path() -> str:
 EXPORTS = ("qd_abi_version", "qd_create", "qd_destroy", "qd_last_error", "qd_set_models", "qd_scan_open",
            "qd_scan_upload", "qd_scan_launch", "qd_scan_open_host", "qd_normalise_obs", "qd_normalise_obs_typed",
            "qd_scan_obs_host", "qd_status", "qd_points_open_host", "qd_launch_count", "qd_measure_fp64_peak",
-           "qd_measure_fp32_peak")
+           "qd_measure_fp32_peak", "qd_scan_closed", "qd_scan_closed_host", "qd_points_closed_host")
 ABI_VERSION = 3
 
 _lib = None
@@ -103,6 +105,12 @@ def load() -> C.CDLL:
     lib.qd_scan_open_host.restype = C.c_int
     lib.qd_points_open_host.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_uint]
     lib.qd_points_open_host.restype = C.c_int
+    lib.qd_scan_closed.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_int, C.c_uint, vp]
+    lib.qd_scan_closed.restype = C.c_int
+    lib.qd_scan_closed_host.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_int, C.c_uint]
+    lib.qd_scan_closed_host.restype = C.c_int
+    lib.qd_points_closed_host.argtypes = [vp, vp, C.c_int32, C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_uint]
+    lib.qd_points_closed_host.restype = C.c_int
     lib.qd_normalise_obs.argtypes = [vp, vp, vp, C.c_int64, C.c_int, C.c_double, C.c_double, vp, vp]
     lib.qd_normalise_obs.restype = C.c_int
     lib.qd_normalise_obs_typed.argtypes = [vp, vp, vp, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double, vp, vp]

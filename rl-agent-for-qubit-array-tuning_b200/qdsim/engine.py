@@ -270,6 +270,57 @@ class Engine:
                                                   flags))
         return z, n
 
+    # -- closed arrays (fixed total charge per scan) -----------------------------------------------------------
+    @staticmethod
+    def _n_charge(n_charge, n_scan: int) -> np.ndarray:
+        """Total charges as a contiguous int32 array of one entry per scan (a scalar applies to every scan)."""
+        q = np.asarray(n_charge)
+        if q.dtype.kind not in "iu" and not (q.dtype.kind == "f" and np.array_equal(q, np.round(q))):
+            raise ValueError(f"n_charge must be integer-valued, got {n_charge!r}")
+        return np.ascontiguousarray(np.broadcast_to(q.astype(np.int32), (n_scan,)))
+
+    def scan_closed(self, scans: np.ndarray, n_charge, z_out, n_out=None, n_type: int = N_NONE, flags: int = 0,
+                    stream=None):
+        """``scan_open`` for closed arrays: scan i holds ``n_charge[i]`` carriers in total (a scalar: every scan)."""
+        assert scans.dtype == SCAN_DTYPE and scans.flags.c_contiguous
+        q = self._n_charge(n_charge, len(scans))
+        self._check(self._lib.qd_scan_closed(self._ctx, len(scans), _ptr(scans), _ptr(q), _ptr(z_out), _ptr(n_out), n_type,
+                                             flags, self._stream(stream)))
+
+    def scan_closed_host(self, scans: np.ndarray, n_charge, n_type: int | None = None, flags: int = 0,
+                         want_z: bool = True, z_out: np.ndarray | None = None, n_out: np.ndarray | None = None):
+        """``scan_open_host`` for closed arrays: scan i holds ``n_charge[i]`` carriers in total (a scalar: every scan)."""
+        assert scans.dtype == SCAN_DTYPE and scans.flags.c_contiguous
+        q = self._n_charge(n_charge, len(scans))
+        if n_type is None:
+            n_type = N_F64 if flags & FLAG_THERMAL else N_U8
+        pixels = int((scans["pix_offset"] + scans["nx"].astype(np.int64) * scans["ny"]).max())
+        z = (z_out if z_out is not None else np.empty(pixels, dtype=np.float32)) if want_z else None
+        n = None
+        if n_type != N_NONE:
+            n = n_out if n_out is not None else np.empty((pixels, self.models.n_dot), dtype=N_DTYPES[n_type])
+        assert z is None or (z.dtype == np.float32 and z.size >= pixels and z.flags.c_contiguous)
+        assert n is None or (n.dtype == N_DTYPES[n_type] and n.size >= pixels * self.models.n_dot and n.flags.c_contiguous), \
+            "n_out must be a C-contiguous array of the n_type's dtype with at least pixels * n_dot elements"
+        self._check(self._lib.qd_scan_closed_host(self._ctx, len(scans), _ptr(scans), _ptr(q), _ptr(z), _ptr(n), n_type,
+                                                  flags))
+        return z, n
+
+    def points_closed_host(self, scan: np.ndarray, n_charge, v: np.ndarray, n_type: int = N_F64, flags: int = 0,
+                           want_z: bool = True):
+        """``points_open_host`` for a closed array of ``n_charge`` carriers in total."""
+        q = int(self._n_charge(n_charge, 1)[0])
+        v = np.ascontiguousarray(v, dtype=np.float64)
+        ny, nx, nv = v.shape
+        if nv != self.models.n_volt:
+            raise ValueError(f"The shape of vg is in correct it should be of shape (..., n_gate) = (...,{self.models.n_volt})")
+        scan = np.ascontiguousarray(scan, dtype=SCAN_DTYPE).reshape(1)
+        z = np.empty((ny, nx), dtype=np.float32) if want_z else None
+        n = np.empty((ny, nx, self.models.n_dot), dtype=N_DTYPES[n_type]) if n_type != N_NONE else None
+        self._check(self._lib.qd_points_closed_host(self._ctx, _ptr(scan), q, ny, nx, _ptr(v), _ptr(z), _ptr(n), n_type,
+                                                    flags))
+        return z, n
+
     def normalise_obs(self, z, out=None, per_env: int | None = None, n_env: int | None = None, q_low: float = 0.5,
                       q_high: float = 99.5, stats=None, stream=None):
         """Per-env percentile normalisation of DEVICE images (``QuantumDeviceEnv._normalise_obs``, env.py:471-509):
