@@ -23,6 +23,7 @@ extern "C" {
 #define QD_ABI_VERSION 3
 #define QD_MAX_DOTS 8   /* BASELINE.json configs go to 8 dots                                  */
 #define QD_MAX_VOLT 16  /* n_gate + n_barrier = (N+1) + (N-1)                                  */
+#define QD_MAX_SENSORS 4 /* charge sensors of a model set (qd_model_desc.n_sensor)                   */
 
 typedef struct qd_ctx qd_ctx;
 
@@ -101,9 +102,9 @@ enum qd_vc_kind { QD_VC_LINEAR = 0, QD_VC_QUADRATIC = 1, QD_VC_SIGMOID = 2 };
 typedef struct qd_model_desc {
   int32_t n_env;
   int32_t n_dot;            /* N, 1..QD_MAX_DOTS                                                          */
-  int32_t n_sensor;         /* 1                                                                          */
+  int32_t n_sensor;         /* S, 1..QD_MAX_SENSORS (see "Several charge sensors" below)                 */
   int32_t n_volt;           /* columns of cgd: n_gate (Path A) or n_gate + n_barrier (tunnel)             */
-  int32_t n_gate;           /* physical gates incl. the sensor gate                                       */
+  int32_t n_gate;           /* physical gates incl. the sensor gates                                      */
   int32_t algorithm;        /* enum qd_algorithm                                                          */
   int32_t num_charge_states;        /* tunnel: basis size (32)                                            */
   int32_t charge_state_batch_size;  /* tunnel: chunk of the candidate scan (1000), 0 = unchunked          */
@@ -144,6 +145,22 @@ const char* qd_last_error(const qd_ctx* ctx);   /* ctx-owned, valid until the ne
  *   cgd_full     [n_env, D, n_volt]   rows [:N] are also the ground-state cgd
  *   cbg          [n_env, B, n_gate]   raw positive barrier-gate matrix (barrier_voltage_model.py:129) or NULL
  *   params       [n_env]
+ *
+ * Several charge sensors (n_sensor = S > 1; qarray's ChargeSensedDotArray with an (S, n_dot) Cds).  Every sensor output
+ * z_out / z_out_host below is then float [pixels, S], pixel-major like n_out: scan i's block starts at element
+ * pix_offset_i * S.  With S = 1 this is the one-float-per-pixel layout.  Sensor s at a pixel, with u = cgd_full v,
+ * dot residuals e_j = n_j - u_j, t_o = rint(u_{N+o}) + xi_o - u_{N+o} for every sensor o (xi_o: sensor o's input
+ * noise) and C = cdd_inv_full:
+ *     dPhi_k = C_ss (2 (t_s + k) + 1) + 2 sum_j C_{s,j} e_j + 2 sum_{o != s} C_{s,o} t_o,   k = -5..4
+ *     z_s    = sum_k 1 / (1 + (dPhi_k / gamma)^2) + eta_s
+ * (sensor s perturbed, the others at their rounded, noisy occupations; indices s, o of C count from row N).  Each sensor
+ * draws its own white, telegraph and 1/f noise with the env's amplitudes and probabilities: Philox counter word c3 =
+ * sensor index for every stream purpose, so sensor 0 draws what a one-sensor model draws.  The latching uniform is per
+ * pixel (sensor 0's block).  Radial noise: mode 1 adds z_rad,s * amp(ix, iy) to channel s (one amplitude map, each
+ * channel's own normal), mode 2 replaces channel s by its own unit normal.  QD_FLAG_WHITE_ON_OUTPUT moves each sensor's
+ * white noise to its own eta_s.  Limits: n_volt <= QD_MAX_VOLT still holds (the tunnel path with barriers: 2N + S - 1
+ * <= 16).  A device z_out of a two- or four-sensor set must be aligned to 4 S bytes (one vector store per pixel).
+ * qd_scan_obs_host (the one-sensor observation of the env) returns QD_ERR_UNSUPPORTED for S > 1.
  */
 int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_gs, const double* cdd_gs,
                   const double* cdd_inv_full, const double* cgd_full, const double* cbg,
@@ -153,7 +170,7 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
  * TunnelCoupledChargeSensed.charge_sensor_open + QarrayBaseClass._apply_radial_noise
  * (qarray_base_class.py:128-139, 163, 202-206).
  *   scans   HOST pointer, [n_scan]; copied to the device inside the call (stream-ordered)
- *   z_out   DEVICE pointer, float [total pixels]: scan i occupies pixels [pix_offset_i, pix_offset_i + nx_i*ny_i),
+ *   z_out   DEVICE pointer, float [total pixels, n_sensor]: scan i occupies pixels [pix_offset_i, pix_offset_i + nx_i*ny_i),
  *           row-major (iy, ix), fast axis x (sizeof(qd_scan) is 480, a multiple of 16: staged by one TMA bulk copy)
  *   n_out   DEVICE pointer or NULL, element type n_type, [pixels, N]
  *   stream  cudaStream_t (NULL = default stream).  Asynchronous: returns after enqueueing.
@@ -175,7 +192,7 @@ int qd_scan_open_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, float* z_ou
 /* Arbitrary voltage list (the escape hatch behind ground_state_open(vg) / charge_sensor_open(vg[, vb]) called with
  * an explicit array, TunnelCoupledChargeSensed.py:312-380).  HOST buffers.
  *   v       [ny*nx, n_volt]   (gate voltages followed by barrier voltages)
- *   z_out   float [ny*nx] or NULL;  n_out [ny*nx, N] of n_type or NULL
+ *   z_out   float [ny*nx, n_sensor] or NULL;  n_out [ny*nx, N] of n_type or NULL
  *   (ny, nx) = measurement shape: latching / telegraph run along nx.
  * `scan` supplies env_id, peak_width, seed and the radial fields; its v0/dx/dy/nx/ny are ignored. */
 int qd_points_open_host(qd_ctx* ctx, const qd_scan* scan, int ny, int nx, const double* v, float* z_out_host,
@@ -224,7 +241,7 @@ int qd_normalise_obs_typed(qd_ctx* ctx, const float* z, void* out, int z_type, i
  * env.py:471-509 -- what the policy is fed), convert to z_type and copy back; chunks of envs are pipelined so that the
  * copy of one chunk overlaps the kernels of the next.
  *   scans          env-major: scans_per_env consecutive descriptors per env, all of one size, pix_offset = i * nx * ny
- *   out_host       [n_scan * ny * nx] elements of z_type (pinned memory for full copy speed)
+ *   out_host       [n_scan * ny * nx] elements of z_type (pinned memory for full copy speed); one-sensor model sets only
  *   normalise      0: raw sensor signal (QD_Z_F32 / QD_Z_F16 only); 1: percentile-normalised to [0, 1]
  *   stats_host     [n_scan / scans_per_env, 2] doubles (p_low, p_high per env) or NULL
  */

@@ -55,6 +55,35 @@ constexpr bool slot_layouts_hold() {
 }
 static_assert(slot_layouts_hold(), "a shared-memory slot layout breaks an alignment or size invariant");
 
+// The same for model sets of 2..QD_MAX_SENSORS sensors (their records are longer): the slots of the multi-sensor scan
+// instances (qd_scan_slot(L, closed, true)), and those of the tunnel kernels, which stage the record prefix before the
+// sensor rows.  One check per sensor count (each within the compiler's constexpr evaluation budget).
+template <int NS>
+constexpr bool msensor_slot_layouts_hold() {
+  constexpr int W = 4, SMEM = 227 * 1024;
+  const auto staged = [](const auto& S) {
+    return S.rec_bytes % 16 == 0 && (S.rec_bytes + S.scan) % 16 == 0 && (S.rec_bytes + S.bar) % 8 == 0 &&
+           S.bytes * W <= SMEM;
+  };
+  const auto at16 = [](const auto& S, int region) { return (S.rec_bytes + region) % 16 == 0; };
+  for (int alg = QD_ALG_DEFAULT; alg <= QD_ALG_TUNNEL; ++alg)
+    for (int n = 1; n <= QD_MAX_DOTS; ++n)
+      for (int g = 1; g <= QD_MAX_VOLT; ++g)
+        for (int nv = g; nv <= QD_MAX_VOLT; ++nv) {
+          const qd_layout L = qd_make_layout(n, nv, g, alg, 32, 1, NS);
+          const qd::ScanSlot a = qd::qd_scan_slot(L, false, true);
+          const qd::ScanSlot ac = qd::qd_scan_slot(L, true, true);
+          if (!(L.o_q % 2 == 0 && L.n_sensor == NS && staged(a) && at16(a, a.pc_mats) && at16(a, a.pc_aff) &&
+                at16(a, a.ms) && staged(ac) && at16(ac, ac.pc_mats) && at16(ac, ac.pc_aff) &&
+                staged(qd::qd_tunnel_slot(L)) && staged(qd::qd_tunnel_select_slot(L)) &&
+                staged(qd::qd_tunnel_eigen_slot(L)) && qd::qd_tunnel_relax_slot(L).bytes <= SMEM))
+            return false;
+        }
+  return true;
+}
+static_assert(msensor_slot_layouts_hold<2>() && msensor_slot_layouts_hold<3>() && msensor_slot_layouts_hold<4>(),
+              "a shared-memory slot layout of a multi-sensor model set breaks an alignment or size invariant");
+
 struct qd_ctx {
   int device = 0;
   int sm_count = 0;
@@ -164,9 +193,10 @@ kernel_fn pick_dots(int n, F k) {
 }
 
 // default / thresholded search with a hard argmin on affine windows runs the restructured kernel (qd_scan_fast_kernel);
-// QDSIM_GENERIC_SCAN=1 keeps the generic one (A/B timing, and the parity tests run both).  Closed arrays: generic only.
+// QDSIM_GENERIC_SCAN=1 keeps the generic one (A/B timing, and the parity tests run both).  Closed arrays and model sets of
+// several sensors: generic only.
 bool use_fast_kernel(const qd_layout& L, unsigned flags, bool points, bool closed) {
-  if (closed || points || (flags & (QD_FLAG_THERMAL | QD_FLAG_PINK))) return false;
+  if (closed || points || L.n_sensor > 1 || (flags & (QD_FLAG_THERMAL | QD_FLAG_PINK))) return false;
   if (L.algorithm != QD_ALG_DEFAULT && L.algorithm != QD_ALG_THRESHOLDED) return false;
   const char* e = getenv("QDSIM_GENERIC_SCAN");
   return !(e && e[0] == '1');
@@ -178,20 +208,34 @@ kernel_fn pick_p(int n, bool points) {
   return pick_dots<1>(n, [](auto k) { return qd::qd_scan_kernel<decltype(k)::value, ALG, THERMAL, false>; });
 }
 
-kernel_fn pick_kernel(const qd_layout& L, unsigned flags, bool points, bool closed) {
+// M = 0: the one-sensor instances; M = QD_MSENSOR: the same set of instances for model sets of several sensors.
+template <int M>
+kernel_fn pick_kernel_m(const qd_layout& L, unsigned flags, bool points, bool closed) {
   const bool thermal = flags & QD_FLAG_THERMAL;
   if (closed) {
-    constexpr int DC = QD_ALG_DEFAULT | qd::QD_CLOSED, BC = QD_ALG_BRUTE_FORCE | qd::QD_CLOSED;
+    constexpr int DC = QD_ALG_DEFAULT | qd::QD_CLOSED | M, BC = QD_ALG_BRUTE_FORCE | qd::QD_CLOSED | M;
     if (L.algorithm == QD_ALG_BRUTE_FORCE) return thermal ? pick_p<BC, true>(L.n_dot, points) : pick_p<BC, false>(L.n_dot, points);
     if (L.algorithm == QD_ALG_DEFAULT) return thermal ? pick_p<DC, true>(L.n_dot, points) : pick_p<DC, false>(L.n_dot, points);
     return nullptr;
   }
-  if (L.algorithm == QD_ALG_TUNNEL) return pick_p<QD_ALG_TUNNEL, false>(L.n_dot, points);
-  if (L.algorithm == QD_ALG_BRUTE_FORCE)
-    return thermal ? pick_p<QD_ALG_BRUTE_FORCE, true>(L.n_dot, points) : pick_p<QD_ALG_BRUTE_FORCE, false>(L.n_dot, points);
+  constexpr int D = QD_ALG_DEFAULT | M, B = QD_ALG_BRUTE_FORCE | M, T = QD_ALG_TUNNEL | M;
+  if (L.algorithm == QD_ALG_TUNNEL) return pick_p<T, false>(L.n_dot, points);
+  if (L.algorithm == QD_ALG_BRUTE_FORCE) return thermal ? pick_p<B, true>(L.n_dot, points) : pick_p<B, false>(L.n_dot, points);
   if (L.algorithm == QD_ALG_DEFAULT || L.algorithm == QD_ALG_THRESHOLDED)
-    return thermal ? pick_p<QD_ALG_DEFAULT, true>(L.n_dot, points) : pick_p<QD_ALG_DEFAULT, false>(L.n_dot, points);
+    return thermal ? pick_p<D, true>(L.n_dot, points) : pick_p<D, false>(L.n_dot, points);
   return nullptr;
+}
+
+kernel_fn pick_kernel(const qd_layout& L, unsigned flags, bool points, bool closed) {
+  return L.n_sensor > 1 ? pick_kernel_m<qd::QD_MSENSOR>(L, flags, points, closed) : pick_kernel_m<0>(L, flags, points, closed);
+}
+
+// z outputs are [pixels, n_sensor] floats; two- and four-sensor sets store a pixel's channels with one vector store
+int check_z_alignment(qd_ctx* ctx, const float* z_out) {
+  const int S = ctx->L.n_sensor;
+  if ((S == 2 || S == 4) && ((uintptr_t)z_out % (4u * S)) != 0)
+    return fail(ctx, QD_ERR_INVALID, "z_out of a %d-sensor model set must be aligned to %d bytes", S, 4 * S);
+  return QD_OK;
 }
 
 int validate_launch(qd_ctx* ctx, int n_type, unsigned flags, const void* n_out) {
@@ -433,7 +477,7 @@ int launch(qd_ctx* ctx, int n_scan, const qd_scan* d_scans, int max_ny, const do
       fast ? SlotKernel{pick_dots<1>(ctx->L.n_dot, [](auto n) { return qd::qd_scan_fast_kernel<decltype(n)::value>; }),
                         qd::qd_fast_slot(ctx->L).bytes}
            : SlotKernel{pick_kernel(ctx->L, flags, d_points != nullptr, closed != nullptr),
-                        qd::qd_scan_slot(ctx->L, closed != nullptr).bytes};
+                        qd::qd_scan_slot(ctx->L, closed != nullptr, ctx->L.n_sensor > 1).bytes};
   if (!k.fn)
     return fail(ctx, QD_ERR_UNSUPPORTED, "no kernel for n_dot=%d algorithm=%d", ctx->L.n_dot, ctx->L.algorithm);
   qd::KArgs a;
@@ -752,7 +796,9 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
   const int N = desc->n_dot, NV = desc->n_volt, G = desc->n_gate, D = N + desc->n_sensor;
   if (desc->n_env <= 0) return fail(ctx, QD_ERR_INVALID, "n_env must be positive");
   if (N < 1 || N > QD_MAX_DOTS) return fail(ctx, QD_ERR_INVALID, "n_dot must be in 1..%d, got %d", QD_MAX_DOTS, N);
-  if (desc->n_sensor != 1) return fail(ctx, QD_ERR_UNSUPPORTED, "n_sensor must be 1, got %d", desc->n_sensor);
+  const int S = desc->n_sensor;
+  if (S < 1 || S > QD_MAX_SENSORS)
+    return fail(ctx, QD_ERR_INVALID, "n_sensor must be in 1..%d, got %d", QD_MAX_SENSORS, S);
   if (NV < 1 || NV > QD_MAX_VOLT || G < 1 || G > NV)
     return fail(ctx, QD_ERR_INVALID, "bad n_volt=%d / n_gate=%d (max %d)", NV, G, QD_MAX_VOLT);
   const int alg = desc->algorithm;
@@ -770,7 +816,7 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
     return fail(ctx, QD_ERR_INVALID, "cdd_gs is required for the default / thresholded algorithms");
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
 
-  const qd_layout L = qd_make_layout(N, NV, G, alg, desc->num_charge_states, desc->charge_state_batch_size);
+  const qd_layout L = qd_make_layout(N, NV, G, alg, desc->num_charge_states, desc->charge_state_batch_size, S);
   const size_t bytes = (size_t)desc->n_env * L.rec_doubles * sizeof(double);
   std::vector<double> host;
   try {
@@ -796,10 +842,12 @@ int qd_set_models(qd_ctx* ctx, const qd_model_desc* desc, const double* cdd_inv_
     if (cdd_gs) memcpy(r + L.o_cdd, cdd_gs + (size_t)e * N * N, sizeof(double) * N * N);
     const double* cg = cgd_full + (size_t)e * D * NV;
     memcpy(r + L.o_a, cg, sizeof(double) * N * NV);
-    memcpy(r + L.o_sa, cg + (size_t)N * NV, sizeof(double) * NV);
+    memcpy(r + L.o_sa, cg + (size_t)N * NV, sizeof(double) * S * NV);     // the S sensor rows
     const double* ci = cdd_inv_full + (size_t)e * D * D;
-    for (int j = 0; j < N; ++j) r[L.o_sw + j] = ci[(size_t)N * D + j];
-    r[L.o_css] = ci[(size_t)N * D + N];
+    for (int s = 0; s < S; ++s) {
+      for (int j = 0; j < N; ++j) r[L.o_sw + s * N + j] = ci[(size_t)(N + s) * D + j];
+      for (int o = 0; o < S; ++o) r[L.o_css + s * S + o] = ci[(size_t)(N + s) * D + N + o];
+    }
     double* par = r + L.o_par;
     par[QD_PAR_KT] = p.kT;
     par[QD_PAR_THRESHOLD] = p.threshold;
@@ -859,6 +907,7 @@ static int scan_device(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int3
   int rc = validate_launch(ctx, n_type, flags, n_out);
   if (rc) return rc;
   if (n_charge && (rc = validate_closed(ctx, n_scan, n_charge))) return rc;
+  if ((rc = check_z_alignment(ctx, z_out))) return rc;
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
   int max_ny = 0;
   rc = stage_scans(ctx, n_scan, scans, (cudaStream_t)stream, &max_ny);
@@ -895,6 +944,7 @@ int qd_scan_launch(qd_ctx* ctx, float* z_out, void* n_out, int n_type, unsigned 
   int rc = validate_launch(ctx, n_type, flags, n_out);
   if (rc) return rc;
   if (ctx->up_n_scan <= 0) return fail(ctx, QD_ERR_STATE, "qd_scan_upload has not been called");
+  if ((rc = check_z_alignment(ctx, z_out))) return rc;
   QD_CUDA(ctx, cudaSetDevice(ctx->device));
   return launch(ctx, ctx->up_n_scan, ctx->d_scans, ctx->up_max_ny, nullptr, z_out, n_out, n_type, flags,
                 (cudaStream_t)stream);
@@ -910,8 +960,9 @@ static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_
   *ctx->h_status = 0u;      // report what THIS call's kernels raise (a caller of the async entries polls qd_status itself)
   int max_ny = 0;
   // one scan of a Path A model (a single do2d_open): the descriptor goes into the kernel parameters, no H2D copy
+  const int S = ctx->L.n_sensor;
   const bool one = n_scan == 1 && scans && ctx->L.algorithm != QD_ALG_TUNNEL && scans[0].pix_offset == 0 &&
-                   (long long)scans[0].nx * scans[0].ny * (4 + ctx->L.n_dot * (long long)n_elem_size(n_type)) <= (1 << 20);
+                   (long long)scans[0].nx * scans[0].ny * (4 * S + ctx->L.n_dot * (long long)n_elem_size(n_type)) <= (1 << 20);
   if (one) {
     const qd_scan& s0 = scans[0];
     rc = check_scan(ctx, 0, s0);
@@ -933,7 +984,7 @@ static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_
   const long long pixels = ctx->up_pixels;
   const int N = ctx->L.n_dot;
   const size_t esz = n_elem_size(n_type);
-  const size_t zbytes = z_out_host ? (size_t)pixels * sizeof(float) : 0, nbytes = (size_t)pixels * N * esz;
+  const size_t zbytes = z_out_host ? (size_t)pixels * S * sizeof(float) : 0, nbytes = (size_t)pixels * N * esz;
   // ---- small calls (a single do2d_open): the kernel writes its outputs straight into mapped pinned host memory, so the
   // call is one descriptor copy, one launch (two on the tunnel path) and one synchronisation -- no device-to-host copies
   if (zbytes + nbytes <= (1u << 20) && n_scan <= 64) {
@@ -976,7 +1027,7 @@ static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_
     return check_status(ctx);
   }
 
-  rc = grow(ctx, &ctx->d_z, &ctx->z_cap, (size_t)pixels * sizeof(float));
+  rc = grow(ctx, &ctx->d_z, &ctx->z_cap, (size_t)pixels * S * sizeof(float));
   if (rc) return rc;
   if (esz) {
     rc = grow(ctx, (unsigned char**)&ctx->d_n, &ctx->n_cap, (size_t)pixels * N * esz);
@@ -985,7 +1036,7 @@ static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_
   const ChunkPlan P = plan_chunks(ctx, n_scan, scans, 1);
   if (!P.tiled) {
     // the copies below move whole pixel ranges: what lies between the scans must not be stale device memory
-    if (z_out_host) QD_CUDA(ctx, cudaMemsetAsync(ctx->d_z, 0, (size_t)pixels * sizeof(float), ctx->s_compute));
+    if (z_out_host) QD_CUDA(ctx, cudaMemsetAsync(ctx->d_z, 0, (size_t)pixels * S * sizeof(float), ctx->s_compute));
     if (esz) QD_CUDA(ctx, cudaMemsetAsync(ctx->d_n, 0, (size_t)pixels * N * esz, ctx->s_compute));
   }
   const int rows_cap = pipe_rows_cap();
@@ -998,7 +1049,7 @@ static int scan_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, const int32_
     QD_CUDA(ctx, cudaStreamWaitEvent(ctx->s_copy, ctx->chunk_done[c], 0));
     const long long lo = P.lo[c], hi = P.hi[c];
     if (z_out_host)
-      QD_CUDA(ctx, cudaMemcpyAsync(z_out_host + lo, ctx->d_z + lo, (size_t)(hi - lo) * sizeof(float),
+      QD_CUDA(ctx, cudaMemcpyAsync(z_out_host + lo * S, ctx->d_z + lo * S, (size_t)(hi - lo) * S * sizeof(float),
                                    cudaMemcpyDeviceToHost, ctx->s_copy));
     if (esz)
       QD_CUDA(ctx, cudaMemcpyAsync((char*)n_out_host + (size_t)lo * N * esz, (char*)ctx->d_n + (size_t)lo * N * esz,
@@ -1057,6 +1108,9 @@ int qd_scan_obs_host(qd_ctx* ctx, int n_scan, const qd_scan* scans, int scans_pe
                      int normalise, double q_low_pct, double q_high_pct, double* stats_host, unsigned flags) {
   int rc = validate_launch(ctx, QD_N_NONE, flags, nullptr);
   if (rc) return rc;
+  if (ctx->L.n_sensor != 1)
+    return fail(ctx, QD_ERR_UNSUPPORTED, "the observation path takes one-sensor model sets, this one has %d sensors",
+                ctx->L.n_sensor);
   if (!out_host) return fail(ctx, QD_ERR_INVALID, "out_host is NULL");
   const size_t zsz = z_elem_size(z_type);
   if (!zsz) return fail(ctx, QD_ERR_INVALID, "bad z_type %d", z_type);
@@ -1145,10 +1199,10 @@ static int points_host(qd_ctx* ctx, const qd_scan* scan, const int32_t* n_charge
   rc = stage_scans(ctx, 1, &s, nullptr, &max_ny, true);
   if (rc) return rc;
   const long long pixels = (long long)nx * ny;
-  const int N = ctx->L.n_dot, NV = ctx->L.n_volt;
+  const int N = ctx->L.n_dot, NV = ctx->L.n_volt, S = ctx->L.n_sensor;
   rc = grow(ctx, &ctx->d_pts, &ctx->pts_cap, (size_t)pixels * NV * sizeof(double));
   if (rc) return rc;
-  rc = grow(ctx, &ctx->d_z, &ctx->z_cap, (size_t)pixels * sizeof(float));
+  rc = grow(ctx, &ctx->d_z, &ctx->z_cap, (size_t)pixels * S * sizeof(float));
   if (rc) return rc;
   const size_t nbytes = (size_t)pixels * N * n_elem_size(n_type);
   if (nbytes) {
@@ -1162,7 +1216,7 @@ static int points_host(qd_ctx* ctx, const qd_scan* scan, const int32_t* n_charge
               n_charge ? &cl : nullptr);
   if (rc) return rc;
   if (z_out_host)
-    QD_CUDA(ctx, cudaMemcpyAsync(z_out_host, ctx->d_z, (size_t)pixels * sizeof(float), cudaMemcpyDeviceToHost, nullptr));
+    QD_CUDA(ctx, cudaMemcpyAsync(z_out_host, ctx->d_z, (size_t)pixels * S * sizeof(float), cudaMemcpyDeviceToHost, nullptr));
   if (nbytes) QD_CUDA(ctx, cudaMemcpyAsync(n_out_host, ctx->d_n, nbytes, cudaMemcpyDeviceToHost, nullptr));
   QD_CUDA(ctx, cudaStreamSynchronize(nullptr));
   ctx->staged_pending = false;

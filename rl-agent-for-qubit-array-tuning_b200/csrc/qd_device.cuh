@@ -7,13 +7,14 @@ namespace qd {
 
 // ---------------------------------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al. SC'11).  Stream contract: see oracle/philox.py (the CPU checker implements the
-// same contract).  key = 64-bit scan seed, counter = (index_lo, index_hi, purpose, 0).
+// same contract).  key = 64-bit scan seed, counter = (index_lo, index_hi, purpose, sensor): c3 is the charge sensor
+// whose noise the block feeds (0 for everything else).
 // ---------------------------------------------------------------------------------------------------------------
 struct Philox4 { uint32_t w0, w1, w2, w3; };
 
-__device__ __forceinline__ Philox4 philox4x32_10(uint64_t seed, uint64_t index, uint32_t purpose) {
+__device__ __forceinline__ Philox4 philox4x32_10(uint64_t seed, uint64_t index, uint32_t purpose, uint32_t sensor = 0u) {
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-  uint32_t c0 = (uint32_t)index, c1 = (uint32_t)(index >> 32), c2 = purpose, c3 = 0u;
+  uint32_t c0 = (uint32_t)index, c1 = (uint32_t)(index >> 32), c2 = purpose, c3 = sensor;
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
     if (r > 0) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }

@@ -941,14 +941,16 @@ __device__ __forceinline__ void item_affine_forms(const KArgs& a, const double* 
 }
 
 // The random draws of a pixel: one Philox4x32-10 block (purpose 0, counter = pixel index) -> Box-Muller pair (white,
-// radial), latching uniform, telegraph uniform.  All zero when nothing random is on.
+// radial), latching uniform, telegraph uniform.  All zero when nothing random is on.  Charge sensor s >= 1 of a
+// multi-sensor model draws its own block (counter word c3 = s) for its white, radial and telegraph noise; its latching
+// word is unused (the latching uniform is sensor 0's).
 struct PixelDraws {
   float z_white, z_rad, u_latch, u_tele;
 };
-__device__ __forceinline__ PixelDraws pixel_draws(bool need_rng, uint64_t seed, long long pix) {
+__device__ __forceinline__ PixelDraws pixel_draws(bool need_rng, uint64_t seed, long long pix, uint32_t sensor = 0u) {
   PixelDraws d = {0.f, 0.f, 0.f, 0.f};
   if (need_rng) {
-    const Philox4 w = philox4x32_10(seed, (uint64_t)pix, 0u);
+    const Philox4 w = philox4x32_10(seed, (uint64_t)pix, 0u, sensor);
     box_muller(w.w0, w.w1, d.z_white, d.z_rad);
     d.u_latch = u24(w.w2);
     d.u_tele = u24(w.w3);
@@ -998,11 +1000,11 @@ __device__ __forceinline__ void latch_chunk(uint64_t& key, uint64_t& held_key, u
   }
 }
 
-// Telegraph state at the start of row iy: the stationary draw (Philox purpose 1), or state 0 on a flat pass, where the
-// chain runs on from row to row.
-__device__ __forceinline__ uint32_t tele_start(bool f_carry, uint64_t seed, int iy, const double* par) {
+// Telegraph state at the start of row iy: the stationary draw (Philox purpose 1; c3 = the charge sensor whose chain it
+// is), or state 0 on a flat pass, where the chain runs on from row to row.
+__device__ __forceinline__ uint32_t tele_start(bool f_carry, uint64_t seed, int iy, const double* par, uint32_t sensor = 0u) {
   if (f_carry) return 0u;
-  const Philox4 wr = philox4x32_10(seed, (uint64_t)iy, 1u);
+  const Philox4 wr = philox4x32_10(seed, (uint64_t)iy, 1u, sensor);
   return ((double)u24(wr.w0) < par[QD_PAR_TELE_STAT]) ? 1u : 0u;
 }
 
@@ -1028,12 +1030,16 @@ __device__ __forceinline__ float radial_amp(const qd_scan* sc, double fx, double
 
 // Slot of qd_scan_kernel.  The projection cache (default / thresholded) and the brute-force block start at the same
 // offset: an instance has one of them, or neither (QD_ALG_TUNNEL), and `bytes` counts only the one it has.  The closed
-// default instances (qd_scan_slot(L, true)) have one more region after the projection cache.
+// default instances (qd_scan_slot(L, true)) have one more region after the projection cache.  The multi-sensor
+// instances (msensor = true) have the `ms` region before the projection cache / brute-force block; the others have no
+// such region, and their offsets are those of a layout without it.
 struct ScanSlot {
   size_t rec_bytes;   // [rec_doubles] the env's record (TMA destination); the offsets below count from its end
   int scan;           // qd_scan, the descriptor (TMA destination)
   int der;            // [48] per item: g0[8] gx[8] gy[8] us0 usx usy pad[5] | carry[8] | 1/f chain states[4] pad[4]
+                      //      (us0, usx, usy and the 1/f chains of sensor 0)
   int bar;            // mbarrier of the two copies (16 bytes)
+  int ms;             // multi-sensor: [24] per item: us0 usx usy pad of sensors 1..3 [3][4], their 1/f chain states [3][4]
   int pc_mats;        // projection cache: [QD_PC_WAYS][64] P_S matrices (mat_stride = 64), read as double2
   int pc_aug;         // [8][16] scratch of the cooperative inversion
   int pc_keys;        // u32 keys[QD_PC_WAYS], then u32 meta[2] (entries in use, next victim): 8 doubles reserved
@@ -1046,13 +1052,14 @@ struct ScanSlot {
   int cl_caff;
   int bytes;
 };
-__host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L, bool closed = false) {
+__host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L, bool closed = false, bool msensor = false) {
   ScanSlot S{};
   S.rec_bytes = (size_t)L.rec_doubles * 8;
   int o = 0;
   S.scan = o;     o += (int)sizeof(qd_scan);
   S.der = o;      o += 48 * 8;
   S.bar = o;      o += 16;
+  S.ms = o;       if (msensor) o += 24 * 8;
   const int pc_or_bf = o;             // QD_ALG_TUNNEL has neither: its slot ends here
   S.pc_mats = o;  o += QD_PC_WAYS * 64 * 8;
   S.pc_aug = o;   o += 8 * 16 * 8;
@@ -1076,15 +1083,21 @@ __host__ __device__ constexpr ScanSlot qd_scan_slot(const qd_layout& L, bool clo
 // ALG of the closed-array instances of qd_scan_kernel: QD_ALG_DEFAULT | QD_CLOSED, QD_ALG_BRUTE_FORCE | QD_CLOSED.  They
 // swap the ground-state stage for its closed form (total charge per scan: KArgs.n_charge / one_n_charge).
 constexpr int QD_CLOSED = 0x10;
+// ALG bit of the multi-sensor instances (model sets of 2..QD_MAX_SENSORS charge sensors, L.n_sensor at run time): the
+// sensor stage runs once per sensor and z is stored as [pixels, n_sensor].  Without the bit the stage is the one-sensor
+// code.
+constexpr int QD_MSENSOR = 0x20;
 
 // THERMAL = false instantiations carry no Boltzmann-average code at all (the hard-argmin kernels are the hot ones; the
 // launch picks THERMAL = true only when QD_FLAG_THERMAL is set).
 // POINTS = true: explicit voltage list (a.points) instead of the affine descriptor -- the single-device entry points.
-// ALG may carry QD_CLOSED (closed arrays, QD_ALG_DEFAULT and QD_ALG_BRUTE_FORCE only).
+// ALG may carry QD_CLOSED (closed arrays, QD_ALG_DEFAULT and QD_ALG_BRUTE_FORCE only) and QD_MSENSOR (several sensors).
 template <int N, int ALG_, bool THERMAL, bool POINTS>
 __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kernel(const KArgs a) {
   constexpr bool CLOSED = (ALG_ & QD_CLOSED) != 0;
-  constexpr int ALG = ALG_ & ~QD_CLOSED;
+  constexpr bool MSENSOR = (ALG_ & QD_MSENSOR) != 0;
+  constexpr int ALG = ALG_ & ~(QD_CLOSED | QD_MSENSOR);
+  constexpr int SM = MSENSOR ? QD_MAX_SENSORS : 1;   // sensors a pixel holds in registers
   extern __shared__ __align__(128) unsigned char qd_smem[];
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
@@ -1093,7 +1106,7 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   const int NV = L.n_volt;
 
   unsigned char* slot = qd_smem + (size_t)warp * a.slot_bytes;
-  const ScanSlot S = qd_scan_slot(L, CLOSED);
+  const ScanSlot S = qd_scan_slot(L, CLOSED, MSENSOR);
   unsigned char* tail = slot + S.rec_bytes;
   double* rec = reinterpret_cast<double*>(slot);
   qd_scan* sc = reinterpret_cast<qd_scan*>(tail + S.scan);
@@ -1117,6 +1130,8 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   pc.mat_stride = 64;
   double* cl_c = reinterpret_cast<double*>(tail + S.cl_c);
   const ShiftCache sh{cl_c, reinterpret_cast<double*>(tail + S.cl_caff)};
+  double* ms = reinterpret_cast<double*>(tail + S.ms);
+  const int ns = MSENSOR ? L.n_sensor : 1;            // charge sensors
 
   if (lane == 0) mbar_init(bar, 1);
   __syncwarp();
@@ -1131,6 +1146,9 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
   const bool f_pink = a.flags & QD_FLAG_PINK;
   double* d_pink = der + 40;    // state of the four 1/f chains at the last pixel processed (warp-uniform, in shared memory)
   const uint32_t rec_bytes = (uint32_t)L.rec_doubles * 8u;
+  // per-item affine form of sensor s's potential and the state of its 1/f chains: sensor 0 in der, sensors 1..3 in ms
+  const auto us_form = [&](int s) { return s == 0 ? d_us : ms + 4 * (s - 1); };
+  const auto pink_state = [&](int s) { return s == 0 ? d_pink : ms + 12 + 4 * (s - 1); };
 
   const long long total_items = (long long)a.n_scan * a.items_per_scan;
   for (long long item = (long long)blockIdx.x * warps_per_cta + warp; item < total_items;
@@ -1161,6 +1179,20 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
     const int row0 = w.row0, row1 = w.row1, cx0 = w.cx0, cx1 = w.cx1;
 
     if constexpr (!POINTS) item_affine_forms<N>(a, rec, sc, der, lane, ALG != QD_ALG_BRUTE_FORCE && !CLOSED);
+    if constexpr (MSENSOR && !POINTS) {
+      if (lane >= 1 && lane < ns) {                     // sensors 1..S-1 (item_affine_forms wrote sensor 0's)
+        const double* arow = rec + L.o_sa + lane * NV;
+        double s0 = 0.0, sx = 0.0, sy = 0.0;
+        for (int k = 0; k < NV; ++k) {
+          const double c = arow[k];
+          s0 = fma(c, sc->v0[k], s0);
+          sx = fma(c, sc->dx[k], sx);
+          sy = fma(c, sc->dy[k], sy);
+        }
+        double* f = ms + 4 * (lane - 1);
+        f[0] = s0; f[1] = sx; f[2] = sy;
+      }
+    }
     __syncwarp();
     if constexpr (ALG == QD_ALG_BRUTE_FORCE) {
       // ---- tree order of this item (most negative potential at the item's centre first) and cdd_inv = U D U^T in it ----
@@ -1212,10 +1244,13 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
     const double inv_gamma = 1.0 / sc->peak_width;
     const double css = rec[L.o_css];
     const bool need_rng = f_noise || latch_on || (f_radial && sc->rad_mode != 0);
+    const bool need_rng_s = f_noise || (f_radial && sc->rad_mode != 0);      // sensors 1..S-1: no latching word
 
     uint64_t held_key = 0;
     bool have_held = false;
-    uint32_t tele_state = 0;
+    uint32_t tele_state[SM];                                  // one telegraph chain per sensor (warp-uniform)
+#pragma unroll
+    for (int s = 0; s < SM; ++s) tele_state[s] = 0;
     bool tele_init = false;
     bool pink_init = false;
 
@@ -1228,28 +1263,39 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
         const long long pix = (long long)iy * nx + ixc;
         const unsigned vmask = __ballot_sync(0xffffffffu, valid);
         const PixelDraws rnd = pixel_draws(need_rng, seed, pix);
+        PixelDraws rs[SM];                                   // the draws of each sensor: sensor 0's block is rnd
+        rs[0] = rnd;
+#pragma unroll
+        for (int s = 1; s < SM; ++s) rs[s] = pixel_draws(need_rng_s && s < ns, seed, pix, (uint32_t)s);
 
         double nd[N];
         double g[N];
-        double us;
-        float zf;
+        double us[SM];                                       // sensor potentials u_{N+s}
+        float zf[SM];
         if (!replace) {
           // ---- dot potentials g = cgd . v ----
           if constexpr (!POINTS) {
             const double fx = (double)ixc, fy = (double)iy;
 #pragma unroll
             for (int j = 0; j < N; ++j) g[j] = fma(fy, d_gy[j], fma(fx, d_gx[j], d_g0[j]));
-            us = fma(fy, d_us[2], fma(fx, d_us[1], d_us[0]));
+#pragma unroll
+            for (int s = 0; s < SM; ++s) {
+              const double* f = us_form(s);
+              us[s] = (s < ns) ? fma(fy, f[2], fma(fx, f[1], f[0])) : 0.0;
+            }
           } else {
             const double* __restrict__ v = a.points + (size_t)pix * NV;
 #pragma unroll
             for (int j = 0; j < N; ++j) g[j] = 0.0;
-            us = 0.0;
+#pragma unroll
+            for (int s = 0; s < SM; ++s) us[s] = 0.0;
             for (int k = 0; k < NV; ++k) {
               const double vk = v[k];
 #pragma unroll
               for (int j = 0; j < N; ++j) g[j] = fma(rec[L.o_a + j * NV + k], vk, g[j]);
-              us = fma(rec[L.o_sa + k], vk, us);
+#pragma unroll
+              for (int s = 0; s < SM; ++s)
+                if (s < ns) us[s] = fma(rec[L.o_sa + s * NV + k], vk, us[s]);
             }
             if constexpr (ALG != QD_ALG_BRUTE_FORCE && !CLOSED) {
               bool big = false;
@@ -1322,107 +1368,134 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
             }
           }
 
-          // ---- sensor input noise: white + telegraph ----
-          double noise_in = 0.0, noise_out = 0.0;
-          if (f_noise) {
-            const double wn = par[QD_PAR_WHITE] * (double)rnd.z_white;
-            if (f_white_out) noise_out = wn; else noise_in = wn;
-            const double tamp = par[QD_PAR_TELE_AMP];
-            if (tamp != 0.0) {
-              if (!tele_init) {
-                tele_state = tele_start(f_carry, seed, iy, par);
-                tele_init = true;
-              }
-              const uint32_t flip0 = ((double)rnd.u_tele < par[QD_PAR_P01]) ? 1u : 0u;
-              const uint32_t flip1 = ((double)rnd.u_tele < par[QD_PAR_P10]) ? 1u : 0u;
-              uint32_t fn = valid ? ((0u ^ flip0) | ((1u ^ flip1) << 1)) : 2u;   // invalid lanes: identity
+          // ---- the sensor stage, once per charge sensor s (sensor s perturbed, the others at their rounded, noisy
+          // occupations; DESIGN.md section 4) ----
+          // sensor input noise: white + telegraph
+          double noise_in[SM], noise_out[SM];
 #pragma unroll
-              for (int d = 1; d < 32; d <<= 1) {
-                const uint32_t other = __shfl_up_sync(0xffffffffu, fn, d);
-                if (lane >= d) fn = compose2(fn, other);
+          for (int s = 0; s < SM; ++s) {
+            noise_in[s] = 0.0;
+            noise_out[s] = 0.0;
+            if (s >= ns) continue;
+            if (f_noise) {
+              const double wn = par[QD_PAR_WHITE] * (double)rs[s].z_white;
+              if (f_white_out) noise_out[s] = wn; else noise_in[s] = wn;
+              const double tamp = par[QD_PAR_TELE_AMP];
+              if (tamp != 0.0) {
+                if (!tele_init) {
+                  tele_state[s] = tele_start(f_carry, seed, iy, par, (uint32_t)s);
+                  if (s == ns - 1) tele_init = true;
+                }
+                const uint32_t flip0 = ((double)rs[s].u_tele < par[QD_PAR_P01]) ? 1u : 0u;
+                const uint32_t flip1 = ((double)rs[s].u_tele < par[QD_PAR_P10]) ? 1u : 0u;
+                uint32_t fn = valid ? ((0u ^ flip0) | ((1u ^ flip1) << 1)) : 2u;   // invalid lanes: identity
+#pragma unroll
+                for (int d = 1; d < 32; d <<= 1) {
+                  const uint32_t other = __shfl_up_sync(0xffffffffu, fn, d);
+                  if (lane >= d) fn = compose2(fn, other);
+                }
+                const uint32_t st = (fn >> tele_state[s]) & 1u;
+                tele_state[s] = __shfl_sync(0xffffffffu, st, 31);
+                noise_in[s] += tamp * (double)st;
               }
-              const uint32_t st = (fn >> tele_state) & 1u;
-              tele_state = __shfl_sync(0xffffffffu, st, 31);
-              noise_in += tamp * (double)st;
             }
-          }
-          // ---- 1/f input noise: four Ornstein-Uhlenbeck chains x_k[i] = a_k x_k[i-1] + sqrt(1 - a_k^2) xi_k[i] along x,
-          // a_k = exp(-1 / tau_k), tau_k = 2, 8, 32, 128 pixels, unit stationary variance each; the term is
-          // pink_amp * (x_0 + x_1 + x_2 + x_3) / 2.  Draws: Philox purpose 2 (per pixel), 3 (stationary start of a row / of
-          // a flat pass).  A chain is a prefix scan of affine maps with a constant slope: five shuffle steps per chain.
-          if (f_pink && par[QD_PAR_PINK] != 0.0) {
-            if (!pink_init) {
-              const Philox4 ws = philox4x32_10(seed, (uint64_t)iy, 3u);
-              float s0, s1, s2, s3;
-              box_muller(ws.w0, ws.w1, s0, s1);
-              box_muller(ws.w2, ws.w3, s2, s3);
+            // ---- 1/f input noise: four Ornstein-Uhlenbeck chains x_k[i] = a_k x_k[i-1] + sqrt(1 - a_k^2) xi_k[i] along x,
+            // a_k = exp(-1 / tau_k), tau_k = 2, 8, 32, 128 pixels, unit stationary variance each; the term is
+            // pink_amp * (x_0 + x_1 + x_2 + x_3) / 2.  Draws: Philox purpose 2 (per pixel), 3 (stationary start of a row / of
+            // a flat pass).  A chain is a prefix scan of affine maps with a constant slope: five shuffle steps per chain.
+            if (f_pink && par[QD_PAR_PINK] != 0.0) {
+              double* ps = pink_state(s);
+              if (!pink_init) {
+                const Philox4 ws = philox4x32_10(seed, (uint64_t)iy, 3u, (uint32_t)s);
+                float s0, s1, s2, s3;
+                box_muller(ws.w0, ws.w1, s0, s1);
+                box_muller(ws.w2, ws.w3, s2, s3);
+                __syncwarp();
+                if (lane == 0) { ps[0] = (double)s0; ps[1] = (double)s1; ps[2] = (double)s2; ps[3] = (double)s3; }
+                __syncwarp();
+                if (s == ns - 1) pink_init = true;
+              }
+              const Philox4 wp = philox4x32_10(seed, (uint64_t)pix, 2u, (uint32_t)s);
+              float e4[4];
+              box_muller(wp.w0, wp.w1, e4[0], e4[1]);
+              box_muller(wp.w2, wp.w3, e4[2], e4[3]);
+              const int last = 31 - __clz(vmask);
+              double psum = 0.0;
+              double xs_new[4];
+#pragma unroll
+              for (int k = 0; k < 4; ++k) {
+                const double ak = (k == 0) ? 0.60653065971263342 : (k == 1) ? 0.88249690258459546
+                                : (k == 2) ? 0.96923323447634413 : 0.99221793826024351;      // exp(-1/2), exp(-1/8), exp(-1/32), exp(-1/128)
+                double Bk = sqrt(1.0 - ak * ak) * (double)e4[k];
+                double ad = ak, apow = 1.0;
+#pragma unroll
+                for (int d = 1; d < 32; d <<= 1) {
+                  const double tb = __hiloint2double(__shfl_up_sync(0xffffffffu, __double2hiint(Bk), d),
+                                                     __shfl_up_sync(0xffffffffu, __double2loint(Bk), d));
+                  if (lane >= d) Bk = fma(ad, tb, Bk);
+                  if ((lane + 1) & d) apow *= ad;
+                  ad *= ad;
+                }
+                if ((lane + 1) & 32) apow *= ad;
+                const double xk = fma(apow, ps[k], Bk);
+                xs_new[k] = shfl_f64(xk, last);
+                psum += xk;
+              }
               __syncwarp();
-              if (lane == 0) { d_pink[0] = (double)s0; d_pink[1] = (double)s1; d_pink[2] = (double)s2; d_pink[3] = (double)s3; }
-              __syncwarp();
-              pink_init = true;
-            }
-            const Philox4 wp = philox4x32_10(seed, (uint64_t)pix, 2u);
-            float e4[4];
-            box_muller(wp.w0, wp.w1, e4[0], e4[1]);
-            box_muller(wp.w2, wp.w3, e4[2], e4[3]);
-            const int last = 31 - __clz(vmask);
-            double psum = 0.0;
-            double xs_new[4];
+              if (lane == 0) {
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const double ak = (k == 0) ? 0.60653065971263342 : (k == 1) ? 0.88249690258459546
-                              : (k == 2) ? 0.96923323447634413 : 0.99221793826024351;      // exp(-1/2), exp(-1/8), exp(-1/32), exp(-1/128)
-              double Bk = sqrt(1.0 - ak * ak) * (double)e4[k];
-              double ad = ak, apow = 1.0;
-#pragma unroll
-              for (int d = 1; d < 32; d <<= 1) {
-                const double tb = __hiloint2double(__shfl_up_sync(0xffffffffu, __double2hiint(Bk), d),
-                                                   __shfl_up_sync(0xffffffffu, __double2loint(Bk), d));
-                if (lane >= d) Bk = fma(ad, tb, Bk);
-                if ((lane + 1) & d) apow *= ad;
-                ad *= ad;
+                for (int k = 0; k < 4; ++k) ps[k] = xs_new[k];
               }
-              if ((lane + 1) & 32) apow *= ad;
-              const double xk = fma(apow, d_pink[k], Bk);
-              xs_new[k] = shfl_f64(xk, last);
-              psum += xk;
+              __syncwarp();
+              noise_in[s] += par[QD_PAR_PINK] * 0.5 * psum;
             }
-            __syncwarp();
-            if (lane == 0) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k) d_pink[k] = xs_new[k];
-            }
-            __syncwarp();
-            noise_in += par[QD_PAR_PINK] * 0.5 * psum;
           }
 
           // ---- sensor: ten Lorentzians of the first differences of the full-system free energy ----
-          double base = 0.0;
+          // t_o = rint(u_o) + xi_o - u_o of every sensor: the offset of its occupation from its potential
+          double tv[SM];
+          if constexpr (MSENSOR) {
 #pragma unroll
-          for (int j = 0; j < N; ++j) base = fma(rec[L.o_sw + j], nd[j] - g[j], base);
-          base *= 2.0;
-          const double t = (rint(us) + noise_in) - us;
-          // dPhi_k = css (2 (t + k) + 1) + base is affine in k: x_k = dPhi_k / gamma = x0 + k * xs
-          const double xs = 2.0 * css * inv_gamma;
-          const double x0 = fma(css, fma(2.0, t, 1.0), base) * inv_gamma;
-          double z;
-          if constexpr (ALG == QD_ALG_TUNNEL) {
-            // tunnel path: fp64 Lorentzians.  <n> carries the eigen-solver's own error (1e-6 budget), so the sensor adds
-            // none of its own; the cost is nothing next to the per-pixel eigen-solve.
-            double zs = 0.0;
-#pragma unroll
-            for (int k = -5; k < 5; ++k) {
-              const double xk = fma((double)k, xs, x0);
-              zs += 1.0 / fma(xk, xk, 1.0);
-            }
-            z = zs + noise_out;
-          } else {
-            z = (double)sensor_lorentz10(x0, xs) + noise_out;
+            for (int s = 0; s < SM; ++s) tv[s] = (s < ns) ? (rint(us[s]) + noise_in[s]) - us[s] : 0.0;
           }
-          if (f_radial && sc->rad_mode == 1) z = fma((double)rnd.z_rad, (double)radial_amp(sc, (double)ixc, (double)iy), z);
-          zf = (float)z;
+#pragma unroll
+          for (int s = 0; s < SM; ++s) {
+            zf[s] = 0.f;
+            if (s >= ns) continue;
+            double base = 0.0;
+#pragma unroll
+            for (int j = 0; j < N; ++j) base = fma(rec[L.o_sw + s * N + j], nd[j] - g[j], base);
+            if constexpr (MSENSOR) {
+#pragma unroll
+              for (int o = 0; o < SM; ++o)
+                if (o < ns && o != s) base = fma(rec[L.o_css + s * ns + o], tv[o], base);
+            }
+            base *= 2.0;
+            const double t = MSENSOR ? tv[s] : (rint(us[s]) + noise_in[s]) - us[s];
+            const double css_s = (s == 0) ? css : rec[L.o_css + s * (ns + 1)];
+            // dPhi_k = css (2 (t + k) + 1) + base is affine in k: x_k = dPhi_k / gamma = x0 + k * xs
+            const double xs = 2.0 * css_s * inv_gamma;
+            const double x0 = fma(css_s, fma(2.0, t, 1.0), base) * inv_gamma;
+            double z;
+            if constexpr (ALG == QD_ALG_TUNNEL) {
+              // tunnel path: fp64 Lorentzians.  <n> carries the eigen-solver's own error (1e-6 budget), so the sensor adds
+              // none of its own; the cost is nothing next to the per-pixel eigen-solve.
+              double zs = 0.0;
+#pragma unroll
+              for (int k = -5; k < 5; ++k) {
+                const double xk = fma((double)k, xs, x0);
+                zs += 1.0 / fma(xk, xk, 1.0);
+              }
+              z = zs + noise_out[s];
+            } else {
+              z = (double)sensor_lorentz10(x0, xs) + noise_out[s];
+            }
+            if (f_radial && sc->rad_mode == 1) z = fma((double)rs[s].z_rad, (double)radial_amp(sc, (double)ixc, (double)iy), z);
+            zf[s] = (float)z;
+          }
         } else {
-          zf = rnd.z_rad;
+#pragma unroll
+          for (int s = 0; s < SM; ++s) zf[s] = rs[s].z_rad;
 #pragma unroll
           for (int j = 0; j < N; ++j) nd[j] = 0.0;
         }
@@ -1430,7 +1503,19 @@ __global__ void __launch_bounds__(QD_CTA_WARPS * 32, QD_MIN_BLOCKS) qd_scan_kern
         // ---- coalesced stores ----
         if (valid) {
           const long long o = pix0 + (long long)iy * nx + ix;
-          if (a.z_out) a.z_out[o] = zf;
+          if (a.z_out) {
+            if constexpr (!MSENSOR) {
+              a.z_out[o] = zf[0];
+            } else if (ns == 2) {                            // z is [pixels, S]: one vector store per pixel
+              *reinterpret_cast<float2*>(a.z_out + o * 2) = make_float2(zf[0], zf[1]);
+            } else if (ns == 4) {
+              *reinterpret_cast<float4*>(a.z_out + o * 4) = make_float4(zf[0], zf[1], zf[2], zf[3]);
+            } else {
+#pragma unroll
+              for (int s = 0; s < SM; ++s)
+                if (s < ns) a.z_out[o * ns + s] = zf[s];
+            }
+          }
           if (a.n_type == QD_N_U8) {
             unsigned char* p = reinterpret_cast<unsigned char*>(a.n_out) + o * N;
             if constexpr (N == 8) {

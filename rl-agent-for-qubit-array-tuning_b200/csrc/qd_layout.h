@@ -31,9 +31,9 @@ struct qd_layout {
   int32_t o_cinv;    // [N*N]      ground-state quadratic form (cdd_inv)
   int32_t o_cdd;     // [N*N]      Maxwell cdd (M-matrix) for the exact relaxation
   int32_t o_a;       // [N*NV]     cgd rows of the dots
-  int32_t o_sw;      // [N]        cdd_inv_full[N, 0:N]   sensor <-> dot couplings
-  int32_t o_css;     // [1]        cdd_inv_full[N, N]
-  int32_t o_sa;      // [NV]       cgd_full[N, :]         sensor row
+  int32_t o_sw;      // [S*N]      cdd_inv_full[N+s, 0:N]      sensor <-> dot couplings, row s per sensor
+  int32_t o_css;     // [S*S]      cdd_inv_full[N+s, N+o]      sensor block
+  int32_t o_sa;      // [S*NV]     cgd_full[N+s, :]            sensor rows
   int32_t o_par;     // [QD_PAR_COUNT]
   int32_t o_alpha;   // [8]        barrier alphas (tunnel)
   int32_t o_pleads;  // [8]
@@ -43,12 +43,16 @@ struct qd_layout {
   int32_t o_q;       // [2^N]      Q[delta] = delta^T cdd_inv delta, delta in {0,1}^N, dot 0 = most significant bit
   int32_t o_cbg;     // [B*G]      (tunnel) raw positive barrier-gate matrix
   int32_t gs_doubles;   // (tunnel) length of the record PREFIX the ground-state kernel stages: cinv | a | par | alpha | cbg
-  int32_t pad0, pad1;
+  int32_t n_sensor;     // S, 1..QD_MAX_SENSORS
+  int32_t pad1;
   int32_t rec_doubles;  // total, multiple of 2 (16 bytes)
 };
 
-static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int algorithm, int num_states, int chunk) {
+// With one sensor (n_sensor = 1) every offset and rec_doubles are those of a layout without the sensor count.
+static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int algorithm, int num_states, int chunk,
+                                          int n_sensor = 1) {
   qd_layout L{};
+  const int S = n_sensor;
   L.n_dot = n_dot; L.n_volt = n_volt; L.n_gate = n_gate; L.algorithm = algorithm;
   L.num_states = num_states; L.chunk = chunk;
   int o = 0;
@@ -63,9 +67,9 @@ static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int
     o = (o + 1) & ~1;
     L.gs_doubles = o;
     L.o_cdd = o;    o += n_dot * n_dot;
-    L.o_sw = o;     o += n_dot;
-    L.o_css = o;    o += 1;
-    L.o_sa = o;     o += n_volt;
+    L.o_sw = o;     o += S * n_dot;
+    L.o_css = o;    o += S * S;
+    L.o_sa = o;     o += S * n_volt;
     L.o_pleads = o; o += 8;
     L.o_pinter = o; o += 64;
     L.o_spos = o;   o += 8;
@@ -75,9 +79,9 @@ static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int
   } else {
     L.o_cdd = o;    o += n_dot * n_dot;
     L.o_a = o;      o += n_dot * n_volt;
-    L.o_sw = o;     o += n_dot;
-    L.o_css = o;    o += 1;
-    L.o_sa = o;     o += n_volt;
+    L.o_sw = o;     o += S * n_dot;
+    L.o_css = o;    o += S * S;
+    L.o_sa = o;     o += S * n_volt;
     L.o_par = o;    o += QD_PAR_COUNT;
     L.o_alpha = o;  o += 8;
     L.o_pleads = o; o += 8;
@@ -90,7 +94,8 @@ static constexpr qd_layout qd_make_layout(int n_dot, int n_volt, int n_gate, int
     L.o_cbg = o;
     L.gs_doubles = 0;
   }
-  L.pad0 = L.pad1 = 0;
+  L.n_sensor = S;
+  L.pad1 = 0;
   // (the tunnel path's block tables depend on a per-item permutation of the dots and are built inside the kernel)
   L.rec_doubles = (o + 1) & ~1;
   return L;

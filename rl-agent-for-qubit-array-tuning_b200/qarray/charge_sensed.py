@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from qdsim import FLAG_LATCH, FLAG_NOISE, FLAG_THERMAL, N_F64, N_U8, maxwell
+from qdsim import FLAG_LATCH, FLAG_NOISE, FLAG_THERMAL, N_F64, N_U8, QD_MAX_SENSORS, QD_MAX_VOLT, maxwell
 from qdsim._lib import CLOSED_MAX_CHARGE
 from qdsim.composer import GateVoltageComposer
 from qdsim.engine import ModelBatch, new_scans
@@ -54,8 +54,10 @@ class ChargeSensedDotArray:
             assert max_charge_carriers is not None, "The maximum number of charge carriers must be specified"
         if n_peak != 5:
             raise NotImplementedError("the sensor kernel evaluates n_peak = 5 (the reference's value)")
-        if self.n_sensor != 1:
-            raise NotImplementedError("libqdsim supports one charge sensor (every reference config has one)")
+        if not 1 <= self.n_sensor <= QD_MAX_SENSORS:
+            raise NotImplementedError(f"libqdsim simulates 1..{QD_MAX_SENSORS} charge sensors, got {self.n_sensor}")
+        if self.n_gate > QD_MAX_VOLT:
+            raise ValueError(f"libqdsim takes at most {QD_MAX_VOLT} gate voltages, got n_gate = {self.n_gate}")
         self.algorithm = algorithm
         self.implementation = implementation
         self.threshold = 1.0 if threshold == "auto" else float(threshold)
@@ -155,7 +157,7 @@ class ChargeSensedDotArray:
         # the kernel has to push over PCIe) and widen here; thermal averages come back as float64
         z, n = engine_for(self, self.device).scan_one_host(s, N_F64 if flags & FLAG_THERMAL else N_U8, flags,
                                                            x_points * y_points)
-        return (z.astype(np.float64).reshape(y_points, x_points, 1),
+        return (z.astype(np.float64).reshape(y_points, x_points, self.n_sensor),
                 n.astype(np.float64).reshape(y_points, x_points, self.n_dot))
 
     def do1d_open(self, gate, min, max, points):  # noqa: A002
@@ -173,7 +175,7 @@ class ChargeSensedDotArray:
             self._scan_record(), vg.reshape(ny, nx, self.n_gate), n_type=N_F64, flags=self._flags(sensor), want_z=sensor)
         n = n.reshape(*lead, self.n_dot)
         if sensor:
-            return z.astype(np.float64).reshape(*lead, 1), n
+            return z.astype(np.float64).reshape(*lead, self.n_sensor), n
         return n
 
     def ground_state_open(self, vg):
@@ -222,7 +224,7 @@ class ChargeSensedDotArray:
             want_z=sensor)
         n = n.reshape(*lead, self.n_dot)
         if sensor:
-            return z.astype(np.float64).reshape(*lead, 1), n
+            return z.astype(np.float64).reshape(*lead, self.n_sensor), n
         return n
 
     def ground_state_closed(self, vg, n_charges):
@@ -247,7 +249,7 @@ class ChargeSensedDotArray:
         s["nx"], s["ny"] = x_points, y_points
         flags = self._flags(True)
         z, n = engine_for(self, self.device).scan_closed_host(s, q, N_F64 if flags & FLAG_THERMAL else N_U8, flags)
-        return (z.astype(np.float64).reshape(y_points, x_points, 1),
+        return (z.astype(np.float64).reshape(y_points, x_points, self.n_sensor),
                 n.astype(np.float64).reshape(y_points, x_points, self.n_dot))
 
     def _assert_shape(self):

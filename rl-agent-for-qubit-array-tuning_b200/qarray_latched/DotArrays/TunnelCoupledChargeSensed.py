@@ -12,7 +12,7 @@ import numpy as np
 
 from qarray.latching_models import LatchingBaseModel
 from qarray.noise_models import BaseNoiseModel
-from qdsim import FLAG_LATCH, FLAG_NOISE, N_F64, PARAMS_DTYPE, QD_MAX_DOTS, maxwell
+from qdsim import FLAG_LATCH, FLAG_NOISE, N_F64, PARAMS_DTYPE, QD_MAX_DOTS, QD_MAX_SENSORS, QD_MAX_VOLT, maxwell
 from qdsim.composer import GateVoltageComposer
 from qdsim.engine import K_B, ModelBatch, new_scans
 from qdsim.runtime import engine_for, fresh_seed
@@ -89,8 +89,11 @@ class TunnelCoupledChargeSensed:
         self.n_gate = self.Cgd.shape[1]
         self.n_barrier = self.Cbd.shape[1] if self.Cbd is not None else 0
         self._assert_shape()
-        if self.n_sensor != 1:
-            raise NotImplementedError("libqdsim supports one charge sensor (every reference config has one)")
+        if not 1 <= self.n_sensor <= QD_MAX_SENSORS:
+            raise NotImplementedError(f"libqdsim simulates 1..{QD_MAX_SENSORS} charge sensors, got {self.n_sensor}")
+        if self.n_gate + self.n_barrier > QD_MAX_VOLT:
+            raise ValueError(f"libqdsim takes at most {QD_MAX_VOLT} gate and barrier voltages, got n_gate + n_barrier = "
+                             f"{self.n_gate} + {self.n_barrier}")
         cdd_nm, cgd_nm = maxwell.embed_sensor(self.Cdd, self.Cgd, self.Cds, self.Cgs, self.Cbd, self.Cbs)
         self.cdd_full, self.cdd_inv_full, self.cgd_full = maxwell.maxwell(cdd_nm, cgd_nm)
         self.cdd, self.cdd_inv, self.cgd = maxwell.maxwell(self.Cdd, self.Cgd)
@@ -174,7 +177,7 @@ class TunnelCoupledChargeSensed:
             s, v.reshape(ny, nx, v.shape[-1]), n_type=N_F64, flags=self._flags(sensor), want_z=sensor)
         n = n.reshape(*lead, self.n_dot)
         if sensor:
-            return z.astype(np.float64).reshape(*lead, 1), n
+            return z.astype(np.float64).reshape(*lead, self.n_sensor), n
         return n
 
     # ---- reference API -------------------------------------------------------------------------------------

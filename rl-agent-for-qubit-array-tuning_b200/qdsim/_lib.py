@@ -9,6 +9,7 @@ import numpy as np
 
 QD_MAX_DOTS = 8
 QD_MAX_VOLT = 16
+QD_MAX_SENSORS = 4
 
 # enum qd_algorithm
 ALG_DEFAULT, ALG_THRESHOLDED, ALG_BRUTE_FORCE, ALG_TUNNEL = 0, 1, 2, 3

@@ -13,7 +13,7 @@ import numpy as np
 from . import _lib, maxwell
 from ._lib import (ALGORITHMS, FLAG_CARRY_ROWS, FLAG_LATCH, FLAG_LATCH_EXACT, FLAG_NOISE, FLAG_PINK, FLAG_RADIAL,  # noqa: F401
                    FLAG_THERMAL, FLAG_WHITE_ON_OUTPUT, N_DTYPES, N_F32, N_F64, N_NONE, N_U8, PARAMS_DTYPE,
-                   QD_MAX_DOTS, QD_MAX_VOLT, SCAN_DTYPE, Z_DTYPES, Z_F16, Z_F32, Z_U8, QdError)
+                   QD_MAX_DOTS, QD_MAX_SENSORS, QD_MAX_VOLT, SCAN_DTYPE, Z_DTYPES, Z_F16, Z_F32, Z_U8, QdError)
 
 K_B = 8.617333262145e-5  # eV/K (src/qarray_latched/DotArrays/_helper_functions.py:213-214)
 
@@ -44,14 +44,19 @@ class ModelBatch:
     def n_volt(self) -> int:
         return self.cgd_full.shape[-1]
 
+    @property
+    def n_sensor(self) -> int:
+        return self.cdd_inv_full.shape[-1] - self.n_dot
+
     @classmethod
     def from_capacitances(cls, Cdd, Cgd, Cds, Cgs, algorithm: str = "default", T=0.0, threshold=1.0,
                           max_charge_carriers: int = 4, p_leads=None, p_inter=None, white_amp=0.0, tele_p01=0.0,
                           tele_p10=0.0, tele_amp=0.0) -> "ModelBatch":
         """Path A (``ChargeSensedDotArray``) batch from non-Maxwell matrices with a leading env axis.
 
-        The dots' ground state uses the dot-only Maxwell matrices, the sensor the full [dots, sensor] system
-        (SURVEY.md Appendix B.1; TunnelCoupledChargeSensed.py:117-130 keeps both sets).
+        The dots' ground state uses the dot-only Maxwell matrices, the sensors the full [dots, sensors] system
+        (SURVEY.md Appendix B.1; TunnelCoupledChargeSensed.py:117-130 keeps both sets).  ``Cds`` (S, N) and ``Cgs`` (S, G)
+        hold one row per charge sensor, 1 <= S <= ``QD_MAX_SENSORS``.
         """
         Cdd = np.asarray(Cdd, dtype=np.float64)
         Cgd = np.asarray(Cgd, dtype=np.float64)
@@ -87,7 +92,7 @@ def tunnel_model_batch(Cdd, Cgd, Cds, Cgs, Cbd, Cbg, Cbs, tc_base, alpha, p_lead
                        tele_p01=0.0, tele_p10=0.0, tele_amp=0.0, num_charge_states: int = 32,
                        charge_state_batch_size: int = 1000) -> ModelBatch:
     """Path B (``TunnelCoupledChargeSensed`` with barriers) batch from non-Maxwell matrices with a leading env axis.
-    Barriers are voltage sources: extra columns of cgd (src/qarray_latched/DotArrays/_helper_functions.py:60-126); the
+    ``Cds`` / ``Cgs`` / ``Cbs`` hold one row per charge sensor.  Barriers are voltage sources: extra columns of cgd (src/qarray_latched/DotArrays/_helper_functions.py:60-126); the
     ground state uses the dot block of the FULL inverse (ground_state.py:60-65)."""
     Cdd, Cgd, Cds, Cgs, Cbd, Cbg, Cbs = (np.asarray(a, dtype=np.float64) for a in (Cdd, Cgd, Cds, Cgs, Cbd, Cbg, Cbs))
     n_env, n_dot, n_barrier = Cdd.shape[0], Cdd.shape[-1], Cbd.shape[-1]
@@ -137,6 +142,7 @@ class Engine:
             raise QdError(rc, self._lib.qd_last_error(None).decode())
         self.device = int(device)
         self.models: ModelBatch | None = None
+        self.n_sensor = 1                   # charge sensors of the uploaded model set: z is [pixels, n_sensor]
         self._one_bufs: dict = {}           # staging buffers of scan_one_host, by (pixels, n_type)
 
     # -- lifecycle -------------------------------------------------------------------------------------------
@@ -168,10 +174,24 @@ class Engine:
         params = np.ascontiguousarray(mb.params, dtype=PARAMS_DTYPE)
         self._check(self._lib.qd_set_models(self._ctx, C.byref(desc), *[_ptr(a) for a in arrs], _ptr(params)))
         self.models = mb
+        self.n_sensor = d - mb.n_dot
+
+    def _z(self, pixels: int, z_out, want_z: bool, shape=None):
+        """The host sensor buffer of a call: ``shape`` (default ``(pixels,)``) for one sensor, ``shape + (S,)`` otherwise."""
+        if not want_z:
+            return None
+        s = self.n_sensor
+        if z_out is None:
+            shape = (pixels,) if shape is None else shape
+            return np.empty(shape if s == 1 else shape + (s,), dtype=np.float32)
+        assert z_out.dtype == np.float32 and z_out.size >= pixels * s and z_out.flags.c_contiguous, \
+            "z_out must be a C-contiguous float32 array with at least pixels * n_sensor elements"
+        return z_out
 
     # -- launches --------------------------------------------------------------------------------------------
     def scan_open(self, scans: np.ndarray, z_out, n_out=None, n_type: int = N_NONE, flags: int = 0, stream=None):
-        """Asynchronous batched launch into DEVICE buffers (torch tensors or raw pointers)."""
+        """Asynchronous batched launch into DEVICE buffers (torch tensors or raw pointers).  ``z_out``: float32
+        [pixels, n_sensor] (aligned to 4 n_sensor bytes for two or four sensors), ``n_out``: [pixels, N]."""
         assert scans.dtype == SCAN_DTYPE and scans.flags.c_contiguous
         self._check(self._lib.qd_scan_open(self._ctx, len(scans), _ptr(scans), _ptr(z_out), _ptr(n_out), n_type,
                                            flags, self._stream(stream)))
@@ -186,11 +206,13 @@ class Engine:
         self._check(self._lib.qd_scan_upload(self._ctx, len(scans), _ptr(scans), self._stream(stream)))
 
     def scan_launch(self, z_out, n_out=None, n_type: int = N_NONE, flags: int = 0, stream=None):
+        """One launch over the uploaded descriptors into DEVICE buffers laid out as in ``scan_open``."""
         self._check(self._lib.qd_scan_launch(self._ctx, _ptr(z_out), _ptr(n_out), n_type, flags, self._stream(stream)))
 
     def scan_open_host(self, scans: np.ndarray, n_type: int | None = None, flags: int = 0, want_z: bool = True,
                        z_out: np.ndarray | None = None, n_out: np.ndarray | None = None):
-        """Synchronous launch returning host arrays ``(z float32 [pixels], n [pixels, N] or None)``.
+        """Synchronous launch returning host arrays ``(z float32 [pixels] (one sensor) or [pixels, S], n [pixels, N] or
+        None)``.
 
         ``n_type`` defaults to what the model produces: uint8 for a hard argmin, float64 for non-integer occupations
         (tunnel-coupled models, ``FLAG_THERMAL``) -- the library refuses a uint8 charge map there instead of truncating.
@@ -202,11 +224,10 @@ class Engine:
         if n_type is None:
             n_type = N_F64 if (self.models.algorithm.lower() == "tunnel" or flags & FLAG_THERMAL) else N_U8
         pixels = int((scans["pix_offset"] + scans["nx"].astype(np.int64) * scans["ny"]).max())
-        z = (z_out if z_out is not None else np.empty(pixels, dtype=np.float32)) if want_z else None
+        z = self._z(pixels, z_out, want_z)
         n = None
         if n_type != N_NONE:
             n = n_out if n_out is not None else np.empty((pixels, self.models.n_dot), dtype=N_DTYPES[n_type])
-        assert z is None or (z.dtype == np.float32 and z.size >= pixels and z.flags.c_contiguous)
         # the library copies pixels * N elements of n_type into n: a short, mistyped or strided buffer would be overrun
         assert n is None or (n.dtype == N_DTYPES[n_type] and n.size >= pixels * self.models.n_dot and n.flags.c_contiguous), \
             "n_out must be a C-contiguous array of the n_type's dtype with at least pixels * n_dot elements"
@@ -215,7 +236,7 @@ class Engine:
 
     def scan_one_host(self, scan: np.ndarray, n_type: int = N_F64, flags: int = 0, pixels: int | None = None):
         """One scan window (a single ``do2d_open``), minimal host overhead: ``scan`` is a 1-element ``SCAN_DTYPE`` array with
-        ``pix_offset == 0``; returns ``(z float32 [ny * nx], n [ny * nx, N])`` -- views of per-engine staging buffers that the
+        ``pix_offset == 0``; returns ``(z float32 [ny * nx] (one sensor) or [ny * nx, S], n [ny * nx, N])`` -- views of per-engine staging buffers that the
         NEXT call overwrites (the drop-in class widens them to fresh float64 arrays).  ``pixels`` = ny * nx if the caller has
         it at hand (reading it back from the record costs a microsecond).  The library takes its single-scan path:
         descriptor in the kernel parameters, outputs written straight into mapped pinned memory, one sync."""
@@ -226,10 +247,10 @@ class Engine:
         if buf is None:
             if len(self._one_bufs) > 16:
                 self._one_bufs.clear()
-            z = np.empty(pixels, dtype=np.float32)
+            z = self._z(pixels, None, True)
             n = np.empty((pixels, self.models.n_dot), dtype=N_DTYPES[n_type])
-            buf = self._one_bufs[key] = (z, n, z.ctypes.data, n.ctypes.data, self.models.n_dot)
-        if buf[4] != self.models.n_dot:
+            buf = self._one_bufs[key] = (z, n, z.ctypes.data, n.ctypes.data, (self.models.n_dot, self.n_sensor))
+        if buf[4] != (self.models.n_dot, self.n_sensor):
             self._one_bufs.clear()
             return self.scan_one_host(scan, n_type, flags, pixels)
         rc = self._lib.qd_scan_open_host(self._ctx, 1, scan.ctypes.data, buf[2], buf[3], n_type, flags)
@@ -243,7 +264,7 @@ class Engine:
         """The observation of one batched env.step in HOST memory, compact element type (``Z_F32`` / ``Z_F16`` /
         ``Z_U8`` = rint(255 x)): scans -> per-env percentile normalisation on the device (env.py:471-509) -> typed
         copy-back, pipelined over chunks of envs.  ``scans``: env-major, ``scans_per_env`` (default N-1) equal-size
-        descriptors per env.  Returns ``(image [n_scan, ny, nx] of the z_type's dtype, stats [n_env, 2] or None)``."""
+        descriptors per env.  One-sensor model sets only (the env's observation is one sensor's image).  Returns ``(image [n_scan, ny, nx] of the z_type's dtype, stats [n_env, 2] or None)``."""
         assert scans.dtype == SCAN_DTYPE and scans.flags.c_contiguous
         spe = scans_per_env or (self.models.n_dot - 1)
         ny, nx = int(scans["ny"][0]), int(scans["nx"][0])
@@ -258,13 +279,14 @@ class Engine:
 
     def points_open_host(self, scan: np.ndarray, v: np.ndarray, n_type: int = N_F64, flags: int = 0,
                          want_z: bool = True):
-        """Arbitrary voltage list ``v`` (ny, nx, n_volt) -> ``(z (ny, nx) float32, n (ny, nx, N))``."""
+        """Arbitrary voltage list ``v`` (ny, nx, n_volt) -> ``(z (ny, nx) (one sensor) or (ny, nx, S) float32,
+        n (ny, nx, N))``."""
         v = np.ascontiguousarray(v, dtype=np.float64)
         ny, nx, nv = v.shape
         if nv != self.models.n_volt:
             raise ValueError(f"The shape of vg is in correct it should be of shape (..., n_gate) = (...,{self.models.n_volt})")
         scan = np.ascontiguousarray(scan, dtype=SCAN_DTYPE).reshape(1)
-        z = np.empty((ny, nx), dtype=np.float32) if want_z else None
+        z = self._z(ny * nx, None, want_z, (ny, nx))
         n = np.empty((ny, nx, self.models.n_dot), dtype=N_DTYPES[n_type]) if n_type != N_NONE else None
         self._check(self._lib.qd_points_open_host(self._ctx, _ptr(scan), ny, nx, _ptr(v), _ptr(z), _ptr(n), n_type,
                                                   flags))
@@ -295,11 +317,10 @@ class Engine:
         if n_type is None:
             n_type = N_F64 if flags & FLAG_THERMAL else N_U8
         pixels = int((scans["pix_offset"] + scans["nx"].astype(np.int64) * scans["ny"]).max())
-        z = (z_out if z_out is not None else np.empty(pixels, dtype=np.float32)) if want_z else None
+        z = self._z(pixels, z_out, want_z)
         n = None
         if n_type != N_NONE:
             n = n_out if n_out is not None else np.empty((pixels, self.models.n_dot), dtype=N_DTYPES[n_type])
-        assert z is None or (z.dtype == np.float32 and z.size >= pixels and z.flags.c_contiguous)
         assert n is None or (n.dtype == N_DTYPES[n_type] and n.size >= pixels * self.models.n_dot and n.flags.c_contiguous), \
             "n_out must be a C-contiguous array of the n_type's dtype with at least pixels * n_dot elements"
         self._check(self._lib.qd_scan_closed_host(self._ctx, len(scans), _ptr(scans), _ptr(q), _ptr(z), _ptr(n), n_type,
@@ -315,7 +336,7 @@ class Engine:
         if nv != self.models.n_volt:
             raise ValueError(f"The shape of vg is in correct it should be of shape (..., n_gate) = (...,{self.models.n_volt})")
         scan = np.ascontiguousarray(scan, dtype=SCAN_DTYPE).reshape(1)
-        z = np.empty((ny, nx), dtype=np.float32) if want_z else None
+        z = self._z(ny * nx, None, want_z, (ny, nx))
         n = np.empty((ny, nx, self.models.n_dot), dtype=N_DTYPES[n_type]) if n_type != N_NONE else None
         self._check(self._lib.qd_points_closed_host(self._ctx, _ptr(scan), q, ny, nx, _ptr(v), _ptr(z), _ptr(n), n_type,
                                                     flags))

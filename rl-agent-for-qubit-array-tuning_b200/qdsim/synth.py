@@ -28,8 +28,11 @@ def _by_distance(rng, n_env, n_rows, n_cols, ranges, offset=0.0):
     return rng.uniform(lo, hi, size=(n_env, n_rows, n_cols))
 
 
-def sample_devices(n_env: int, n_dot: int, seed: int = 1234):
-    """Raw (non-Maxwell) capacitance matrices + model parameters of ``n_env`` random devices."""
+def sample_devices(n_env: int, n_dot: int, seed: int = 1234, n_sensor: int = 1):
+    """Raw (non-Maxwell) capacitance matrices + model parameters of ``n_env`` random devices.
+
+    ``n_sensor`` > 1: sensor 0 and every other draw are those of the one-sensor device; sensors 1.. have their own gates
+    (gate N + s), couplings to the dots from the same range as sensor 0's and up to 0.02 to the other sensor gates."""
     rng = np.random.default_rng(seed)
     N = n_dot
     cdd = _by_distance(rng, n_env, N, N, [(0.0, 0.0), (0.0, 0.2), (0.0, 0.1), (0.0, 0.0)])
@@ -45,6 +48,17 @@ def sample_devices(n_env: int, n_dot: int, seed: int = 1234):
     p_inter = rng.uniform(0.2, 1.0, size=(n_env, N, N))
     p_inter = np.triu(p_inter, 1)
     p_inter = p_inter + np.swapaxes(p_inter, -1, -2)
+    if n_sensor > 1:
+        S = n_sensor
+        rs = np.random.default_rng([seed, 91])
+        cgd = np.concatenate([cgd, np.zeros((n_env, N, S - 1))], axis=-1)
+        cds = np.concatenate([cds, rs.uniform(0.035, 0.05, size=(n_env, S - 1, N))], axis=1)
+        cgs_all = np.zeros((n_env, S, N + S))
+        cgs_all[:, 0, :N + 1] = cgs[:, 0]
+        cgs_all[:, 1:, :N] = rs.uniform(0.0, 1e-4, size=(n_env, S - 1, N))
+        cgs_all[:, :, N:] += rs.uniform(0.0, 0.02, size=(n_env, S, S)) * (1.0 - np.eye(S))
+        cgs_all[:, np.arange(1, S), N + np.arange(1, S)] = rs.uniform(0.95, 1.0, size=(n_env, S - 1))
+        cgs = cgs_all
     return {
         "Cdd": cdd, "Cgd": cgd, "Cds": cds, "Cgs": cgs,
         "white_amp": rng.uniform(0.0, 1e-4, n_env),
@@ -65,17 +79,22 @@ def model_batch(dev: dict, algorithm: str = "default", thermal: bool = False, la
         tele_p10=dev["tele_p10"] if noise else 0.0, tele_amp=dev["tele_amp"] if noise else 0.0)
 
 
-def sample_barrier_devices(n_env: int, n_dot: int, seed: int = 1234):
+def sample_barrier_devices(n_env: int, n_dot: int, seed: int = 1234, n_sensor: int = 1):
     """``sample_devices`` plus the barrier matrices and the barrier-voltage model of the tunnel-coupled path
-    (qarray_config.yaml:72-100; qarray_base_class.py:300-357, 521-534)."""
-    dev = sample_devices(n_env, n_dot, seed)
+    (qarray_config.yaml:72-100; qarray_base_class.py:300-357, 521-534).  ``n_sensor`` as in ``sample_devices``."""
+    dev = sample_devices(n_env, n_dot, seed, n_sensor)
     rng = np.random.default_rng([seed, 77])
     N, B, G = n_dot, n_dot - 1, n_dot + 1
     dev["Cbd"] = _by_distance(rng, n_env, N, B, [(0.04, 0.08), (0.04, 0.08), (0.01, 0.03), (0.005, 0.015)], offset=0.5)
     cbg = _by_distance(rng, n_env, G, B, [(0.08, 0.15), (0.08, 0.15), (0.03, 0.18), (0.01, 0.03)], offset=0.5)
     cbg[:, N, :] = rng.uniform(0.03, 0.18, size=(n_env, B))                 # sensor gate: the distance-2 rule
+    cbs = rng.uniform(3e-4, 1e-3, size=(n_env, 1, B))
+    if n_sensor > 1:                                                        # the other sensor gates: the same rules
+        rs = np.random.default_rng([seed, 78])
+        cbg = np.concatenate([cbg, rs.uniform(0.03, 0.18, size=(n_env, n_sensor - 1, B))], axis=1)
+        cbs = np.concatenate([cbs, rs.uniform(3e-4, 1e-3, size=(n_env, n_sensor - 1, B))], axis=1)
     dev["Cbg"] = np.ascontiguousarray(np.swapaxes(cbg, -1, -2))              # (E, B, G)
-    dev["Cbs"] = rng.uniform(3e-4, 1e-3, size=(n_env, 1, B))
+    dev["Cbs"] = cbs
     dev["tc_base"] = rng.uniform(0.5, 3.0, n_env)
     dev["alpha"] = rng.uniform(0.8, 2.0, size=(n_env, B))
     return dev
@@ -90,8 +109,8 @@ def tunnel_batch(dev: dict, latching: bool = True, noise: bool = True) -> ModelB
 
 
 def ground_truth(mb: ModelBatch, dots: float = 1.0, sensor: float = 0.53):
-    """Gate voltages (E, G) that put every dot at ``dots`` carriers and the sensor at ``sensor``."""
-    n = np.concatenate([np.full(mb.n_dot, dots), [sensor]])
+    """Gate voltages (E, G) that put every dot at ``dots`` carriers and every sensor at ``sensor``."""
+    n = np.concatenate([np.full(mb.n_dot, dots), np.full(mb.n_sensor, sensor)])
     return maxwell.optimal_vg(mb.cdd_inv_full, mb.cgd_full[:, :, :mb.n_gate], n)
 
 
